@@ -2,6 +2,7 @@
 """Benchmark of the IIC MI loss hot path (BASELINE.json: "IIC MI loss fwd+bwd Mpixels/s").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--workload udaiic]
+                    [--dump-outputs DIR]
 
 Headline workload at every N (weak scaling, per-GPU work fixed) = BASELINE config 2: global + local IIC (padding 1,
 patch 512, i.e. one patch) on Up_conv2-shaped maps, per GPU 32 x 10 x 224 x 224 float32 probability maps for the two
@@ -19,8 +20,15 @@ The JSON line carries, beyond the base contract:
             MEASURED_PEAKS.json's HBM copy bandwidth
   cpu_baseline  the reference's own loss classes (oracle/_ref, loaded by oracle/ref_loader.py) on the host cores
   extra     secondary shapes and terms, and the whole udaiic iteration on the reference's own epocher
+  dumped_outputs  with ``--dump-outputs DIR``: which arrays were written there
 
 ``--impl reference`` times the reference's own CPU implementation of the same workload (same config dict).
+
+``--dump-outputs DIR`` writes what the last of the ``--steps`` timed steps returned -- the total loss and the gradient of
+every differentiable input -- as ``DIR/<name>.npy`` (float32, at most 60 MiB in all; a large gradient is stored as a fixed,
+seeded sample of its elements).  The inputs depend only on the arguments, so two builds can be compared array by array;
+the local-term gradients vary by a few float32 ulps from run to run (the order of their reductions is not fixed), so
+compare them with a tolerance.
 """
 from __future__ import annotations
 
@@ -76,9 +84,16 @@ def parse():
                     help="udaiic: whole training iterations/s of the reference's UDAIICEpocher, losses swapped vs not")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replay")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and input gradients of the last timed step as DIR/<name>.npy (float32; "
+                         "rank 0's shard when several GPUs run)")
     a = ap.parse_args()
     if a.steps is None:
         a.steps = 2000 if (a.config == 2 and a.impl == "b200") else 20
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "loss"):
+        ap.error("--dump-outputs applies to the loss workload of the b200 implementation")
     return a
 
 
@@ -240,6 +255,44 @@ def build_step(wl, B, crits, iic_losses, uda_fn, torch):
         return total, torch.autograd.grad(total, diff)
 
     return step
+
+
+DUMP_BYTES = 60 * 2**20        # --dump-outputs writes at most this many bytes of array data
+
+
+def output_names(wl):
+    """Names of what build_step's step returns: the total loss, then the gradient of every differentiable input."""
+    names = ["loss"]
+    for gi, (kind, *_rest) in enumerate(wl["groups"]):
+        names += [f"grad_{gi}_{kind}_x", f"grad_{gi}_{kind}_y"]
+    if wl["uda"]:
+        names.append("grad_uda_student")
+    return names
+
+
+def dump_outputs(out_dir, wl, loss, grads, seed=0):
+    """Writes the loss and the gradients of one step as out_dir/<name>.npy in float32, DUMP_BYTES in all.  The arrays
+    are taken smallest first, each with an equal share of what the ones before it left unused; an array larger than its
+    share is replaced by the elements at a fixed, seeded set of flat indices (sorted), the same set for the same shapes,
+    so that two builds of the project can be compared output for output."""
+    import numpy as np
+    arrays = [loss.detach().reshape(1)] + [g.detach() for g in grads]
+    names = output_names(wl)
+    assert len(names) == len(arrays), (names, len(arrays))
+    left = DUMP_BYTES // 4
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    for n, i in enumerate(sorted(range(len(arrays)), key=lambda i: arrays[i].numel())):
+        t = arrays[i]
+        a = t.float().cpu().numpy().reshape(-1)
+        cap = left // (len(arrays) - n)
+        if a.size > cap:
+            idx = np.random.default_rng([seed, a.size, cap]).choice(a.size, size=cap, replace=False)
+            a = a[np.sort(idx)]
+        left -= a.size
+        np.save(os.path.join(out_dir, names[i] + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+        written[names[i]] = {"numel": int(t.numel()), "written": int(a.size)}
+    return {name: written[name] for name in names}
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -533,10 +586,11 @@ def run_b200(args):
             torch.cuda.synchronize()
 
     def run_one(i):
+        """One step on input set i % NSETS; returns its (loss, gradients)."""
         if use_graph:
             graphs[i % NSETS][0].replay()
-        else:
-            step_fn(sets[i % NSETS])
+            return graphs[i % NSETS][1]
+        return step_fn(sets[i % NSETS])
 
     def barrier():
         if world > 1:
@@ -555,7 +609,7 @@ def run_b200(args):
     t_wall0 = time.perf_counter()
     e0.record()
     for i in range(args.steps):
-        run_one(i)
+        last = run_one(i)
     e1.record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
@@ -568,6 +622,8 @@ def run_b200(args):
     ms_step = ms_total / args.steps
     value = px_job / (ms_step * 1e-3) / 1e6
     iic_b200.raise_if_flagged(dev)           # the deferred simplex / NaN checks of every step above
+    dumped = dump_outputs(args.dump_outputs, wl, *last) if (args.dump_outputs and rank == 0) else None
+    del last
 
     ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
 
@@ -906,6 +962,9 @@ def run_b200(args):
             "wall_s_timed_region": round(t_wall, 4),
             "extra": extra,
         }
+        if dumped is not None:
+            line["dumped_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "step": args.steps - 1,
+                                      "input_set": (args.steps - 1) % NSETS, "arrays": dumped}
         print(json.dumps(line), flush=True)
     watchdog.cancel()
     if world > 1:

@@ -2,7 +2,9 @@
 
 The golden vectors in tests/golden/ were produced by oracle/make_golden.py, which runs the
 UNMODIFIED reference classes (fp64 and fp32).  These tests pin the restatement to them; they run
-on CPU.  When /root/reference is mounted (the build container) the reference is also re-run live.
+on CPU.  When the original project's source is provided (IIC_REFERENCE_ROOT, or the copy oracle/make_ref.py lays out
+under oracle/_ref/) the reference is also re-run live.  The live tests use inputs of their own for which no reference
+outputs are stored, so without the source they skip and what they check is not covered.
 """
 import os
 import sys
@@ -160,8 +162,11 @@ def test_torch_port_global(name):
     assert relmax(P.detach().numpy(), g["P_f64"]) < 1e-11
 
 
-# ---- live re-run of the reference (build container only) ----------------------------------------
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
+# ---- live re-run of the reference (when its source is provided) ---------------------------------
+REF_MISSING = "the original project's source is not provided (IIC_REFERENCE_ROOT or oracle/_ref/reference)"
+
+
+@pytest.mark.skipif(not ref_loader.available(), reason=REF_MISSING)
 def test_live_reference_agrees_with_oracle_on_fresh_inputs():
     ns = ref_loader.load()
     torch = ns.torch
@@ -176,7 +181,7 @@ def test_live_reference_agrees_with_oracle_on_fresh_inputs():
     assert relmax(ox, gx.numpy()) < 1e-8 and relmax(oy, gy.numpy()) < 1e-8
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not ref_loader.available(), reason=REF_MISSING)
 def test_live_reference_supervised_branch():
     ns = ref_loader.load()
     torch = ns.torch
@@ -194,7 +199,7 @@ def test_live_reference_supervised_branch():
     assert np.array_equal(meter._unions[0].numpy(), union)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not ref_loader.available(), reason=REF_MISSING)
 def test_live_reference_flip_draws():
     ns = ref_loader.load()
     torch = ns.torch
