@@ -2,7 +2,7 @@
 
     python tools/near_uniform_check.py
 
-Compares the tensor-core path, the FP32 path (IIC_B200_NO_TC=1) and the fp64 oracle on the loss and the gradients for
+Compares the tensor-core path, the FP32 path (the no_tc switch) and the fp64 oracle on the loss and the gradients for
 K = 20 (padding 3) and K = 128 (padding 1) maps made by a weak random 1x1 head, the regime of the first training
 iterations.
 """
@@ -22,8 +22,8 @@ for (B, K, H, W, pad, scale) in [(10, 20, 224, 224, 3, 0.05), (10, 20, 224, 224,
     crit = iic_b200.IIDSegmentationSmallPathLoss(padding=pad, patch_size=1024)
     res = {}
     for mode in ("tc", "notc"):
-        if mode == "notc": os.environ["IIC_B200_NO_TC"] = "1"
-        else: os.environ.pop("IIC_B200_NO_TC", None)
+        # the library reads IIC_B200_NO_TC once, when it loads: switch at run time
+        iic_b200._lib.set_option("no_tc", 1 if mode == "notc" else 0)
         l = crit(x, y)
         gx, gy = torch.autograd.grad(l, (x, y))
         res[mode] = (l.item(), gx.clone(), gy.clone())
