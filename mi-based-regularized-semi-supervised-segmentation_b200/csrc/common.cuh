@@ -61,9 +61,7 @@ const Options& options();
 // Layout of the Wx / Wy buffers (iic_local_coeff_floats floats each): the coefficient tensor [patch][cin][tap][Kp] that
 // iic_local_epilogue writes, then -- 1 KB aligned -- room for the operand-order "weight image" the tensor-core backward
 // kernels build from it (0 bytes when (K, pad, n_patches) never selects such a kernel).  The image is per call and
-// per buffer, so concurrent backwards on different streams never share scratch.
-size_t local_bwd_tc_image_bytes(int K, int pad);      // local_bwd_tc.cu   (K = 128, padding 1)
-size_t local_bwd_tcrb_image_bytes(int K, int pad);    // local_bwd_tcrb.cu (16 <= K <= 24, padding 1 or 3)
+// per buffer, so concurrent backwards on different streams never share scratch.  Image sizes: local_kernels.cuh.
 inline size_t local_coeff_base_floats(int K, int pad, int n_patches) {
   const int T = 2 * pad + 1, Kp = (K + 3) & ~3;
   return (size_t)n_patches * K * T * T * Kp;

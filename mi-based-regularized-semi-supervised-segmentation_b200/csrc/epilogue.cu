@@ -3,6 +3,7 @@
 //     analytic dL/dJ                                    (contrastyou/losses/iic_loss.py:124-146,186)
 //   * global joint / epilogue / backward on (N,K) rows  (contrastyou/losses/iic_loss.py:43-94)
 #include "epilogue.cuh"
+#include "local_kernels.cuh"
 
 namespace iic {
 

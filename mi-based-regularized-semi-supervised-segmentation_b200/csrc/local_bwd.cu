@@ -13,6 +13,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 
 namespace iic {
 
@@ -195,29 +196,6 @@ static int dispatch_ocb(int ocb, const LocalBwdParams& P, dim3 grid, size_t smem
 
 }  // namespace iic
 
-namespace iic {
-int local_bwd_tma_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                      long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                      const float* Wx, const float* Wy, const float* grad_loss, float* gx, float* gy, long long gx_sn,
-                      long long gy_sn, int sms, cudaStream_t st);
-int local_bwd_fast_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                       long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                       const float* Wx, const float* Wy, const float* grad_loss, float* gx, float* gy, long long gx_sn,
-                       long long gy_sn, int sms, int from_logits, float inv_temp, cudaStream_t st);
-int local_bwd_tc_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                     long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* Wx, float* Wy,
-                     const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, cudaStream_t st);
-int local_bwd_tcrb_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                       long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* Wx, float* Wy,
-                       const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, cudaStream_t st);
-int local_bwd_tcrb10h_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                          long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, const float* Wx, const float* Wy,
-                          const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, int from_logits,
-                          float inv_temp, cudaStream_t st);
-int local_bwd_tcrb10_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                         long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, const float* Wx, const float* Wy,
-                         const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, cudaStream_t st);
-}
 using namespace iic;
 
 extern "C" int iic_local_backward(const float* x, long long x_sn, long long x_sc, long long x_sh,
@@ -241,36 +219,22 @@ extern "C" int iic_local_backward(const float* x, long long x_sn, long long x_sc
   const int sms = sm_count_cached(current_device());
   IIC_REQUIRE(sms > 0, "iic_local_backward: no device");
 
-  // fast path: one patch, no mask, TMA-describable rows, small window (local_bwd_tma.cu)
+  // fast path: one patch, no mask, TMA-describable rows -> the specialised kernels (local_kernels.cuh)
   if (n_patches == 1 && mask == nullptr && !options().no_tma) {
+    const LocalMaps m{{x, x_sn, x_sc, x_sh}, {y, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
+    const LocalGrads gr{grad_loss, gx, gy, gx_sn, gy_sn};
+    int rc = -1;
     // wide cluster heads (K = 128): tcgen05 3xTF32 sweeps (local_bwd_tc.cu)
-    if (!options().no_tc) {
-      const int rc_tc = local_bwd_tc_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss,
-                                         gx, gy, gx_sn, gy_sn, st);
-      if (rc_tc >= 0) return rc_tc;
-      // 10 clusters, padding 1 (config 2): row-block tensor-core sweeps with the leftover-slot MMA (local_bwd_tcrb10.cu)
-      if (!options().no_tc10) {
-        // fp16-split variant (6 MMAs per source row and tile) by default; tc10_tf32 selects the tf32 + bf16 one (8 MMAs)
-        const int rc_10 = options().tc10_tf32 ? local_bwd_tcrb10_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy,
-                                                                      grad_loss, gx, gy, gx_sn, gy_sn, st)
-                                              : local_bwd_tcrb10h_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss,
-                                               gx, gy, gx_sn, gy_sn, 0, 1.f, st);
-        if (rc_10 >= 0) return rc_10;
-      }
-      // the reference's default cluster count (16 <= K <= 24), padding 1 or 3: row-block tensor-core sweeps
-      // (local_bwd_tcrb.cu; at padding 1 only when the map has enough row blocks to fill the SMs, decided inside)
-      {
-        const int rc_rb = local_bwd_tcrb_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss,
-                                             gx, gy, gx_sn, gy_sn, st);
-        if (rc_rb >= 0) return rc_rb;
-      }
-    }
-    int rc = options().no_fast ? -1
-                 : local_bwd_fast_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy,
-                                      grad_loss, gx, gy, gx_sn, gy_sn, sms, 0, 1.f, st);
-    if (rc < 0)
-      rc = local_bwd_tma_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss,
-                             gx, gy, gx_sn, gy_sn, sms, st);
+    if (!options().no_tc) rc = local_bwd_tc_try(m, Wx, Wy, gr, st);
+    // 10 clusters, padding 1 (config 2): row-block tensor-core sweeps with the leftover-slot MMA (local_bwd_tcrb10.cu);
+    // fp16-split variant (6 MMAs per source row and tile) by default, tc10_tf32 selects the tf32 + bf16 one (8 MMAs)
+    if (rc < 0 && !options().no_tc && !options().no_tc10)
+      rc = options().tc10_tf32 ? local_bwd_tcrb10_try(m, Wx, Wy, gr, st) : local_bwd_tcrb10h_try(m, Wx, Wy, gr, 0, 1.f, st);
+    // the reference's default cluster count (16 <= K <= 24), padding 1 or 3: row-block tensor-core sweeps
+    // (local_bwd_tcrb.cu; at padding 1 only when the map has enough row blocks to fill the SMs, decided inside)
+    if (rc < 0 && !options().no_tc) rc = local_bwd_tcrb_try(m, Wx, Wy, gr, st);
+    if (rc < 0 && !options().no_fast) rc = local_bwd_fast_try(m, Wx, Wy, gr, 0, 1.f, st);
+    if (rc < 0) rc = local_bwd_tma_try(m, Wx, Wy, gr, st);
     if (rc >= 0) return rc;
   }
 
@@ -332,15 +296,14 @@ extern "C" int iic_local_backward_from_logits(const float* lx, long long x_sn, l
   IIC_REQUIRE(lx && ly && Wx && Wy && g_lx && g_ly, "iic_local_backward_from_logits: null pointer");
   const int sms = sm_count_cached(current_device());
   IIC_REQUIRE(sms > 0, "iic_local_backward_from_logits: no device");
+  const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
+  const LocalGrads gr{grad_loss, g_lx, g_ly, gx_sn, gy_sn};
+  int rc = -1;
   // the fp16-split tensor-core backward has a from-logits form (softmax in its transform warps, adjoint in its drain);
   // same shape rule as for probabilities (enough rows to fill the SMs, or tc10_force)
-  if (!options().no_tc && !options().no_tc10 && !options().no_tma) {
-    const int rc_tc = local_bwd_tcrb10h_try(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss, g_lx,
-                                            g_ly, gx_sn, gy_sn, 1, inv_temperature, st);
-    if (rc_tc >= 0) return rc_tc;
-  }
-  const int rc = local_bwd_fast_try(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, Wx, Wy, grad_loss,
-                                    g_lx, g_ly, gx_sn, gy_sn, sms, 1, inv_temperature, st);
+  if (!options().no_tc && !options().no_tc10 && !options().no_tma)
+    rc = local_bwd_tcrb10h_try(m, Wx, Wy, gr, 1, inv_temperature, st);
+  if (rc < 0) rc = local_bwd_fast_try(m, Wx, Wy, gr, 1, inv_temperature, st);
   if (rc < 0) {
     set_error("iic_local_backward_from_logits: shape not covered by the fused kernel (needs padding 1, K == 10, "
               "W %% 4 == 0, W <= 248, 16-byte aligned rows)");

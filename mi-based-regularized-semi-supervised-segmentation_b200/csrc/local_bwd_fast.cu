@@ -25,6 +25,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tma.cuh"
 
 namespace iic {
@@ -294,12 +295,10 @@ static int launch_bwd_fast(const CUtensorMap& mx, const CUtensorMap& my, const B
   return 0;
 }
 
-// 0 = launched, 1 = error, -1 = not eligible (caller falls back to the other kernels)
-int local_bwd_fast_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                       long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                       const float* Wx, const float* Wy, const float* grad_loss, float* gx, float* gy, long long gx_sn,
-                       long long gy_sn, int sms, int from_logits, float inv_temp, cudaStream_t st) {
+int local_bwd_fast_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, int from_logits,
+                       float inv_temp, cudaStream_t st) {
   using namespace bwdfast;
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad;
   if (pad != 1 && pad != 3) return -1;
   // output-channel block: 10 for the udaiic cluster counts (10, 20), 8 for other multiples of 8 (.., 128)
   const int KB = (K % 10 == 0 && K <= 40) ? 10 : (K % 8 == 0 ? 8 : 0);
@@ -308,7 +307,8 @@ int local_bwd_fast_try(const float* x, long long x_sn, long long x_sc, long long
   const int WROW = (KB + 3) & ~3;
   if (W % 4 != 0 || W < 4) return -1;
   if (from_logits && W > 248) return -1;
-  if ((reinterpret_cast<uintptr_t>(gx) & 15) || (reinterpret_cast<uintptr_t>(gy) & 15) || (gx_sn & 3) || (gy_sn & 3)) return -1;
+  if ((reinterpret_cast<uintptr_t>(g.gx) & 15) || (reinterpret_cast<uintptr_t>(g.gy) & 15) || (g.gx_sn & 3) || (g.gy_sn & 3))
+    return -1;
   const int T = 2 * pad + 1, T2 = T * T, Kp = (K + 3) & ~3;
   const int CB = from_logits ? 10 : (KB == 10 ? 5 : 4);   // the fused softmax needs all K channels in one stage
   const int nthreads = 512, stages = from_logits ? 2 : (pad == 1 ? 4 : 3);
@@ -329,16 +329,17 @@ int local_bwd_fast_try(const float* x, long long x_sn, long long x_sc, long long
   P.stage_bytes = (P.box_bytes + 127u) & ~127u;
   const size_t smem = (size_t)P.stage_bytes * stages;
   if (smem > 226 * 1024) return -1;
-  P.grad_loss = grad_loss; P.gx = gx; P.gy = gy; P.gx_sn = gx_sn; P.gy_sn = gy_sn;
-  P.lx = x; P.lx_sn = x_sn; P.lx_sc = x_sc; P.lx_sh = x_sh;
-  P.ly = y; P.ly_sn = y_sn; P.ly_sc = y_sc; P.ly_sh = y_sh;
+  P.grad_loss = g.grad_loss; P.gx = g.gx; P.gy = g.gy; P.gx_sn = g.gx_sn; P.gy_sn = g.gy_sn;
+  P.lx = m.x.p; P.lx_sn = m.x.sn; P.lx_sc = m.x.sc; P.lx_sh = m.x.sh;
+  P.ly = m.y.p; P.ly_sn = m.y.sn; P.ly_sc = m.y.sc; P.ly_sh = m.y.sh;
   P.inv_temp = inv_temp;
-  if (from_logits && ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15) ||
-                      (x_sh % 4) || (x_sc % 4) || (x_sn % 4) || (y_sh % 4) || (y_sc % 4) || (y_sn % 4)))
-    return -1;
+  auto rows16 = [](const View4& v) {
+    return (reinterpret_cast<uintptr_t>(v.p) & 15) == 0 && v.sh % 4 == 0 && v.sc % 4 == 0 && v.sn % 4 == 0;
+  };
+  if (from_logits && (!rows16(m.x) || !rows16(m.y))) return -1;
   CUtensorMap mx, my;
-  if (!make_map_4d(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, P.XP, P.XR, CB)) return -1;
-  if (!make_map_4d(&my, y, B, K, H, W, y_sn, y_sc, y_sh, P.XP, P.XR, CB)) return -1;
+  if (!make_map_4d(&mx, m.x, m, P.XP, P.XR, CB)) return -1;
+  if (!make_map_4d(&my, m.y, m, P.XP, P.XR, CB)) return -1;
   const int nob = K / KB;
 
   // How many (sweep, output block) weight slabs fit in the constant bank at once decides the launches:
@@ -365,7 +366,7 @@ int local_bwd_fast_try(const float* x, long long x_sn, long long x_sc, long long
       }
     P.wc_base = base / 2;
     P.sw0 = sw0; P.nsw = nsw; P.ob0 = ob0;
-    int gxd = sms / nobl;
+    int gxd = m.sms / nobl;
     if (gxd < 1) gxd = 1;
     if (gxd > P.rows_total) gxd = (int)P.rows_total;
     const dim3 grid(gxd, nobl);

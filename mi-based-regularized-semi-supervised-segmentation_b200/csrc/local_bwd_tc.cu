@@ -28,6 +28,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -282,38 +283,19 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
   if (wid == 3) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
 }
 
-static bool make_map(CUtensorMap* map, const float* base, int B, int H, int W, long long sn, long long sc, long long sh) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
-  if ((sh * 4) % 16 != 0 || (sc * 4) % 16 != 0 || (sn * 4) % 16 != 0) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)KC, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-  cuuint32_t box[4] = {(cuuint32_t)(W + 8), 2, (cuuint32_t)SL, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace bwdtc
 
 size_t local_bwd_tc_image_bytes(int K, int pad) {
   return (K == bwdtc::KC && pad == 1) ? (size_t)bwdtc::NSL * 9 * bwdtc::W_TILE : 0;
 }
 
-// Returns 0 when launched, < 0 when the shape is not covered (the caller falls back to the FFMA2 kernels), > 0 on error.
-int local_bwd_tc_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                     long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* Wx, float* Wy,
-                     const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, cudaStream_t st) {
+int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
   using namespace bwdtc;
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad, sms = m.sms;
   if (K != KC || pad != 1 || W % 4 != 0 || W > MAXW || W < 8) return -1;
   CUtensorMap mx, my;
-  if (!make_map(&mx, x, B, H, W, x_sn, x_sc, x_sh)) return -1;
-  if (!make_map(&my, y, B, H, W, y_sn, y_sc, y_sh)) return -1;
-  const int device = current_device();
-  const int sms = sm_count_cached(device);
-  if (sms <= 0) return -1;
+  if (!make_map_4d(&mx, m.x, m, W + 8, 2, SL)) return -1;
+  if (!make_map_4d(&my, m.y, m, W + 8, 2, SL)) return -1;
   // the weight image lives in the tail of the caller's coefficient buffer (common.cuh)
   float* img_x = Wx + local_coeff_image_offset(K, pad, 1);
   float* img_y = Wy + local_coeff_image_offset(K, pad, 1);
@@ -325,9 +307,9 @@ int local_bwd_tc_try(const float* x, long long x_sn, long long x_sc, long long x
   weight_image_kernel<<<(wthreads + 255) / 256, 256, 0, st>>>(Wy, img_y);
   IIC_CHECK_CUDA(cudaGetLastError());
   const int dbg = tc::bringup_env("IIC_TC_DBG", 0);
-  Params Pgx{B, H, W, n_items, img_x, grad_loss, gx, gx_sn, dbg};     // dL/dx from y
+  Params Pgx{B, H, W, n_items, img_x, g.grad_loss, g.gx, g.gx_sn, dbg};     // dL/dx from y
   local_bwd_tc_kernel<<<grid, NTHREADS, SMEM_BYTES, st>>>(my, Pgx);
-  Params Pgy{B, H, W, n_items, img_y, grad_loss, gy, gy_sn, dbg};     // dL/dy from x
+  Params Pgy{B, H, W, n_items, img_y, g.grad_loss, g.gy, g.gy_sn, dbg};     // dL/dy from x
   local_bwd_tc_kernel<<<grid, NTHREADS, SMEM_BYTES, st>>>(mx, Pgy);
   IIC_CHECK_CUDA(cudaGetLastError());
   return 0;

@@ -20,6 +20,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -319,20 +320,6 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
   if (wid == 3) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
 }
 
-static bool make_map(CUtensorMap* map, const float* base, int B, int K, int H, int W, long long sn, long long sc, long long sh, int box_w) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
-  if ((sh * 4) % 16 != 0 || (sc * 4) % 16 != 0 || (sn * 4) % 16 != 0) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)K, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-  cuuint32_t box[4] = {(cuuint32_t)box_w, 1, (cuuint32_t)SL, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <int T>
 static int launch(const CUtensorMap& m, const Params& P, int grid, size_t smem, cudaStream_t st) {
   IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tcrb_kernel<T>), (int)(SMEM_LIMIT)));
@@ -349,11 +336,9 @@ size_t local_bwd_tcrb_image_bytes(int K, int pad) {
   return (size_t)(KP / bwdrb::SL) * 64 * T * T * KP;
 }
 
-// Returns 0 when launched, < 0 when the shape is not covered (the caller falls back to the FFMA2 kernels), > 0 on error.
-int local_bwd_tcrb_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                       long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* Wx, float* Wy,
-                       const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, cudaStream_t st) {
+int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
   using namespace bwdrb;
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad, sms = m.sms;
   if (K < 16 || K > 24 || (pad != 1 && pad != 3) || W % 4 != 0 || W < 8) return -1;
   // maps wider than one TMA box are cut into column panels: 128 columns (one pixel tile, no padding) when that divides
   // the width, else equal panels of at most 248 columns
@@ -375,11 +360,8 @@ int local_bwd_tcrb_try(const float* x, long long x_sn, long long x_sc, long long
   while (na < NA_MAX && spare >= (long long)(na + 1) * A_ROW + (long long)nraw * RAW_MAX) ++na;
   const size_t smem = (size_t)2 * ((wslice + 127) & ~127) + (size_t)na * A_ROW + (size_t)nraw * RAW_MAX + 1024;
   CUtensorMap mx, my;
-  if (!make_map(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, PW + 8)) return -1;
-  if (!make_map(&my, y, B, K, H, W, y_sn, y_sc, y_sh, PW + 8)) return -1;
-  const int device = current_device();
-  const int sms = sm_count_cached(device);
-  if (sms <= 0) return -1;
+  if (!make_map_4d(&mx, m.x, m, PW + 8, 1, SL)) return -1;
+  if (!make_map_4d(&my, m.y, m, PW + 8, 1, SL)) return -1;
   const int nblk = (H + R - 1) / R;
   const int n_items = B * nblk * npanel;
   // 3 x 3 window: the FFMA2 kernel is as fast unless there are enough row blocks to keep every SM busy (measured:
@@ -393,8 +375,8 @@ int local_bwd_tcrb_try(const float* x, long long x_sn, long long x_sc, long long
   weight_image_kernel<<<(wthreads + 255) / 256, 256, 0, st>>>(Wx, img_x, K, Kp4, KP, NS, T);
   weight_image_kernel<<<(wthreads + 255) / 256, 256, 0, st>>>(Wy, img_y, K, Kp4, KP, NS, T);
   IIC_CHECK_CUDA(cudaGetLastError());
-  Params Pgx{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_x, grad_loss, gx, gx_sn};     // dL/dx from y
-  Params Pgy{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_y, grad_loss, gy, gy_sn};     // dL/dy from x
+  Params Pgx{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_x, g.grad_loss, g.gx, g.gx_sn};     // dL/dx from y
+  Params Pgy{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_y, g.grad_loss, g.gy, g.gy_sn};     // dL/dy from x
   if (T == 3) {
     if (int rc = launch<3>(my, Pgx, grid, smem, st)) return rc;
     return launch<3>(mx, Pgy, grid, smem, st);

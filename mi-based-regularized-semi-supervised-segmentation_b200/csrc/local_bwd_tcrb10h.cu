@@ -20,6 +20,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -580,41 +581,22 @@ local_bwd_tcrb10h_kernel(const __grid_constant__ CUtensorMap map0, const __grid_
   if (wid == 3) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
 }
 
-static bool make_map(CUtensorMap* map, const float* base, int B, int K, int H, int W, long long sn, long long sc, long long sh) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
-  if ((sh * 4) % 16 != 0 || (sc * 4) % 16 != 0 || (sn * 4) % 16 != 0) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)K, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-  cuuint32_t box[4] = {(cuuint32_t)(W + 8), 1, (cuuint32_t)K, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace bwdrb10h
 
-// Returns 0 when launched, < 0 when the shape is not covered (the caller falls back to the FFMA2 kernels), > 0 on error.
-int local_bwd_tcrb10h_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                         long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, const float* Wx, const float* Wy,
-                         const float* grad_loss, float* gx, float* gy, long long gx_sn, long long gy_sn, int from_logits,
-                         float inv_temp, cudaStream_t st) {
+int local_bwd_tcrb10h_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, int from_logits,
+                          float inv_temp, cudaStream_t st) {
   using namespace bwdrb10h;
-  if ((K != 9 && K != 10) || pad != 1 || W % 4 != 0 || W > MAXW || W < 8) return -1;
-  const int device = current_device();
-  const int sms = sm_count_cached(device);
-  if (sms <= 0) return -1;
+  const int B = m.B, K = m.K, H = m.H, W = m.W, sms = m.sms;
+  if ((K != 9 && K != 10) || m.pad != 1 || W % 4 != 0 || W > MAXW || W < 8) return -1;
   if ((long long)B * H < 8LL * sms && !options().tc10_force) return -1;   // too few rows to fill the SMs: FFMA2 is faster
   CUtensorMap mx, my;
-  if (!make_map(&mx, x, B, K, H, W, x_sn, x_sc, x_sh)) return -1;
-  if (!make_map(&my, y, B, K, H, W, y_sn, y_sc, y_sh)) return -1;
+  if (!make_map_4d(&mx, m.x, m, W + 8, 1, K)) return -1;
+  if (!make_map_4d(&my, m.y, m, W + 8, 1, K)) return -1;
   IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tcrb10h_kernel<false>), (int)(SMEM_BYTES)));
   IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tcrb10h_kernel<true>), (int)(SMEM_BYTES_FL)));
   const int Kp4 = (K + 3) & ~3;
-  Params P{B, H, W, K, {Wx, Wy}, Kp4, grad_loss, {gx, gy}, {gx_sn, gy_sn}, from_logits, inv_temp, {x, y}, {x_sn, y_sn}, {x_sc, y_sc},
-           {x_sh, y_sh}};
+  Params P{B, H, W, K, {Wx, Wy}, Kp4, g.grad_loss, {g.gx, g.gy}, {g.gx_sn, g.gy_sn}, from_logits, inv_temp, {m.x.p, m.y.p},
+           {m.x.sn, m.y.sn}, {m.x.sc, m.y.sc}, {m.x.sh, m.y.sh}};
   // one launch, two sweeps per CTA: dL/dx from y (sweep 0), then dL/dy from x (sweep 1)
   if (from_logits) local_bwd_tcrb10h_kernel<true><<<sms, NTHREADS_FL, SMEM_BYTES_FL, st>>>(my, mx, P);
   else local_bwd_tcrb10h_kernel<false><<<sms, NTHREADS, SMEM_BYTES, st>>>(my, mx, P);

@@ -9,6 +9,7 @@
 // broadcast 128-bit shared-memory loads that are already (w[c], w[c+1]) pairs, so every update is one
 // fma.rn.f32x2 (FFMA2).
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tma.cuh"
 
 namespace iic {
@@ -198,15 +199,13 @@ static int launch_bwd_tma(const CUtensorMap& mx, const CUtensorMap& my, const Bw
   return 0;
 }
 
-// 0 = launched, 1 = error, -1 = not eligible (caller falls back to the generic kernel)
-int local_bwd_tma_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                      long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                      const float* Wx, const float* Wy, const float* grad_loss, float* gx, float* gy, long long gx_sn,
-                      long long gy_sn, int sms, cudaStream_t st) {
+int local_bwd_tma_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, cudaStream_t st) {
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad;
   const int T = 2 * pad + 1;
   if (T > 3 || K > 12 || K < 1) return -1;
   if (W % 4 != 0) return -1;
-  if ((reinterpret_cast<uintptr_t>(gx) & 15) || (reinterpret_cast<uintptr_t>(gy) & 15) || (gx_sn & 3) || (gy_sn & 3)) return -1;
+  if ((reinterpret_cast<uintptr_t>(g.gx) & 15) || (reinterpret_cast<uintptr_t>(g.gy) & 15) || (g.gx_sn & 3) || (g.gy_sn & 3))
+    return -1;
   BwdTmaParams P;
   P.B = B; P.K = K; P.Kp = (K + 3) & ~3; P.H = H; P.W = W; P.pad = pad;
   P.tiles_h = (H + BT_ROWS - 1) / BT_ROWS;
@@ -226,12 +225,12 @@ int local_bwd_tma_try(const float* x, long long x_sn, long long x_sc, long long 
   P.CB = CB; P.nchunk = K / CB;
   P.box_bytes = (unsigned)((size_t)CB * P.XR * BT_XP * 4);
   P.stage_bytes = (P.box_bytes + 127u) & ~127u;
-  P.Wx = Wx; P.Wy = Wy; P.grad_loss = grad_loss; P.gx = gx; P.gy = gy; P.gx_sn = gx_sn; P.gy_sn = gy_sn;
+  P.Wx = Wx; P.Wy = Wy; P.grad_loss = g.grad_loss; P.gx = g.gx; P.gy = g.gy; P.gx_sn = g.gx_sn; P.gy_sn = g.gy_sn;
   CUtensorMap mx, my;
-  if (!make_map_4d(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, BT_XP, P.XR, CB)) return -1;
-  if (!make_map_4d(&my, y, B, K, H, W, y_sn, y_sc, y_sh, BT_XP, P.XR, CB)) return -1;
+  if (!make_map_4d(&mx, m.x, m, BT_XP, P.XR, CB)) return -1;
+  if (!make_map_4d(&my, m.y, m, BT_XP, P.XR, CB)) return -1;
   long long items = (long long)B * P.tiles_h * P.tiles_w;
-  int grid = sms;
+  int grid = m.sms;
   if (grid > items) grid = (int)items;
   const size_t smem = (size_t)P.stage_bytes * BT_STAGES + wbytes;
   if (T == 1) {

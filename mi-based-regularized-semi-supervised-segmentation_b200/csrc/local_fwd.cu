@@ -16,6 +16,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 
 namespace iic {
 
@@ -305,7 +306,7 @@ static void tile_shape_for(int T, int* IT, int* JT, int* DYB) {
   }
 }
 
-static bool make_fwd_plan(int device, int B, int K, const PatchGrid& g, int pad, FwdPlan* pl) {
+static bool make_fwd_plan(int sms, int B, int K, const PatchGrid& g, int pad, FwdPlan* pl) {
   pl->T = 2 * pad + 1;
   if (pad < 0 || pad > 7) return false;
   tile_shape_for(pl->T, &pl->IT, &pl->JT, &pl->DYB);
@@ -326,7 +327,6 @@ static bool make_fwd_plan(int device, int B, int K, const PatchGrid& g, int pad,
   pl->tiles_w = (g.pw + TW - 1) / TW;
   pl->smem_bytes = (size_t)pl->kchunk * ((size_t)pl->XR * pl->XP + (size_t)TH * TW) * sizeof(float);
   pl->n_patches = g.nh * g.nw;
-  const int sms = sm_count_cached(device);
   if (sms <= 0) return false;
   long long items = (long long)B * pl->tiles_h * pl->tiles_w;
   long long per = sms / pl->n_patches;
@@ -346,6 +346,31 @@ static int launch_fwd(const LocalFwdParams& P, dim3 grid, int nthreads, size_t s
   return 0;
 }
 
+// info == nullptr: reduce the per-CTA slots into J (fp64, fixed order) with the reduce kernel of their layout.
+// info != nullptr: leave them in `partial` and describe them in *info (for iic_finish); J is unused.
+static int reduce_or_describe_slots(const SlotInfo& s, const float* partial, int T, int K, int n_patches, double* J,
+                                    iic_slot_info* info, cudaStream_t st) {
+  if (info) {
+    info->layout = s.layout;
+    info->n_slots = s.n_slots;
+    info->slot_stride = s.slot_stride;
+    info->nb = s.nb;
+    return 0;
+  }
+  if (s.layout == SLOT_PACKED) {
+    const int E = T * T * K * K;
+    fwdtcp::reduce_packed_kernel<<<(E + 31) / 32, 1024, 0, st>>>(partial, s.n_slots, (int)s.slot_stride, T, K, s.nb, J);
+  } else {
+    const dim3 rgrid((unsigned)((s.slot_stride + 31) / 32), n_patches);
+    if (s.layout == SLOT_TC128)
+      reduce_partials_kernel<true><<<rgrid, RED_GROUPS * 32, 0, st>>>(partial, s.n_slots, s.slot_stride, J);
+    else
+      reduce_partials_kernel<false><<<rgrid, RED_GROUPS * 32, 0, st>>>(partial, s.n_slots, s.slot_stride, J);
+  }
+  IIC_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 }  // namespace iic
 
 using namespace iic;
@@ -360,14 +385,12 @@ extern "C" int iic_local_num_patches(int H, int W, int patch_h, int patch_w, int
   return g.nh * g.nw;
 }
 
-namespace iic { size_t local_joint_tcp_slot_floats(int K, int pad); }
-
 extern "C" size_t iic_local_joint_workspace_bytes(int device, int B, int K, int H, int W, int pad,
                                                   int patch_h, int patch_w, int step_h, int step_w) {
   PatchGrid g;
   FwdPlan pl;
   if (!make_patch_grid(H, W, patch_h, patch_w, step_h, step_w, &g)) return 0;
-  if (!make_fwd_plan(device, B, K, g, pad, &pl)) return 0;
+  if (!make_fwd_plan(sm_count_cached(device), B, K, g, pad, &pl)) return 0;
   size_t bytes = (size_t)pl.n_patches * pl.slots_per_patch * pl.T * pl.T * K * K * sizeof(float);
   // the packed tensor-core joint (local_fwd_tcp.cu) keeps whole accumulator tiles per CTA slot
   const size_t tcp = local_joint_tcp_slot_floats(K, pad) * (size_t)pl.slots_per_patch * sizeof(float);
@@ -375,38 +398,13 @@ extern "C" size_t iic_local_joint_workspace_bytes(int device, int B, int K, int 
   return bytes;
 }
 
-namespace iic {
-int local_joint_tma_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                        long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                        float* partial, int max_ctas, int* ncta, cudaStream_t st);
-int local_joint_fast_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                         long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                         float* partial, int max_ctas, int* ncta, int* flags, int* checked, int from_logits,
-                         float inv_temp, cudaStream_t st);
-int local_joint_fast7_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                          long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                          float* partial, int max_ctas, int* ncta, cudaStream_t st);
-int local_joint_tc_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                       long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                       float* partial, int max_ctas, int* ncta, cudaStream_t st);
-size_t local_joint_tcp_slot_floats(int K, int pad);
-int local_joint_tcj10_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                          long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* partial, int max_ctas,
-                          int* ncta, int* flags, int* checked, int from_logits, float inv_temp, cudaStream_t st);
-int local_joint_tcp_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                        long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* partial,
-                        size_t partial_floats, double* J_out, SlotInfo* info, cudaStream_t st);
-}
-
-// info == nullptr: the per-CTA slots are reduced into J_out (fp64, fixed order) by a second launch.
-// info != nullptr: the slots are left in `workspace` and described in *info (for iic_finish); J_out is unused.
 static int local_joint_impl(const float* x, long long x_sn, long long x_sc, long long x_sh,
                             const float* y, long long y_sn, long long y_sc, long long y_sh,
                             const float* mask, long long m_sn, long long m_sc, long long m_sh,
                             int B, int K, int H, int W, int pad,
                             int patch_h, int patch_w, int step_h, int step_w,
                             double* J_out, void* workspace, size_t workspace_bytes, int* flags,
-                            SlotInfo* info, void* stream) {
+                            iic_slot_info* info, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   IIC_REQUIRE(x && y && (J_out || info), "iic_local_joint: null pointer");
   IIC_REQUIRE(!flags || x_sh == W, "iic_local_joint: the fused simplex assertion needs dense rows (x_sh == W)");
@@ -416,13 +414,14 @@ static int local_joint_impl(const float* x, long long x_sn, long long x_sc, long
   IIC_REQUIRE(make_patch_grid(H, W, patch_h, patch_w, step_h, step_w, &g),
               "iic_local_joint: bad patch geometry H=%d W=%d patch=(%d,%d) step=(%d,%d)", H, W, patch_h,
               patch_w, step_h, step_w);
-  const int device = current_device();
+  const int sms = sm_count_cached(current_device());
   FwdPlan pl;
-  IIC_REQUIRE(make_fwd_plan(device, B, K, g, pad, &pl), "iic_local_joint: cannot plan launch");
+  IIC_REQUIRE(make_fwd_plan(sms, B, K, g, pad, &pl), "iic_local_joint: cannot plan launch");
   const size_t E = (size_t)pl.T * pl.T * K * K;
   const size_t need = (size_t)pl.n_patches * pl.slots_per_patch * E * sizeof(float);
   IIC_REQUIRE(workspace && workspace_bytes >= need, "iic_local_joint: workspace too small (%zu < %zu)",
               workspace_bytes, need);
+  float* partial = (float*)workspace;
 
   // simplex assertion on x when the joint kernel chosen below cannot fuse it: one streaming pass
   auto simplex_pass = [&]() -> int {
@@ -430,60 +429,32 @@ static int local_joint_impl(const float* x, long long x_sn, long long x_sc, long
     return iic_simplex_check(x, B, K, (long long)H * W, x_sn, x_sc, flags, stream);
   };
 
-  // fast path: one patch, no mask, TMA-describable rows -> pipelined FFMA2 kernel (local_fwd_tma.cu)
+  // fast path: one patch, no mask, TMA-describable rows -> the specialised kernels (local_kernels.cuh)
   if (pl.n_patches == 1 && mask == nullptr && !options().no_tma) {
-    int ncta = 0, checked = 0;
+    const LocalMaps m{{x, x_sn, x_sc, x_sh}, {y, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
+    SlotInfo slots{};
+    int rc = -1, checked = 0;
     // the reference's default cluster count (16 <= K <= 24), padding 3: packed tensor-core joint (local_fwd_tcp.cu);
     // padding 1 stays on the FFMA2 kernel unless IIC_B200_TCP_P1 is set
-    if (!options().no_tc && (pad == 3 || options().tcp_p1)) {
-      const int rc_p = local_joint_tcp_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, (float*)workspace,
-                                           workspace_bytes / sizeof(float), J_out, info, st);
-      if (rc_p > 0) return rc_p;
-      if (rc_p == 0) return simplex_pass();
-    }
+    if (!options().no_tc && (pad == 3 || options().tcp_p1))
+      rc = local_joint_tcp_try(m, partial, workspace_bytes / sizeof(float), &slots, st);
     // wide cluster heads (K = 128): tcgen05 3xTF32 contraction (local_fwd_tc.cu)
-    if (!options().no_tc) {
-      const int rc_tc = local_joint_tc_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, (float*)workspace,
-                                           pl.slots_per_patch, &ncta, st);
-      if (rc_tc > 0) return rc_tc;
-      if (rc_tc == 0) {
-        if (int e = simplex_pass()) return e;
-        if (info) { *info = SlotInfo{SLOT_TC128, ncta, (long long)E, 0}; return 0; }
-        dim3 rgrid((unsigned)((E + 31) / 32), 1);
-        reduce_partials_kernel<true><<<rgrid, RED_GROUPS * 32, 0, st>>>((const float*)workspace, ncta, (long long)E, J_out);
-        IIC_CHECK_CUDA(cudaGetLastError());
-        return 0;
-      }
-    }
+    if (rc < 0 && !options().no_tc)
+      rc = local_joint_tc_try(m, partial, pl.slots_per_patch, &slots, st);
     // 10 clusters, 3 x 3 window, large maps (BASELINE config 2): fp16-split tensor-core joint (local_fwd_tcj10.cu)
-    int rc = -1;
-    if (!options().no_tc && !options().no_tcj10) {
-      const int sms = sm_count_cached(device);
-      if (sms > 0 && sms <= pl.slots_per_patch) {
-        rc = local_joint_tcj10_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, (float*)workspace, sms, &ncta,
-                                   flags, &checked, 0, 1.f, st);
-        if (rc == 0 && checked) flags = nullptr;
-      }
-    }
-    if (rc < 0)
-      rc = options().no_fast ? -1
-                 : local_joint_fast_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad,
-                                        (float*)workspace, pl.slots_per_patch, &ncta, flags, &checked, 0, 1.f, st);
-    if (rc == 0 && checked) flags = nullptr;       // done inside the joint kernel
+    if (rc < 0 && !options().no_tc && !options().no_tcj10 && sms <= pl.slots_per_patch)
+      rc = local_joint_tcj10_try(m, partial, sms, &slots, flags, &checked, 0, 1.f, st);
     if (rc < 0 && !options().no_fast)
-      rc = local_joint_fast7_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, (float*)workspace,
-                                 pl.slots_per_patch, &ncta, st);
+      rc = local_joint_fast_try(m, partial, pl.slots_per_patch, &slots, flags, &checked, 0, 1.f, st);
+    if (rc < 0 && !options().no_fast)
+      rc = local_joint_fast7_try(m, partial, pl.slots_per_patch, &slots, st);
     if (rc < 0)
-      rc = local_joint_tma_try(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad,
-                               (float*)workspace, pl.slots_per_patch, &ncta, st);
+      rc = local_joint_tma_try(m, partial, pl.slots_per_patch, &slots, st);
     if (rc > 0) return rc;
     if (rc == 0) {
+      if (checked) flags = nullptr;       // done inside the joint kernel
       if (int e = simplex_pass()) return e;
-      if (info) { *info = SlotInfo{SLOT_STD, ncta, (long long)E, 0}; return 0; }
-      dim3 rgrid((unsigned)((E + 31) / 32), 1);
-      reduce_partials_kernel<false><<<rgrid, RED_GROUPS * 32, 0, st>>>((const float*)workspace, ncta, (long long)E, J_out);
-      IIC_CHECK_CUDA(cudaGetLastError());
-      return 0;
+      return reduce_or_describe_slots(slots, partial, pl.T, K, 1, J_out, info, st);
     }
   }
 
@@ -495,7 +466,7 @@ static int local_joint_impl(const float* x, long long x_sn, long long x_sc, long
   P.B = B; P.K = K; P.pad = pad; P.g = g;
   P.TH = pl.TH; P.TWS = pl.TWS; P.tiles_h = pl.tiles_h; P.tiles_w = pl.tiles_w;
   P.XR = pl.XR; P.XP = pl.XP;
-  P.partial = (float*)workspace;
+  P.partial = partial;
   const int NDY = pl.T / pl.DYB;
   dim3 grid(pl.ctas_per_patch, pl.n_patches);
 
@@ -536,14 +507,8 @@ static int local_joint_impl(const float* x, long long x_sn, long long x_sc, long
       if (rc) return rc;
     }
   }
-  if (info) { *info = SlotInfo{SLOT_STD, pl.ctas_per_patch, (long long)E, 0}; return 0; }
-  {
-    dim3 rgrid((unsigned)((E + 31) / 32), pl.n_patches);
-    reduce_partials_kernel<false><<<rgrid, RED_GROUPS * 32, 0, st>>>((const float*)workspace, pl.ctas_per_patch,
-                                                             (long long)E, J_out);
-    IIC_CHECK_CUDA(cudaGetLastError());
-  }
-  return 0;
+  return reduce_or_describe_slots(SlotInfo{SLOT_STD, pl.ctas_per_patch, (long long)E, 0}, partial, pl.T, K,
+                                  pl.n_patches, J_out, info, st);
 }
 
 extern "C" int iic_local_joint(const float* x, long long x_sn, long long x_sc, long long x_sh,
@@ -566,16 +531,8 @@ extern "C" int iic_local_joint_partials(const float* x, long long x_sn, long lon
                                         void* workspace, size_t workspace_bytes, int* flags,
                                         iic_slot_info* info_host, void* stream) {
   IIC_REQUIRE(info_host, "iic_local_joint_partials: null pointer");
-  SlotInfo info{SLOT_STD, 0, 0, 0};
-  const int rc = local_joint_impl(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, mask, m_sn, m_sc, m_sh, B, K, H, W, pad,
-                                  patch_h, patch_w, step_h, step_w, nullptr, workspace, workspace_bytes, flags, &info,
-                                  stream);
-  if (rc) return rc;
-  info_host->layout = info.layout;
-  info_host->n_slots = info.n_slots;
-  info_host->slot_stride = info.slot_stride;
-  info_host->nb = info.nb;
-  return 0;
+  return local_joint_impl(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, mask, m_sn, m_sc, m_sh, B, K, H, W, pad, patch_h,
+                          patch_w, step_h, step_w, nullptr, workspace, workspace_bytes, flags, info_host, stream);
 }
 
 // Fused cluster-head softmax + local joint: only the shapes the fast kernel covers
@@ -587,37 +544,26 @@ extern "C" int iic_local_joint_from_logits(const float* lx, long long x_sn, long
   cudaStream_t st = (cudaStream_t)stream;
   IIC_REQUIRE(lx && ly && (J_out || info_host) && workspace, "iic_local_joint_from_logits: null pointer");
   IIC_REQUIRE(B > 0 && K > 0 && H > 0 && W > 0, "iic_local_joint_from_logits: empty input");
-  const int device = current_device();
-  const int sms = sm_count_cached(device);
+  const int sms = sm_count_cached(current_device());
   IIC_REQUIRE(sms > 0, "iic_local_joint_from_logits: no device");
   const size_t E = (size_t)9 * K * K;
   IIC_REQUIRE(workspace_bytes >= (size_t)sms * E * sizeof(float),
               "iic_local_joint_from_logits: workspace too small (%zu < %zu)", workspace_bytes,
               (size_t)sms * E * sizeof(float));
-  int ncta = 0, checked = 0;
+  const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
+  float* partial = (float*)workspace;
+  SlotInfo slots{};
+  int rc = -1, checked = 0;
   // large maps: the tensor-core joint with the softmax in its staging warps (csrc/local_fwd_tcj10.cu); else the FFMA2 kernel
-  int rc = -1;
   if (!options().no_tc && !options().no_tcj10 && pad == 1)
-    rc = local_joint_tcj10_try(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, (float*)workspace, sms, &ncta,
-                               nullptr, &checked, 1, inv_temperature, st);
+    rc = local_joint_tcj10_try(m, partial, sms, &slots, nullptr, &checked, 1, inv_temperature, st);
   if (rc < 0)
-    rc = local_joint_fast_try(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad,
-                              (float*)workspace, sms, &ncta, nullptr, &checked, 1, inv_temperature, st);
+    rc = local_joint_fast_try(m, partial, sms, &slots, nullptr, &checked, 1, inv_temperature, st);
   if (rc < 0) {
     set_error("iic_local_joint_from_logits: shape not covered by the fused kernel (needs padding 1, K == 10, "
               "W %% 4 == 0, 16-byte aligned rows); apply the softmax and call iic_local_joint");
     return IIC_UNSUPPORTED;
   }
   if (rc > 0) return rc;
-  if (info_host) {          // leave the slots for iic_finish
-    info_host->layout = SLOT_STD;
-    info_host->n_slots = ncta;
-    info_host->slot_stride = (long long)E;
-    info_host->nb = 0;
-    return 0;
-  }
-  dim3 rgrid((unsigned)((E + 31) / 32), 1);
-  reduce_partials_kernel<false><<<rgrid, RED_GROUPS * 32, 0, st>>>((const float*)workspace, ncta, (long long)E, J_out);
-  IIC_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  return reduce_or_describe_slots(slots, partial, 3, K, 1, J_out, info_host, st);
 }

@@ -18,6 +18,7 @@
 //   * K = 20, 30, ...: blockIdx.y selects the (x block, y block) pair, the tensor-map channel coordinate
 //     does the slicing.
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tma.cuh"
 
 namespace iic {
@@ -44,20 +45,14 @@ namespace iic {
 #undef IIC_FWD_NS
 #undef IIC_FWD_KB
 
-// 0 = launched, 1 = error, -1 = not eligible.  *ncta = number of partial slots written.
-// *checked = 1 when `flags` was given and the simplex assertion on x ran inside the kernel.
 // Channel blocks of 10 for the udaiic cluster counts (10, 20, ..), of 8 for other multiples of 8 (.., 128).
-int local_joint_fast_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                         long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                         float* partial, int max_ctas, int* ncta, int* flags, int* checked, int from_logits,
-                         float inv_temp, cudaStream_t st) {
+int local_joint_fast_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, int* flags, int* checked,
+                         int from_logits, float inv_temp, cudaStream_t st) {
   *checked = 0;
-  if (K % 10 == 0 && K <= 40)
-    return fwd3_kb10::local_joint_fast_try_kb(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, partial,
-                                              max_ctas, ncta, flags, checked, from_logits, inv_temp, st);
-  if (K % 8 == 0 && K <= 256 && !from_logits)
-    return fwd3_kb8::local_joint_fast_try_kb(x, x_sn, x_sc, x_sh, y, y_sn, y_sc, y_sh, B, K, H, W, pad, partial,
-                                             max_ctas, ncta, flags, checked, 0, 1.f, st);
+  if (m.K % 10 == 0 && m.K <= 40)
+    return fwd3_kb10::local_joint_fast_try_kb(m, partial, max_ctas, slots, flags, checked, from_logits, inv_temp, st);
+  if (m.K % 8 == 0 && m.K <= 256 && !from_logits)
+    return fwd3_kb8::local_joint_fast_try_kb(m, partial, max_ctas, slots, flags, checked, 0, 1.f, st);
   return -1;
 }
 
@@ -218,15 +213,14 @@ local_joint_fast7_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_
 }
 
 // 7 x 7 counterpart of local_joint_fast_try (probability inputs only)
-int local_joint_fast7_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                          long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                          float* partial, int max_ctas, int* ncta, cudaStream_t st) {
+int local_joint_fast7_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st) {
   using namespace fwdfast7;
-  if (pad != PAD || K < KB || K % KB != 0 || K > 20) return -1;
+  const int B = m.B, K = m.K, H = m.H, W = m.W;
+  if (m.pad != PAD || K < KB || K % KB != 0 || K > 20) return -1;
   if (W % 4 != 0) return -1;
   CUtensorMap mx, my;
-  if (!make_map_4d(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, XP, TH, KB)) return -1;
-  if (!make_map_4d(&my, y, B, K, H, W, y_sn, y_sc, y_sh, TW, TH, KB)) return -1;
+  if (!make_map_4d(&mx, m.x, m, XP, TH, KB)) return -1;
+  if (!make_map_4d(&my, m.y, m, TW, TH, KB)) return -1;
   FwdFastParams P;
   P.B = B; P.K = K; P.H = H; P.W = W;
   P.flags = nullptr; P.inv_temp = 1.f;
@@ -238,7 +232,7 @@ int local_joint_fast7_try(const float* x, long long x_sn, long long x_sc, long l
   int gx = max_ctas / ny;
   if (gx < 1) gx = 1;
   if (gx > items) gx = (int)items;
-  *ncta = gx;
+  *slots = SlotInfo{SLOT_STD, gx, (long long)T * T * K * K, 0};
   IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_fast7_kernel), (int)((int)(STAGES * STAGE_BYTES))));
   local_joint_fast7_kernel<<<dim3(gx, ny), NTHREADS, STAGES * STAGE_BYTES, st>>>(mx, my, P);
   IIC_CHECK_CUDA(cudaGetLastError());

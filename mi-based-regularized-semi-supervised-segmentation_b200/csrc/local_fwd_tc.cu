@@ -28,6 +28,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -280,36 +281,17 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
   if (wid == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
 }
 
-static bool make_map(CUtensorMap* map, const float* base, int B, int H, int W, long long sn, long long sc, long long sh,
-                     int box_w, CUtensorMapSwizzle swz) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
-  if ((sh * 4) % 16 != 0 || (sc * 4) % 16 != 0 || (sn * 4) % 16 != 0) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)KC, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-  cuuint32_t box[4] = {(cuuint32_t)box_w, 1, (cuuint32_t)KC, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace fwdtc
 
-// Returns 0 when launched, < 0 when the shape is not covered (the caller falls back to the FFMA2 kernels), > 0 on error.
-int local_joint_tc_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                       long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* partial, int max_ctas,
-                       int* ncta, cudaStream_t st) {
+int local_joint_tc_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st) {
   using namespace fwdtc;
-  if (K != KC || pad != 1 || W % PXB != 0 || max_ctas < 1) return -1;
+  const int B = m.B, H = m.H, W = m.W;
+  if (m.K != KC || m.pad != 1 || W % PXB != 0 || max_ctas < 1) return -1;
   CUtensorMap mx, my;
-  if (!make_map(&mx, x, B, H, W, x_sn, x_sc, x_sh, XRW, CU_TENSOR_MAP_SWIZZLE_NONE)) return -1;
-  if (!make_map(&my, y, B, H, W, y_sn, y_sc, y_sh, PXB, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
-  const int sms = sm_count_cached(current_device());
-  if (sms <= 0) return -1;
+  if (!make_map_4d(&mx, m.x, m, XRW, 1, KC)) return -1;
+  if (!make_map_4d(&my, m.y, m, PXB, 1, KC, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
   const long long nkb = (long long)B * H * (W / PXB);
-  int gx = sms / 3;                                   // three displacement rows per share of the pixels
+  int gx = m.sms / 3;                                 // three displacement rows per share of the pixels
   if (gx > max_ctas) gx = max_ctas;
   if (gx > nkb) gx = (int)nkb;
   if (gx < 1) gx = 1;
@@ -318,7 +300,7 @@ int local_joint_tc_try(const float* x, long long x_sn, long long x_sc, long long
            tc::bringup_env("IIC_TC_DBG", 0)};
   local_joint_tc_kernel<<<dim3(gx, 3), NTHREADS, SMEM_BYTES, st>>>(mx, my, P);
   IIC_CHECK_CUDA(cudaGetLastError());
-  *ncta = gx;
+  *slots = SlotInfo{SLOT_TC128, gx, (long long)9 * KC * KC, 0};
   return 0;
 }
 

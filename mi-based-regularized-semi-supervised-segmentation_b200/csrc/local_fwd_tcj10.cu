@@ -23,6 +23,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -428,34 +429,33 @@ __global__ void __launch_bounds__(NTHREADS, 1) local_joint_tcj10_kernel(const Pa
 
 }  // namespace fwdtcj10
 
-// 0 = launched, 1 = error, -1 = not eligible.  *ncta = number of partial slots written ([9][K][K] floats each).
-// *checked = 1 when `flags` was given and the simplex assertion on x ran inside the kernel.
-int local_joint_tcj10_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                          long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* partial, int max_ctas,
-                          int* ncta, int* flags, int* checked, int from_logits, float inv_temp, cudaStream_t st) {
+// One slot of [9][K][K] floats per CTA.
+int local_joint_tcj10_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, int* flags, int* checked,
+                          int from_logits, float inv_temp, cudaStream_t st) {
   using namespace fwdtcj10;
+  const int B = m.B, K = m.K, H = m.H, W = m.W;
   *checked = 0;
-  if (pad != PAD || K < 2 || K > 10 || W < 8 || W > MAXW) return -1;
+  if (m.pad != PAD || K < 2 || K > 10 || W < 8 || W > MAXW) return -1;
   if (from_logits && K != 10) return -1;           // the fused forward takes exactly the shapes every fused backward takes
   const long long rows = (long long)B * H;
   if (rows < 8LL * max_ctas) return -1;            // small maps: the pipeline fill dominates, the FFMA2 kernel is faster
   Params P;
-  P.x = x; P.x_sn = x_sn; P.x_sc = x_sc; P.x_sh = x_sh;
-  P.y = y; P.y_sn = y_sn; P.y_sc = y_sc; P.y_sh = y_sh;
+  P.x = m.x.p; P.x_sn = m.x.sn; P.x_sc = m.x.sc; P.x_sh = m.x.sh;
+  P.y = m.y.p; P.y_sn = m.y.sn; P.y_sc = m.y.sc; P.y_sh = m.y.sh;
   P.B = B; P.H = H; P.W = W; P.K = K;
   P.partial = partial;
   P.flags = from_logits ? nullptr : flags;      // a softmax output needs no simplex assertion
   P.from_logits = from_logits;
   P.inv_temp = inv_temp;
-  auto rows16 = [&](const float* b, long long sn, long long sc, long long sh) {
-    return (reinterpret_cast<uintptr_t>(b) & 15) == 0 && sn % 4 == 0 && sc % 4 == 0 && sh % 4 == 0;
+  auto rows16 = [&](const View4& v) {
+    return (reinterpret_cast<uintptr_t>(v.p) & 15) == 0 && v.sn % 4 == 0 && v.sc % 4 == 0 && v.sh % 4 == 0;
   };
-  if (W % 4 != 0 || !rows16(x, x_sn, x_sc, x_sh) || !rows16(y, y_sn, y_sc, y_sh)) return -1;     // 16-byte loads
+  if (W % 4 != 0 || !rows16(m.x) || !rows16(m.y)) return -1;     // 16-byte loads
 #ifdef IIC_TCJ_DEBUG
   P.dbg = 0;
 #endif
   *checked = P.flags != nullptr;
-  *ncta = max_ctas;
+  *slots = SlotInfo{SLOT_STD, max_ctas, (long long)9 * K * K, 0};
   IIC_CHECK_RC(ensure_dyn_smem((const void*)local_joint_tcj10_kernel, SMEM_BYTES));
   local_joint_tcj10_kernel<<<max_ctas, NTHREADS, SMEM_BYTES, st>>>(P);
   IIC_CHECK_CUDA(cudaGetLastError());

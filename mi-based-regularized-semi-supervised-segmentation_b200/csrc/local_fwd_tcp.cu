@@ -20,6 +20,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tc_common.cuh"
 #include "tma.cuh"
 
@@ -297,21 +298,6 @@ reduce_packed_kernel(const float* __restrict__ partial, int ncta, int slot_float
   }
 }
 
-static bool make_map(CUtensorMap* map, const float* base, int B, int K, int H, int W, long long sn, long long sc, long long sh,
-                     int box_w, int box_h, CUtensorMapSwizzle swz) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
-  if ((sh * 4) % 16 != 0 || (sc * 4) % 16 != 0 || (sn * 4) % 16 != 0) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)K, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-  cuuint32_t box[4] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)KPC, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <int T>
 static int launch(const CUtensorMap& mx, const CUtensorMap& my, const Params& P, int grid, size_t smem, cudaStream_t st) {
   IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tcp_kernel<T>), (int)(SMEM_LIMIT)));
@@ -322,29 +308,24 @@ static int launch(const CUtensorMap& mx, const CUtensorMap& my, const Params& P,
 
 }  // namespace fwdtcp
 
-// floats of one CTA slot of the packed kernel (0 when the shape is not covered); iic_local_joint_workspace_bytes sizes for it
 size_t local_joint_tcp_slot_floats(int K, int pad) {
   if (K < 16 || K > 24 || (pad != 1 && pad != 3)) return 0;
   const int T = 2 * pad + 1;
   return (size_t)((T * K + 127) / 128) * 128 * (T * fwdtcp::KPC);
 }
 
-// Returns 0 when launched (J_out written), < 0 when the shape is not covered, > 0 on error.
-int local_joint_tcp_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y, long long y_sn,
-                        long long y_sc, long long y_sh, int B, int K, int H, int W, int pad, float* partial,
-                        size_t partial_floats, double* J_out, SlotInfo* info, cudaStream_t st) {
+int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_floats, SlotInfo* slots, cudaStream_t st) {
   using namespace fwdtcp;
-  const size_t slot_floats = local_joint_tcp_slot_floats(K, pad);
+  const int B = m.B, K = m.K, H = m.H, W = m.W;
+  const size_t slot_floats = local_joint_tcp_slot_floats(K, m.pad);
   if (slot_floats == 0 || W % PXB != 0) return -1;
-  const int T = 2 * pad + 1;
+  const int T = 2 * m.pad + 1;
   const int nmt = (T * K + 127) / 128, nb = T * KPC;
   CUtensorMap mx, my;
-  if (!make_map(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, XRW, 1, CU_TENSOR_MAP_SWIZZLE_NONE)) return -1;
-  if (!make_map(&my, y, B, K, H, W, y_sn, y_sc, y_sh, PXB, T, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
-  const int sms = sm_count_cached(current_device());
-  if (sms <= 0) return -1;
+  if (!make_map_4d(&mx, m.x, m, XRW, 1, KPC)) return -1;
+  if (!make_map_4d(&my, m.y, m, PXB, T, KPC, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
   const long long nkb = (long long)B * H * (W / PXB);
-  long long grid = sms;
+  long long grid = m.sms;
   if ((long long)(partial_floats / slot_floats) < grid) grid = (long long)(partial_floats / slot_floats);
   if (grid > nkb) grid = nkb;
   if (grid < 1) return -1;
@@ -360,10 +341,7 @@ int local_joint_tcp_try(const float* x, long long x_sn, long long x_sc, long lon
            tc::bringup_env("IIC_TC_DBG", 0), partial};
   const int rc = T == 3 ? launch<3>(mx, my, P, (int)grid, smem, st) : launch<7>(mx, my, P, (int)grid, smem, st);
   if (rc) return rc;
-  if (info) { *info = SlotInfo{SLOT_PACKED, (int)grid, (long long)slot_floats, nb}; return 0; }
-  const int E = T * T * K * K;
-  reduce_packed_kernel<<<(E + 31) / 32, 1024, 0, st>>>(partial, (int)grid, (int)slot_floats, T, K, nb, J_out);
-  IIC_CHECK_CUDA(cudaGetLastError());
+  *slots = SlotInfo{SLOT_PACKED, (int)grid, (long long)slot_floats, nb};
   return 0;
 }
 

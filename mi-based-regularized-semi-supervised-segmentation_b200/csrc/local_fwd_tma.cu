@@ -6,6 +6,7 @@
 //   * packed FP32: accumulators are float2 pairs over two x channels (i0, i0+1) and every update is one
 //     fma.rn.f32x2 (FFMA2), halving the FMA issue slots so the loads and address math fit beside them.
 #include "common.cuh"
+#include "local_kernels.cuh"
 #include "tma.cuh"
 
 namespace iic {
@@ -199,11 +200,8 @@ static int launch_fwd_tma(const CUtensorMap& mx, const CUtensorMap& my, const Fw
 
 static int jt_for(int T) { return T == 1 ? 8 : T == 3 ? 5 : T == 5 ? 2 : 1; }
 
-// Returns 0 when the TMA kernel was launched, 1 on error, -1 when this case is not eligible (caller
-// falls back to the generic kernel).  *ncta receives the number of per-CTA partial slots written.
-int local_joint_tma_try(const float* x, long long x_sn, long long x_sc, long long x_sh, const float* y,
-                        long long y_sn, long long y_sc, long long y_sh, int B, int K, int H, int W, int pad,
-                        float* partial, int max_ctas, int* ncta, cudaStream_t st) {
+int local_joint_tma_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st) {
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad;
   const int T = 2 * pad + 1;
   if (T > 5 || K > 32 || K < 1) return -1;     // T = 7 keeps the generic kernel (register budget)
   if (W % 4 != 0) return -1;
@@ -255,13 +253,13 @@ int local_joint_tma_try(const float* x, long long x_sn, long long x_sc, long lon
   P.partial = partial;
 
   CUtensorMap mx, my;
-  if (!make_map_4d(&mx, x, B, K, H, W, x_sn, x_sc, x_sh, P.XP, P.XR, K)) return -1;
-  if (!make_map_4d(&my, y, B, K, H, W, y_sn, y_sc, y_sh, TW, TH, K)) return -1;
+  if (!make_map_4d(&mx, m.x, m, P.XP, P.XR, K)) return -1;
+  if (!make_map_4d(&my, m.y, m, TW, TH, K)) return -1;
 
   long long items = (long long)B * P.tiles_h * P.tiles_w;
   int grid = max_ctas;
   if (grid > items) grid = (int)items;
-  *ncta = grid;
+  *slots = SlotInfo{SLOT_STD, grid, (long long)T * T * K * K, 0};
   const size_t smem = (size_t)sb * FWD_STAGES;
   int rc;
   switch (T) {

@@ -28,11 +28,13 @@ inline EncodeTiledFn get_encode_tiled() {
 }
 
 // A (B, K, H, W) float32 tensor with element strides (sn, sc, sh, 1) as a rank-4 tensor map with
-// box (box_w, box_h, box_c, 1); out-of-range elements are filled with zeros (which is exactly the
-// zero padding of the F.conv2d at iic_loss.py:123).  Returns false when the tensor cannot be described
-// (unaligned base or strides) -- the caller then uses the non-TMA kernel.
+// box (box_w, box_h, box_c, 1), written to shared memory with swizzle `swz`; out-of-range elements are
+// filled with zeros (which is exactly the zero padding of the F.conv2d at iic_loss.py:123).  Returns false
+// when the tensor cannot be described (unaligned base or strides, box too large) -- the caller then uses
+// another kernel.
 inline bool make_map_4d(CUtensorMap* map, const float* base, int B, int K, int H, int W, long long sn,
-                        long long sc, long long sh, int box_w, int box_h, int box_c) {
+                        long long sc, long long sh, int box_w, int box_h, int box_c,
+                        CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_NONE) {
   EncodeTiledFn enc = get_encode_tiled();
   if (!enc) return false;
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return false;
@@ -43,7 +45,7 @@ inline bool make_map_4d(CUtensorMap* map, const float* base, int B, int K, int H
   cuuint32_t box[4] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)box_c, 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
   CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS;
 }

@@ -1,21 +1,12 @@
 // Stand-alone harness for the row-block tcgen05 backward sweeps at K = 9 or 10, padding 1 (csrc/local_bwd_tcrb10.cu): random source
 // maps and random coefficient tensors, a sample of output pixels checked against an fp64 CPU loop.
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_bwdrb10 tools/tc_bwdrb10_harness.cu
-//   tools/_bin/tc_bwdrb [B H W K pad]
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_bwdrb10 tools/tc_bwdrb10_harness.cu mi-based-regularized-semi-supervised-segmentation_b200/csrc/runtime.cu
+//   tools/_bin/tc_bwdrb10 [B H W K pad]
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
-#include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/common.cuh"
-namespace iic {
-static thread_local char g_err[512] = "";
-void set_error(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap); }
-const char* get_error() { return g_err; }
-int current_device() { return 0; }
-int sm_count_cached(int) { return 148; }
-}
 #include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/local_bwd_tcrb10.cu"
 
 int main(int argc, char** argv) {
@@ -43,14 +34,17 @@ int main(int argc, char** argv) {
   cudaMemcpy(dg, &g, 4, cudaMemcpyHostToDevice);
   cudaMemset(dgx, 0xff, n * 4); cudaMemset(dgy, 0xff, n * 4);
   const long long sc = (long long)H * W, sn = sc * KC;
-  int rc = iic::local_bwd_tcrb10_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dwx, dwy, dg, dgx, dgy, 0);
+  const iic::LocalMaps m{{dx_, sn, sc, W}, {dy_, sn, sc, W}, B, KC, H, W, pad, iic::sm_count_cached(iic::current_device())};
+  const iic::LocalGrads gr{dg, dgx, dgy, sn, sn};
+  iic_b200_set_option("tc10_force", 1);     // the kernel at any shape: skip the dispatcher's size rule
+  int rc = iic::local_bwd_tcrb10_try(m, dwx, dwy, gr, 0);
   cudaError_t err = cudaDeviceSynchronize();
   printf("try rc=%d (%s); first launch: %s\n", rc, iic::get_error(), cudaGetErrorString(err));
   if (rc != 0 || err != cudaSuccess) return 1;
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   const int reps = 3;
   cudaEventRecord(e0);
-  for (int r = 0; r < reps; ++r) iic::local_bwd_tcrb10_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dwx, dwy, dg, dgx, dgy, 0);
+  for (int r = 0; r < reps; ++r) iic::local_bwd_tcrb10_try(m, dwx, dwy, gr, 0);
   cudaEventRecord(e1);
   err = cudaDeviceSynchronize();
   if (err != cudaSuccess) { printf("timed launches: %s\n", cudaGetErrorString(err)); return 1; }

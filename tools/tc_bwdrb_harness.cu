@@ -1,21 +1,12 @@
 // Stand-alone harness for the row-block tcgen05 backward sweeps at 16 <= K <= 24, padding 1 or 3 (csrc/local_bwd_tcrb.cu): random source
 // maps and random coefficient tensors, a sample of output pixels checked against an fp64 CPU loop.
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_bwdrb tools/tc_bwdrb_harness.cu
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_bwdrb tools/tc_bwdrb_harness.cu mi-based-regularized-semi-supervised-segmentation_b200/csrc/runtime.cu
 //   tools/_bin/tc_bwdrb [B H W K pad]
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
-#include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/common.cuh"
-namespace iic {
-static thread_local char g_err[512] = "";
-void set_error(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap); }
-const char* get_error() { return g_err; }
-int current_device() { return 0; }
-int sm_count_cached(int) { return 148; }
-}
 #include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/local_bwd_tcrb.cu"
 
 int main(int argc, char** argv) {
@@ -34,7 +25,9 @@ int main(int argc, char** argv) {
   for (size_t i = 0; i < nw; ++i) { hwx[i] = (float)rand() / RAND_MAX - 0.4f; hwy[i] = (float)rand() / RAND_MAX - 0.6f; }
   float *dx_, *dy_, *dwx, *dwy, *dgx, *dgy, *dg;
   cudaMalloc(&dx_, n * 4); cudaMalloc(&dy_, n * 4); cudaMalloc(&dgx, n * 4); cudaMalloc(&dgy, n * 4);
-  cudaMalloc(&dwx, nw * 4); cudaMalloc(&dwy, nw * 4); cudaMalloc(&dg, 4);
+  // coefficient buffers as iic_local_coeff_floats sizes them: the kernel writes its weight image into their tail
+  const size_t nwbuf = iic::local_coeff_image_offset(KC, pad, 1) + iic::local_bwd_tcrb_image_bytes(KC, pad) / 4;
+  cudaMalloc(&dwx, nwbuf * 4); cudaMalloc(&dwy, nwbuf * 4); cudaMalloc(&dg, 4);
   cudaMemcpy(dx_, hx.data(), n * 4, cudaMemcpyHostToDevice);
   cudaMemcpy(dy_, hy.data(), n * 4, cudaMemcpyHostToDevice);
   cudaMemcpy(dwx, hwx.data(), nw * 4, cudaMemcpyHostToDevice);
@@ -43,14 +36,17 @@ int main(int argc, char** argv) {
   cudaMemcpy(dg, &g, 4, cudaMemcpyHostToDevice);
   cudaMemset(dgx, 0xff, n * 4); cudaMemset(dgy, 0xff, n * 4);
   const long long sc = (long long)H * W, sn = sc * KC;
-  int rc = iic::local_bwd_tcrb_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dwx, dwy, dg, dgx, dgy, 0);
+  const iic::LocalMaps m{{dx_, sn, sc, W}, {dy_, sn, sc, W}, B, KC, H, W, pad, iic::sm_count_cached(iic::current_device())};
+  const iic::LocalGrads gr{dg, dgx, dgy, sn, sn};
+  iic_b200_set_option("tcrb_p1", 1);     // the kernel at any shape: skip the dispatcher's size rule
+  int rc = iic::local_bwd_tcrb_try(m, dwx, dwy, gr, 0);
   cudaError_t err = cudaDeviceSynchronize();
   printf("try rc=%d (%s); first launch: %s\n", rc, iic::get_error(), cudaGetErrorString(err));
   if (rc != 0 || err != cudaSuccess) return 1;
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   const int reps = 3;
   cudaEventRecord(e0);
-  for (int r = 0; r < reps; ++r) iic::local_bwd_tcrb_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dwx, dwy, dg, dgx, dgy, 0);
+  for (int r = 0; r < reps; ++r) iic::local_bwd_tcrb_try(m, dwx, dwy, gr, 0);
   cudaEventRecord(e1);
   err = cudaDeviceSynchronize();
   if (err != cudaSuccess) { printf("timed launches: %s\n", cudaGetErrorString(err)); return 1; }

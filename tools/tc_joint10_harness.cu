@@ -1,24 +1,12 @@
 // Stand-alone timing harness for the fp16-split tensor-core joint (csrc/local_fwd_tcj10.cu): the kernel alone, and with
 // one pipeline stage switched off at a time (which stage bounds the row rate).
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -DIIC_TCJ_DEBUG -lcuda -o tools/_bin/tc_joint10 tools/tc_joint10_harness.cu
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -DIIC_TCJ_DEBUG -o tools/_bin/tc_joint10 tools/tc_joint10_harness.cu mi-based-regularized-semi-supervised-segmentation_b200/csrc/runtime.cu
 //   tools/_bin/tc_joint10 [B H W K]
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
-#include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/common.cuh"
-namespace iic {
-static thread_local char g_err[512] = "";
-void set_error(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap); }
-const char* get_error() { return g_err; }
-int current_device() { return 0; }
-int sm_count_cached(int) { return 148; }
-static Options g_opt;
-const Options& options() { return g_opt; }
-int ensure_dyn_smem(const void* f, int bytes) { return cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess ? 0 : 1; }
-}
 #include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/local_fwd_tcj10.cu"
 
 int main(int argc, char** argv) {
@@ -28,8 +16,9 @@ int main(int argc, char** argv) {
   std::vector<float> h(n);
   srand(3);
   for (size_t i = 0; i < n; ++i) h[i] = (float)rand() / RAND_MAX / K * 2.f;
+  const int sms = iic::sm_count_cached(iic::current_device());
   float *dx_, *dy_, *part;
-  cudaMalloc(&dx_, n * 4); cudaMalloc(&dy_, n * 4); cudaMalloc(&part, (size_t)148 * 9 * K * K * 4);
+  cudaMalloc(&dx_, n * 4); cudaMalloc(&dy_, n * 4); cudaMalloc(&part, (size_t)sms * 9 * K * K * 4);
   cudaMemcpy(dx_, h.data(), n * 4, cudaMemcpyHostToDevice);
   cudaMemcpy(dy_, h.data(), n * 4, cudaMemcpyHostToDevice);
   using namespace iic;
@@ -42,12 +31,12 @@ int main(int argc, char** argv) {
     P.x = dx_; P.x_sn = sn; P.x_sc = sc; P.x_sh = W;
     P.y = dy_; P.y_sn = sn; P.y_sc = sc; P.y_sh = W;
     P.B = B; P.H = H; P.W = W; P.K = K; P.partial = part; P.flags = nullptr; P.from_logits = 0; P.inv_temp = 1.f; P.dbg = m;
-    local_joint_tcj10_kernel<<<148, NTHREADS, SMEM_BYTES>>>(P);
+    local_joint_tcj10_kernel<<<sms, NTHREADS, SMEM_BYTES>>>(P);
     cudaError_t err = cudaDeviceSynchronize();
     if (err != cudaSuccess) { printf("mode %d: %s\n", m, cudaGetErrorString(err)); return 1; }
     const int reps = 5;
     cudaEventRecord(e0);
-    for (int r = 0; r < reps; ++r) local_joint_tcj10_kernel<<<148, NTHREADS, SMEM_BYTES>>>(P);
+    for (int r = 0; r < reps; ++r) local_joint_tcj10_kernel<<<sms, NTHREADS, SMEM_BYTES>>>(P);
     cudaEventRecord(e1);
     cudaDeviceSynchronize();
     float ms; cudaEventElapsedTime(&ms, e0, e1);
@@ -64,9 +53,9 @@ int main(int argc, char** argv) {
       static unsigned long long ct[160][2];
       cudaMemcpyFromSymbol(ct, g_tcj_cta, sizeof(ct));
       unsigned long long t0 = ~0ull, t1 = 0;
-      for (int i = 0; i < 148; ++i) { if (ct[i][0] < t0) t0 = ct[i][0]; if (ct[i][1] > t1) t1 = ct[i][1]; }
+      for (int i = 0; i < sms; ++i) { if (ct[i][0] < t0) t0 = ct[i][0]; if (ct[i][1] > t1) t1 = ct[i][1]; }
       printf("  last launch: first CTA start to last CTA end %.1f us; per CTA (start offset, duration) us:\n   ", (t1 - t0) * 1e-3);
-      if (0) for (int i = 0; i < 148; ++i) { printf(" %d:(%.1f,%.1f)", i, (ct[i][0] - t0) * 1e-3, (ct[i][1] - ct[i][0]) * 1e-3); if (i % 8 == 7) printf("\n   "); }
+      if (0) for (int i = 0; i < sms; ++i) { printf(" %d:(%.1f,%.1f)", i, (ct[i][0] - t0) * 1e-3, (ct[i][1] - ct[i][0]) * 1e-3); if (i % 8 == 7) printf("\n   "); }
       printf("\n");
     }
     printf("mode %d (%s%s%s%s): %.1f us\n", m, m & 1 ? "no-mma " : "", m & 2 ? "no-transform " : "", m & 4 ? "no-l2-prefetch " : "", m & 8 ? "no-loads" : "", ms / reps * 1e3);

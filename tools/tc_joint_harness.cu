@@ -1,22 +1,13 @@
 // Stand-alone harness for the tcgen05 (UMMA) local joint at K = 128 clusters, 3 x 3 window (csrc/local_fwd_tc.cu):
 // runs the kernel on random simplex-like maps, adds the per-CTA slots in fp64 and compares a sample of entries with
 // an fp64 CPU loop; prints the time per launch and the fp32-equivalent TFLOP/s.
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_joint tools/tc_joint_harness.cu
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_joint tools/tc_joint_harness.cu mi-based-regularized-semi-supervised-segmentation_b200/csrc/runtime.cu
 //   tools/_bin/tc_joint [B H W]
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
-#include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/common.cuh"
-namespace iic {
-static thread_local char g_err[512] = "";
-void set_error(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap); }
-const char* get_error() { return g_err; }
-int current_device() { return 0; }
-int sm_count_cached(int) { return 148; }
-}
 #include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/local_fwd_tc.cu"
 
 int main(int argc, char** argv) {
@@ -39,16 +30,18 @@ int main(int argc, char** argv) {
   const size_t E = (size_t)9 * KC * KC;
   cudaMalloc(&dout, 49 * E * 4);
   cudaMemset(dout, 0xff, 49 * E * 4);
-  int ncta = 0;
   const long long sc = (long long)H * W, sn = sc * KC;
-  int rc = iic::local_joint_tc_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, 1, dout, 49, &ncta, 0);
+  const iic::LocalMaps m{{dx_, sn, sc, W}, {dy_, sn, sc, W}, B, KC, H, W, 1, iic::sm_count_cached(iic::current_device())};
+  iic::SlotInfo slots{};
+  int rc = iic::local_joint_tc_try(m, dout, 49, &slots, 0);
+  const int ncta = slots.n_slots;
   cudaError_t err = cudaDeviceSynchronize();
   printf("try rc=%d ncta=%d (%s); first launch: %s\n", rc, ncta, iic::get_error(), cudaGetErrorString(err));
   if (rc != 0 || err != cudaSuccess) return 1;
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   const int reps = 5;
   cudaEventRecord(e0);
-  for (int r = 0; r < reps; ++r) iic::local_joint_tc_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, 1, dout, 49, &ncta, 0);
+  for (int r = 0; r < reps; ++r) iic::local_joint_tc_try(m, dout, 49, &slots, 0);
   cudaEventRecord(e1);
   err = cudaDeviceSynchronize();
   if (err != cudaSuccess) { printf("timed launches: %s\n", cudaGetErrorString(err)); return 1; }

@@ -1,22 +1,13 @@
 // Stand-alone harness for the packed tcgen05 local joint at 16 <= K <= 24, padding 1 or 3 (csrc/local_fwd_tcp.cu):
 // runs the kernel on random simplex-like maps, adds the per-CTA slots in fp64 and compares a sample of entries with
 // an fp64 CPU loop; prints the time per launch and the fp32-equivalent TFLOP/s.
-//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_jointp tools/tc_jointp_harness.cu
+//   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o tools/_bin/tc_jointp tools/tc_jointp_harness.cu mi-based-regularized-semi-supervised-segmentation_b200/csrc/runtime.cu
 //   tools/_bin/tc_jointp [B H W K pad]
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
-#include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/common.cuh"
-namespace iic {
-static thread_local char g_err[512] = "";
-void set_error(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap); }
-const char* get_error() { return g_err; }
-int current_device() { return 0; }
-int sm_count_cached(int) { return 148; }
-}
 #include "../mi-based-regularized-semi-supervised-segmentation_b200/csrc/local_fwd_tcp.cu"
 
 int main(int argc, char** argv) {
@@ -38,19 +29,28 @@ int main(int argc, char** argv) {
   cudaMemcpy(dx_, hx.data(), n * 4, cudaMemcpyHostToDevice);
   cudaMemcpy(dy_, hy.data(), n * 4, cudaMemcpyHostToDevice);
   const size_t E = (size_t)T * T * KC * KC;
-  const size_t wsf = iic::local_joint_tcp_slot_floats(KC, pad) * 148;
+  const int sms = iic::sm_count_cached(iic::current_device());
+  const size_t wsf = iic::local_joint_tcp_slot_floats(KC, pad) * sms;
   cudaMalloc(&dws, wsf * 4);
   cudaMemset(dws, 0xff, wsf * 4);
   cudaMalloc(&dJ, E * 8);
   const long long sc = (long long)H * W, sn = sc * KC;
-  int rc = iic::local_joint_tcp_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dws, wsf, dJ, 0);
+  const iic::LocalMaps m{{dx_, sn, sc, W}, {dy_, sn, sc, W}, B, KC, H, W, pad, sms};
+  auto run = [&]() {           // the joint, then the slot reduce of iic_local_joint
+    iic::SlotInfo s{};
+    const int rc = iic::local_joint_tcp_try(m, dws, wsf, &s, 0);
+    if (rc == 0)
+      iic::fwdtcp::reduce_packed_kernel<<<(int)((E + 31) / 32), 1024>>>(dws, s.n_slots, (int)s.slot_stride, T, KC, s.nb, dJ);
+    return rc;
+  };
+  int rc = run();
   cudaError_t err = cudaDeviceSynchronize();
   printf("try rc=%d (%s); first launch: %s\n", rc, iic::get_error(), cudaGetErrorString(err));
   if (rc != 0 || err != cudaSuccess) return 1;
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   const int reps = 5;
   cudaEventRecord(e0);
-  for (int r = 0; r < reps; ++r) iic::local_joint_tcp_try(dx_, sn, sc, W, dy_, sn, sc, W, B, KC, H, W, pad, dws, wsf, dJ, 0);
+  for (int r = 0; r < reps; ++r) run();
   cudaEventRecord(e1);
   err = cudaDeviceSynchronize();
   if (err != cudaSuccess) { printf("timed launches: %s\n", cudaGetErrorString(err)); return 1; }
