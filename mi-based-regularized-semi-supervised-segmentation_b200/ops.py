@@ -8,6 +8,7 @@ The mathematical contract of each op (reference file:line) is stated in include/
 """
 from __future__ import annotations
 
+import math
 from typing import Optional, Tuple
 
 import torch
@@ -882,12 +883,29 @@ def _block_view(G: torch.Tensor, like: torch.Tensor, n0: int, c0: int) -> torch.
     return G.view(N, -1)[n0:n0 + B, c0:c0 + K]
 
 
+def _region(v: torch.Tensor, blk, src: torch.Tensor):
+    """The part of `src` that the use `v` (block `blk` = (n0, c0) of it, or None = all of it) covers, as
+    (first row, end row, first element, end element) with elements counted inside one row of `src`."""
+    N = src.shape[0]
+    if blk is None:
+        return (0, N, 0, src.numel() // N if N else 0)
+    B, K = v.shape[:2]
+    plane = math.prod(v.shape[2:])
+    return (blk[0], blk[0] + B, blk[1] * plane, (blk[1] + K) * plane)
+
+
+def _intersect(a, b) -> bool:
+    return (a[0] < a[1] and a[2] < a[3] and b[0] < b[1] and b[2] < b[3]
+            and a[0] < b[1] and b[0] < a[1] and a[2] < b[3] and b[2] < a[3])
+
+
 class IICTermsFunction(torch.autograd.Function):
     """The losses of one or many IIC terms -- local (iic_loss.py:107-149,171-186) and global (iic_loss.py:43-94) -- from
     ONE finish launch.  apply(terms, check_simplex, slots, *sources): `terms` carries geometry and the input views,
     `sources` the distinct differentiable tensors behind them, `slots[2*i]`, `slots[2*i+1]` = (source index, block or
     None) for x and y of term i.  Outputs per local term: loss; per global term: loss, loss_no_lamb, P.  In backward
-    every term's gradient kernel writes directly into its block of the source's gradient."""
+    every term's gradient kernel writes directly into its block of the source's gradient -- or into a temporary that is
+    added to the block, when the same block was written before or when the source's regions overlap."""
 
     @staticmethod
     def forward(ctx, terms, check_simplex, slots, *sources):
@@ -916,7 +934,14 @@ class IICTermsFunction(torch.autograd.Function):
             if blk is not None and (si, blk) not in seen:
                 seen.add((si, blk))
                 cover[si] += v.numel()
-        ctx.covered = [c == s_.numel() for c, s_ in zip(cover, sources)]
+        # a source with two distinct regions that intersect (overlapping blocks, or the whole tensor and a block of it):
+        # every use then adds into a zero-filled buffer
+        regions = [set() for _ in sources]
+        for k, (si, blk) in enumerate(slots):
+            t = terms[k // 2]
+            regions[si].add(_region(t.x if k % 2 == 0 else t.y, blk, sources[si]))
+        ctx.overlap = [any(_intersect(a, b) for a in rs for b in rs if a < b) for rs in regions]
+        ctx.covered = [c == s_.numel() and not o for c, s_, o in zip(cover, sources, ctx.overlap)]
         ctx.set_materialize_grads(False)
         return tuple(outs)
 
@@ -945,11 +970,12 @@ class IICTermsFunction(torch.autograd.Function):
             si, blk = slots[k]
             shape, dev = ctx.src_meta[si]
             if G[si] is None:
-                zero = need_zero[si] or (blk is not None and not ctx.covered[si])
+                zero = need_zero[si] or ctx.overlap[si] or (blk is not None and not ctx.covered[si])
                 G[si] = (torch.zeros if zero else torch.empty)(shape, dtype=torch.float32, device=dev)
             dst = G[si] if blk is None else _block_view(G[si], like, blk[0], blk[1])
-            if (si, blk) in written:
-                return torch.zeros_like(like, memory_format=torch.contiguous_format), dst      # second use: add afterwards
+            if ctx.overlap[si] or (si, blk) in written:
+                # second use of the block, or a region that another use overlaps: add afterwards
+                return torch.zeros_like(like, memory_format=torch.contiguous_format), dst
             written.add((si, blk))
             return dst, None
 
