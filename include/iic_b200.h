@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IIC_B200_ABI_VERSION 6
+#define IIC_B200_ABI_VERSION 7
 
 /* flag bits written (OR-ed) into the int* `flags` words by the kernels */
 #define IIC_FLAG_NAN_LOSS 1      /* iic_loss.py:147-148,184-185 -> RuntimeError on the host  */
@@ -160,6 +160,39 @@ int iic_local_backward_from_logits(const float* lx, long long x_sn, long long x_
                                    int B, int K, int H, int W, int pad, float inv_temperature,
                                    const float* Wx, const float* Wy, const float* grad_loss,
                                    float* g_lx, float* g_ly, long long gx_sn, long long gy_sn, void* stream);
+
+/* The same for the reference's default cluster count (16 <= K <= 24, padding 1 or 3; ABI 7).  Its tensor-core kernels
+ * stage 8-channel slices and never hold a whole pixel, so a first pass writes per pixel of both maps
+ *   m = max_k(l_k * inv_temperature),  r = 1 / sum_k exp(l_k * inv_temperature - m)
+ * into the caller's `stats` buffer (iic_local_logit_stats_floats floats, 16-byte aligned: [2B][2][H][W], planes m and r,
+ * lx at samples 0..B-1, ly at B..2B-1), and the kernels use p = exp(l * inv_temperature - m) * r.  The caller keeps
+ * stats, Wx and Wy from the forward to the backward; nothing is allocated inside the library.
+ *   iic_local_from_logits_covered       1 when these entry points fuse the term on the given maps (device pointers and
+ *                                       strides as for the calls), 0 when the caller must apply the softmax and use
+ *                                       the probability entry points; the ONE rule both calls follow.  16 <= K <= 24:
+ *                                       padding 3, or padding 1 with enough row blocks to fill the SMs; W % 16 == 0;
+ *                                       16-byte aligned rows; tensor-core and TMA kernels not switched off.  K == 10:
+ *                                       the shapes of iic_local_joint_from_logits above.
+ *   iic_local_joint_from_logits_workspace_bytes   the workspace of the joint (per-SM slots of the kernel it selects)
+ *   iic_local_joint_from_logits_stats   as iic_local_joint_from_logits, also writing stats; on a K == 10 shape it is
+ *                                       that call (stats untouched, may be NULL); IIC_UNSUPPORTED when not covered
+ *   iic_local_backward_from_logits_stats  its backward, reading stats; Wx / Wy are writable because the K = 20 kernels
+ *                                       lay their weight images into the buffers' tails (iic_local_coeff_floats) */
+size_t iic_local_logit_stats_floats(int B, int H, int W);
+size_t iic_local_joint_from_logits_workspace_bytes(int device, int B, int K, int H, int W, int pad);
+int iic_local_from_logits_covered(int device, const float* lx, long long x_sn, long long x_sc, long long x_sh,
+                                  const float* ly, long long y_sn, long long y_sc, long long y_sh,
+                                  int B, int K, int H, int W, int pad);
+int iic_local_joint_from_logits_stats(const float* lx, long long x_sn, long long x_sc, long long x_sh,
+                                      const float* ly, long long y_sn, long long y_sc, long long y_sh,
+                                      int B, int K, int H, int W, int pad, float inv_temperature, float* stats,
+                                      double* J_out, void* workspace, size_t workspace_bytes,
+                                      iic_slot_info* info_host, void* stream);
+int iic_local_backward_from_logits_stats(const float* lx, long long x_sn, long long x_sc, long long x_sh,
+                                         const float* ly, long long y_sn, long long y_sc, long long y_sh,
+                                         int B, int K, int H, int W, int pad, float inv_temperature,
+                                         const float* stats, float* Wx, float* Wy, const float* grad_loss,
+                                         float* g_lx, float* g_ly, long long gx_sn, long long gy_sn, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Global IIC on (N,K) simplex rows.  Replaces compute_joint (iic_loss.py:74-94) and IIDLoss.forward

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libiic_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 FLAG_NAN_LOSS = 1
 FLAG_NOT_SIMPLEX = 2
 FLAG_BAD_LABEL = 4
@@ -52,6 +52,13 @@ PROTOTYPES = {
     "iic_finish": (_i, [_p, _i, _p, _ll, _p, _p, _p, _i, _i, _ll, _i, _p]),
     "iic_local_backward_from_logits": (_i, [_p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _i, _i, _i, _i, _i, C.c_float,
                                             _p, _p, _p, _p, _p, _ll, _ll, _p]),
+    "iic_local_logit_stats_floats": (_sz, [_i, _i, _i]),
+    "iic_local_joint_from_logits_workspace_bytes": (_sz, [_i] * 6),
+    "iic_local_from_logits_covered": (_i, [_i, _p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _i, _i, _i, _i, _i]),
+    "iic_local_joint_from_logits_stats": (_i, [_p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _i, _i, _i, _i, _i, C.c_float, _p,
+                                               _p, _p, _sz, _p, _p]),
+    "iic_local_backward_from_logits_stats": (_i, [_p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _i, _i, _i, _i, _i, C.c_float,
+                                                  _p, _p, _p, _p, _p, _p, _ll, _ll, _p]),
     "iic_global_joint_workspace_bytes": (_sz, [_i, _ll, _i]),
     "iic_global_joint": (_i, [_p, _ll, _p, _ll, _ll, _i, _p, _p, _sz, _p, _p]),
     "iic_global_epilogue": (_i, [_p, _i, _d, _i, _p, _p, _p, _p]),

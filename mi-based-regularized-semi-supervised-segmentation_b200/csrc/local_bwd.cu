@@ -311,3 +311,30 @@ extern "C" int iic_local_backward_from_logits(const float* lx, long long x_sn, l
   }
   return rc;
 }
+
+// Backward of iic_local_joint_from_logits_stats: the stats are the ones its forward wrote.  16 <= K <= 24 where
+// local_fl_tc_covered holds: row-block tensor-core sweeps on the logits (their weight images go into the tails of Wx / Wy,
+// hence float*); the K = 10 shapes as iic_local_backward_from_logits.
+extern "C" int iic_local_backward_from_logits_stats(const float* lx, long long x_sn, long long x_sc, long long x_sh,
+                                                    const float* ly, long long y_sn, long long y_sc, long long y_sh,
+                                                    int B, int K, int H, int W, int pad, float inv_temperature,
+                                                    const float* stats, float* Wx, float* Wy, const float* grad_loss,
+                                                    float* g_lx, float* g_ly, long long gx_sn, long long gy_sn,
+                                                    void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  IIC_REQUIRE(lx && ly && Wx && Wy && g_lx && g_ly, "iic_local_backward_from_logits_stats: null pointer");
+  const int sms = sm_count_cached(current_device());
+  IIC_REQUIRE(sms > 0, "iic_local_backward_from_logits_stats: no device");
+  const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
+  if (!local_fl_tc_covered(m))
+    return iic_local_backward_from_logits(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, inv_temperature, Wx,
+                                          Wy, grad_loss, g_lx, g_ly, gx_sn, gy_sn, stream);
+  IIC_REQUIRE(stats, "iic_local_backward_from_logits_stats: null stats");
+  if (gx_sn <= 0) gx_sn = (long long)K * H * W;
+  if (gy_sn <= 0) gy_sn = (long long)K * H * W;
+  const LocalGrads gr{grad_loss, g_lx, g_ly, gx_sn, gy_sn};
+  const int rc = local_bwd_tcrb_fl_try(m, stats, inv_temperature, Wx, Wy, gr, st);
+  if (rc > 0) return rc;
+  IIC_REQUIRE(rc == 0, "iic_local_backward_from_logits_stats: the row-block tensor-core backward refused a covered shape");
+  return 0;
+}

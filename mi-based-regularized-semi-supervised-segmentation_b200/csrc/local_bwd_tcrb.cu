@@ -17,6 +17,15 @@
 // warps ((128-pixel tile 0 / 1) x (even / odd source rows)): see local_bwd_tcrb10.cu.  Per item: for each 8-channel
 // slice the slice's weight image (64*T*T*24 bytes, double buffered, one bulk copy) stays resident while the
 // R + T - 1 source rows stream through the operand ring.
+//
+// From-logits form (FL, the cluster head's SoftmaxWithT fused): the maps hold logits.  The TMA warp also stages the
+// (m, r) of every staged source pixel (local_logit_stats_kernel, local_logits.cu) and the transform converts each logit
+// slice to p = exp(l * inv_temp - m) * r (r = 0 in the TMA zero fill outside the map, so p stays 0 there; channels
+// >= K are zeroed).  The drain holds all 24 accumulator channels g_o of its pixel and applies the softmax adjoint
+//   d logit_o = inv_temp * p_o * (g_o - sum_k g_k p_k)
+// with p at the OUTPUT pixel from its own logits and (m, r), read coalesced (lane = pixel) after an L2 prefetch of the
+// item's rows issued while the MMAs run.  The FL form issues each tile's MMAs from ONE warp (the even / odd source-row
+// split of two issuers sums into the same accumulators in a timing-dependent order), so two calls give the same bits.
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -35,6 +44,7 @@ constexpr int A_PART = 2 * APX * 16;     // fp32 part / bf16 part of one row buf
 constexpr int A_ROW = 2 * A_PART;        // 17408
 constexpr int NA_MAX = 6, NRAW_MAX = 8;  // ring depths are chosen per launch from the shared memory the weight slots leave
 constexpr int RAW_MAX = SL * 256 * 4;    // 8192
+constexpr int FL_STATS = 2 * 256 * 4;    // FL: a raw slot also holds the staged pixels' stats [2][SW] after RAW_MAX bytes
 constexpr int NTHREADS = 448;            // warps: 0 TMA, 3 TMEM + weights, 1 2 12 13 MMA issuers, 4-7 transform, 8-11 epilogue
 constexpr int SMEM_LIMIT = 225 * 1024;    // dynamic shared memory we may ask for (the static barriers share the 227 KB)
 
@@ -59,6 +69,16 @@ struct Params {
   long long out_sn;             // sample stride of `out` in elements
 };
 
+// the from-logits form's extra arguments (unused by the probability instantiations)
+struct FLParams {
+  CUtensorMap stats;            // the (2B, 2, H, W) stats tensor, box [2][1][PW + 8]: x stats at n, y stats at B + n
+  int src_n;                    // stats sample offset of the source map (B for y, 0 for x)
+  float inv_temp;
+  const float* lout;            // logits of the OUTPUT map (its gradient is `out`), strides below
+  long long l_sn, l_sc, l_sh;
+  const float* sout;            // its (m, r) planes: sample n at sout + n * 2HW
+};
+
 // Wc[cin][ty*T+tx][Kp4] -> per (slice, tx) a tile {fp32 [2 chunks][T*KP rows][4 in], bf16 [wh, wl][T*KP rows][8 in]},
 // rows ordered (T-1-ty)*KP + o
 __global__ void weight_image_kernel(const float* __restrict__ Wc, float* __restrict__ img, int K, int Kp4, int KP, int NS, int T) {
@@ -80,9 +100,14 @@ __global__ void weight_image_kernel(const float* __restrict__ Wc, float* __restr
   reinterpret_cast<uint4*>(tile)[3 * rows + row] = pack8<true>(v);      // wl (pairs with ah)
 }
 
-template <int T>
+// bytes between raw-ring slots (a namespace-scope function rather than a constexpr local, which changes the probability
+// instantiation's register assignment)
+template <bool FL>
+__device__ constexpr int raw_stride() { return FL ? RAW_MAX + FL_STATS : RAW_MAX; }
+
+template <int T, bool FL>
 __global__ void __launch_bounds__(NTHREADS, 1)
-local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
+local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P, const __grid_constant__ FLParams F) {
   constexpr int PAD = T / 2;
   extern __shared__ __align__(1024) unsigned char smem_dyn[];
   __shared__ __align__(8) uint64_t raw_full[NRAW_MAX], raw_empty[NRAW_MAX], a_full[NA_MAX], a_empty[NA_MAX], w_full[2], w_empty[2], accum_full, tmem_ready;
@@ -123,6 +148,7 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
     // ===== TMA producer: one source row of one channel slice per stage =====
     if (lane == 0) {
       tma_prefetch_desc(&maps);
+      if constexpr (FL) tma_prefetch_desc(&F.stats);
       int t = 0, s = 0;                                 // ring slot and phase as running counters: no divisions per stage
       unsigned sph = 0;
       for (int i = 0; i < nit; ++i) {
@@ -134,8 +160,11 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
             { const int tt = t; (void)tt; TRACE(0, 0); }
             if (t >= NRAW) mbar_wait(&raw_empty[s], sph ^ 1u, 1);
             { const int tt = t; (void)tt; TRACE(0, 1); }
-            mbar_arrive_expect_tx(&raw_full[s], raw_bytes);
-            tma_load_4d(raw_ring + s * RAW_MAX, &maps, &raw_full[s], panel * P.PW - 4, r0 - PAD + q, js * SL, n);
+            mbar_arrive_expect_tx(&raw_full[s], FL ? raw_bytes + 2 * SW * 4 : raw_bytes);
+            tma_load_4d(raw_ring + s * raw_stride<FL>(), &maps, &raw_full[s], panel * P.PW - 4, r0 - PAD + q, js * SL, n);
+            if constexpr (FL)                              // the source pixels' (m, r), behind the logits
+              tma_load_4d(raw_ring + s * raw_stride<FL>() + RAW_MAX, &F.stats, &raw_full[s], panel * P.PW - 4, r0 - PAD + q, 0,
+                          F.src_n + n);
             if (++s == NRAW) { s = 0; sph ^= 1u; }
           }
       }
@@ -162,7 +191,10 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
     const uint32_t rows = (uint32_t)(T * KP);              // rows of one weight part chunk
     int a = 0, tt = 0;
     unsigned aph = 0;
-    for (int i = 0; i < nit; ++i) {
+    // FL: the odd-row issuers stay out altogether (waiting on barriers they do not consume, they could fall two phases
+    // behind)
+    const int nit_issue = FL && par ? 0 : nit;
+    for (int i = 0; i < nit_issue; ++i) {
       mbar_wait(&tmem_ready, (unsigned)i & 1u, 6);          // accumulators zeroed
       asm volatile("tcgen05.fence::after_thread_sync;");
       for (int js = 0; js < NS; ++js) {
@@ -170,7 +202,9 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
         mbar_wait(&w_full[ws], (unsigned)(w >> 1) & 1u, 7);
         const uint64_t w_base = make_desc_kmajor_noswz(smem_u32(w_ring + ws * wslot_bytes), rows * 16);
         for (int q = 0; q < NQ; ++q, ++tt) {
-          if ((q & 1) != par) {                          // the other issuer of this tile takes this source row
+          // FL: one issuer per tile takes every source row, in order, so that the fp32 accumulation order (and the
+          // gradient's bits) is the same on every call; the barrier counts hold (its last-row commits come twice)
+          if (!FL && (q & 1) != par) {                   // the other issuer of this tile takes this source row
             if (++a == NA) { a = 0; aph ^= 1u; }
             continue;
           }
@@ -223,11 +257,18 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
       mbar_wait(&raw_full[s], sph, 4);
       if (threadIdx.x == 128) TRACE(3, 2);
       unsigned char* abuf = a_ring + a * A_ROW;
-      const float* raw = reinterpret_cast<const float*>(raw_ring + s * RAW_MAX);
+      const float* raw = reinterpret_cast<const float*>(raw_ring + s * raw_stride<FL>());
       for (int px = tid; px < SW; px += 128) {
         float v[SL];
 #pragma unroll
         for (int c = 0; c < SL; ++c) v[c] = raw[c * SW + px];
+        if constexpr (FL) {
+          const float* sm = reinterpret_cast<const float*>(raw_ring + s * raw_stride<FL>() + RAW_MAX);   // m [SW], then r [SW]
+          const float mx = sm[px], rr = sm[SW + px];
+          const int fjs = (t / NQ) % NS;                                // channel slice of this stage
+#pragma unroll
+          for (int c = 0; c < SL; ++c) v[c] = fjs * SL + c < P.K ? __expf(__fmul_rn(v[c], F.inv_temp) - mx) * rr : 0.f;
+        }
         const int off = (px + 4) * 16;                                   // staged pixel px is column px - 4
         *reinterpret_cast<float4*>(abuf + off) = make_float4(v[0], v[1], v[2], v[3]);
         *reinterpret_cast<float4*>(abuf + off + APX * 16) = make_float4(v[4], v[5], v[6], v[7]);
@@ -264,6 +305,18 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
       const int panel = item % P.npanel, ib = item / P.npanel;
       const int n = ib / P.nblk, r0 = (ib - n * P.nblk) * R;
       const int col0 = panel * P.PW;
+      if constexpr (FL) {
+        // while the MMAs run: pull the item's output logits and stats into L2 (128-byte lines, all drain lanes)
+        const int rv = (P.H - r0 < R) ? P.H - r0 : R;
+        const int lines = (P.PW * 4 + 127) / 128;
+        const int per_plane = rv * lines;
+        for (int e = threadIdx.x - 256; e < (P.K + 2) * per_plane; e += 128) {
+          const int ch = e / per_plane, rem = e - ch * per_plane, row = rem / lines, ln = rem - row * lines;
+          const float* src = ch < P.K ? F.lout + (size_t)n * F.l_sn + (size_t)ch * F.l_sc + (size_t)(r0 + row) * F.l_sh
+                                      : F.sout + ((size_t)n * 2 + (ch - P.K)) * plane + (size_t)(r0 + row) * P.W;
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(src + col0 + ln * 32));
+        }
+      }
       mbar_wait(&accum_full, (unsigned)i & 1u, 8);
       asm volatile("tcgen05.fence::after_thread_sync;");
       // The MMAs of the next item wait for this drain (all TMEM columns are in use), so it is kept short: the 2 x 24
@@ -290,22 +343,56 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
             }
           }
           asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-          if (live) {
+          if constexpr (FL) {
+            if (live) {
+  #pragma unroll
+              for (int h = 0; h < 2; ++h) {
+                if (orow + h < rv) {
+                  const int row = r0 + orow + h;
+                  float* dst = P.out + (size_t)n * P.out_sn + (size_t)row * P.W + c;
+                  const float* lp = F.lout + (size_t)n * F.l_sn + (size_t)row * F.l_sh + c;
+                  const float* sp = F.sout + (size_t)n * 2 * plane + (size_t)row * P.W + c;
+                  const float mx = __ldg(sp), rr = __ldg(sp + plane);
+                  float pr[24];
+                  float dot = 0.f;
+  #pragma unroll
+                  for (int o = 0; o < 24; ++o) {
+                    if (o < P.K) {                                          // (columns >= KP were not loaded)
+                      pr[o] = __expf(__fmul_rn(__ldg(lp + (size_t)o * F.l_sc), F.inv_temp) - mx) * rr;
+                      dot = fmaf(g * __uint_as_float(v[h][o]), pr[o], dot);
+                    }
+                  }
+  #pragma unroll
+                  for (int o = 0; o < 16; ++o) dst[(size_t)o * plane] = F.inv_temp * pr[o] * (g * __uint_as_float(v[h][o]) - dot);
+                  if (P.K == 20) {
+  #pragma unroll
+                    for (int o = 16; o < 20; ++o) dst[(size_t)o * plane] = F.inv_temp * pr[o] * (g * __uint_as_float(v[h][o]) - dot);
+                  } else {
+  #pragma unroll
+                    for (int o = 16; o < 24; ++o)
+                      if (o < P.K) dst[(size_t)o * plane] = F.inv_temp * pr[o] * (g * __uint_as_float(v[h][o]) - dot);
+                  }
+                }
+              }
+            }
+          } else {
+            if (live) {
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              if (orow + h < rv) {
-                float* dst = P.out + (size_t)n * P.out_sn + (size_t)(r0 + orow + h) * P.W + c;
-                // straight-line stores for the channels every covered head has (K >= 16; a branch per channel costs ~10
-                // instructions and a uniform-register reload per store), the yaml default K = 20 entirely
+              for (int h = 0; h < 2; ++h) {
+                if (orow + h < rv) {
+                  float* dst = P.out + (size_t)n * P.out_sn + (size_t)(r0 + orow + h) * P.W + c;
+                  // straight-line stores for the channels every covered head has (K >= 16; a branch per channel costs ~10
+                  // instructions and a uniform-register reload per store), the yaml default K = 20 entirely
 #pragma unroll
-                for (int o = 0; o < 16; ++o) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
-                if (P.K == 20) {
+                  for (int o = 0; o < 16; ++o) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
+                  if (P.K == 20) {
 #pragma unroll
-                  for (int o = 16; o < 20; ++o) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
-                } else {
+                    for (int o = 16; o < 20; ++o) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
+                  } else {
 #pragma unroll
-                  for (int o = 16; o < 24; ++o)
-                    if (o < P.K) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
+                    for (int o = 16; o < 24; ++o)
+                      if (o < P.K) dst[(size_t)o * plane] = g * __uint_as_float(v[h][o]);
+                  }
                 }
               }
             }
@@ -320,10 +407,10 @@ local_bwd_tcrb_kernel(const __grid_constant__ CUtensorMap maps, const Params P) 
   if (wid == 3) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
 }
 
-template <int T>
-static int launch(const CUtensorMap& m, const Params& P, int grid, size_t smem, cudaStream_t st) {
-  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tcrb_kernel<T>), (int)(SMEM_LIMIT)));
-  local_bwd_tcrb_kernel<T><<<grid, NTHREADS, smem, st>>>(m, P);
+template <int T, bool FL>
+static int launch(const CUtensorMap& m, const Params& P, const FLParams& F, int grid, size_t smem, cudaStream_t st) {
+  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tcrb_kernel<T, FL>), (int)(SMEM_LIMIT)));
+  local_bwd_tcrb_kernel<T, FL><<<grid, NTHREADS, smem, st>>>(m, P, F);
   IIC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -336,37 +423,65 @@ size_t local_bwd_tcrb_image_bytes(int K, int pad) {
   return (size_t)(KP / bwdrb::SL) * 64 * T * T * KP;
 }
 
-int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
+// Column panels, rows per item and item count of a (B, K, H, W) map; false when the family does not cover it.  Maps wider
+// than one TMA box are cut into column panels: 128 columns (one pixel tile, no padding) when that divides the width, else
+// equal panels of at most 248 columns.
+bool local_bwd_tcrb_plan(int B, int K, int H, int W, int pad, int* PW_out, int* npanel_out, int* R_out, int* n_items_out) {
   using namespace bwdrb;
-  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad, sms = m.sms;
-  if (K < 16 || K > 24 || (pad != 1 && pad != 3) || W % 4 != 0 || W < 8) return -1;
-  // maps wider than one TMA box are cut into column panels: 128 columns (one pixel tile, no padding) when that divides
-  // the width, else equal panels of at most 248 columns
+  if (K < 16 || K > 24 || (pad != 1 && pad != 3) || W % 4 != 0 || W < 8) return false;
   int npanel = 1, PW = W;
   if (W > MAXW) {
     if (W % 128 == 0) { PW = 128; npanel = W / 128; }
     else { npanel = (W + MAXW - 1) / MAXW; PW = (((W + npanel - 1) / npanel) + 3) & ~3; }
   }
-  const int T = 2 * pad + 1, KP = (K + 7) & ~7, NS = KP / SL, Kp4 = (K + 3) & ~3;
+  const int KP = (K + 7) & ~7;
   const int ntile = PW > 128 ? 2 : 1;
   int R = 512 / (ntile * KP);
   if (R > H) R = H;
+  *PW_out = PW; *npanel_out = npanel; *R_out = R;
+  *n_items_out = B * ((H + R - 1) / R) * npanel;
+  return true;
+}
+
+// 3 x 3 window: the FFMA2 kernel is as fast unless there are enough row blocks to keep every SM busy (measured:
+// (32,20,224,224) 0.32 ms vs 0.42 ms, (8,20,112,112) no gain)
+bool local_bwd_tcrb_p1_gate(int n_items, int sms) { return n_items >= 2 * sms || options().tcrb_p1; }
+
+// stats == nullptr: probabilities; else logits with the per-pixel (m, r) of local_logit_stats_kernel in `stats`
+static int tcrb_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                    cudaStream_t st) {
+  using namespace bwdrb;
+  const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad, sms = m.sms;
+  int PW, npanel, R, n_items;
+  if (!local_bwd_tcrb_plan(B, K, H, W, pad, &PW, &npanel, &R, &n_items)) return -1;
+  const int T = 2 * pad + 1, KP = (K + 7) & ~7, NS = KP / SL, Kp4 = (K + 3) & ~3;
+  const bool fl = stats != nullptr;
+  const int raw_stride = fl ? RAW_MAX + FL_STATS : RAW_MAX;
   const int wslice = 64 * T * T * KP;
-  // ring depths: what the two weight slots leave, shared between the operand ring (17 KB slots) and the raw ring (8 KB)
+  // ring depths: what the two weight slots leave, shared between the operand ring (17 KB slots) and the raw ring (8 KB,
+  // 10 KB from logits)
   const long long spare = (long long)SMEM_LIMIT - 1024 - 2LL * ((wslice + 127) & ~127);
   int na = 3, nraw = 2;
-  if (spare < (long long)na * A_ROW + (long long)nraw * RAW_MAX) return -1;
-  while (nraw < NRAW_MAX && spare >= (long long)na * A_ROW + (long long)(nraw + 1) * RAW_MAX) ++nraw;
-  while (na < NA_MAX && spare >= (long long)(na + 1) * A_ROW + (long long)nraw * RAW_MAX) ++na;
-  const size_t smem = (size_t)2 * ((wslice + 127) & ~127) + (size_t)na * A_ROW + (size_t)nraw * RAW_MAX + 1024;
+  if (spare < (long long)na * A_ROW + (long long)nraw * raw_stride) return -1;
+  while (nraw < NRAW_MAX && spare >= (long long)na * A_ROW + (long long)(nraw + 1) * raw_stride) ++nraw;
+  while (na < NA_MAX && spare >= (long long)(na + 1) * A_ROW + (long long)nraw * raw_stride) ++na;
+  const size_t smem = (size_t)2 * ((wslice + 127) & ~127) + (size_t)na * A_ROW + (size_t)nraw * raw_stride + 1024;
   CUtensorMap mx, my;
   if (!make_map_4d(&mx, m.x, m, PW + 8, 1, SL)) return -1;
   if (!make_map_4d(&my, m.y, m, PW + 8, 1, SL)) return -1;
   const int nblk = (H + R - 1) / R;
-  const int n_items = B * nblk * npanel;
-  // 3 x 3 window: the FFMA2 kernel is as fast unless there are enough row blocks to keep every SM busy (measured:
-  // (32,20,224,224) 0.32 ms vs 0.42 ms, (8,20,112,112) no gain)
-  if (pad == 1 && n_items < 2 * sms && !options().tcrb_p1) return -1;
+  if (pad == 1 && !local_bwd_tcrb_p1_gate(n_items, sms)) return -1;
+  const long long hw = (long long)H * W;
+  FLParams Fgx{}, Fgy{};
+  if (fl) {
+    if (!make_map_4d(&Fgx.stats, stats, 2 * B, 2, H, W, 2 * hw, hw, W, PW + 8, 1, 2)) return -1;
+    Fgy.stats = Fgx.stats;
+    // dL/dx: source y (stats at B + n), output x;  dL/dy: source x, output y
+    Fgx.src_n = B; Fgx.inv_temp = inv_temp; Fgx.lout = m.x.p; Fgx.l_sn = m.x.sn; Fgx.l_sc = m.x.sc; Fgx.l_sh = m.x.sh;
+    Fgx.sout = stats;
+    Fgy.src_n = 0; Fgy.inv_temp = inv_temp; Fgy.lout = m.y.p; Fgy.l_sn = m.y.sn; Fgy.l_sc = m.y.sc; Fgy.l_sh = m.y.sh;
+    Fgy.sout = stats + 2 * B * hw;
+  }
   const int grid = n_items < sms ? n_items : sms;
   // the weight image lives in the tail of the caller's coefficient buffer (common.cuh)
   float* img_x = Wx + local_coeff_image_offset(K, pad, 1);
@@ -377,12 +492,29 @@ int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrad
   IIC_CHECK_CUDA(cudaGetLastError());
   Params Pgx{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_x, g.grad_loss, g.gx, g.gx_sn};     // dL/dx from y
   Params Pgy{B, H, W, K, KP, NS, R, nblk, n_items, PW, npanel, wslice, na, nraw, img_y, g.grad_loss, g.gy, g.gy_sn};     // dL/dy from x
-  if (T == 3) {
-    if (int rc = launch<3>(my, Pgx, grid, smem, st)) return rc;
-    return launch<3>(mx, Pgy, grid, smem, st);
+  if (fl) {
+    if (T == 3) {
+      if (int rc = launch<3, true>(my, Pgx, Fgx, grid, smem, st)) return rc;
+      return launch<3, true>(mx, Pgy, Fgy, grid, smem, st);
+    }
+    if (int rc = launch<7, true>(my, Pgx, Fgx, grid, smem, st)) return rc;
+    return launch<7, true>(mx, Pgy, Fgy, grid, smem, st);
   }
-  if (int rc = launch<7>(my, Pgx, grid, smem, st)) return rc;
-  return launch<7>(mx, Pgy, grid, smem, st);
+  if (T == 3) {
+    if (int rc = launch<3, false>(my, Pgx, Fgx, grid, smem, st)) return rc;
+    return launch<3, false>(mx, Pgy, Fgy, grid, smem, st);
+  }
+  if (int rc = launch<7, false>(my, Pgx, Fgx, grid, smem, st)) return rc;
+  return launch<7, false>(mx, Pgy, Fgy, grid, smem, st);
+}
+
+int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
+  return tcrb_try(m, nullptr, 1.f, Wx, Wy, g, st);
+}
+
+int local_bwd_tcrb_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                          cudaStream_t st) {
+  return tcrb_try(m, stats, inv_temp, Wx, Wy, g, st);
 }
 
 }  // namespace iic

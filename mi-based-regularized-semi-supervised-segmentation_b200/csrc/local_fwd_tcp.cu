@@ -17,6 +17,11 @@
 //   warps 1, 3 MMA issuers (one row tile each)
 // The slot holds D in a coalesced permuted order; reduce_packed_kernel adds the slots in fp64 in a fixed order and
 // writes J in its [dy][dx][i][j] layout.
+//
+// From-logits form (FL): x and y hold the cluster head's logits and local_logit_stats_kernel (local_logits.cu) has
+// written each pixel's (m, r); the TMA warp also stages the stats of the staged pixels, and the transform converts
+// every logit to p = exp(l * inv_temp - m) * r before the fp32 / bf16 split.  Outside the map the TMA zero fill gives
+// r = 0, so p = 0 there (the conv padding), not softmax(0) = 1/K; B rows of channels K..23 are zeroed explicitly.
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -37,6 +42,10 @@ constexpr int NTHREADS = 512;                  // 4 control warps + 12 transform
 constexpr int SEG_KB_DEFAULT = 64;             // k-blocks per TMEM accumulation run (1024 pixels: uniform bias <= 2e-5,
                                                // see local_fwd_tc.cu; the drain is costlier here relative to the MMAs)
 constexpr int SMEM_LIMIT = 225 * 1024;
+// FL: the staged stats follow the y box in a raw slot: x stats [2][XRW] at fl_sx(T), y stats [2][T][PXB] 256 bytes on
+__host__ __device__ constexpr int fl_sx(int T) { return 3072 + KPC * T * 64; }
+constexpr int FL_SX_BYTES = 2 * XRW * 4;       // 224
+__host__ __device__ constexpr int fl_sy_bytes(int T) { return 2 * T * PXB * 4; }
 
 
 #ifdef IIC_TC_TRACE
@@ -57,12 +66,19 @@ struct Params {
   float* partial;               // [gridDim.x][slot_floats]
 };
 
+// the from-logits form's extra arguments (unused by the probability instantiations)
+struct FLParams {
+  CUtensorMap sx, sy;           // the (2B, 2, H, W) stats tensor: x stats at n, y stats at B + n
+  float inv_temp;
+};
+
 using iic::packed_slot_index;
 __host__ __device__ inline size_t slot_index(int mt, int m, int c, int nb) { return packed_slot_index(mt, m, c, nb); }
 
-template <int T>
+template <int T, bool FL>
 __global__ void __launch_bounds__(NTHREADS, 1)
-local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_constant__ CUtensorMap mapy, const Params P) {
+local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_constant__ CUtensorMap mapy, const Params P,
+                       const __grid_constant__ FLParams F) {
   constexpr int PAD = T / 2;
   constexpr int NOP_MAX = 8;
   extern __shared__ __align__(1024) unsigned char smem_dyn[];
@@ -103,6 +119,7 @@ local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_co
     if (lane == 0) {
       tma_prefetch_desc(&mapx);
       tma_prefetch_desc(&mapy);
+      if constexpr (FL) { tma_prefetch_desc(&F.sx); tma_prefetch_desc(&F.sy); }
       // (image, row, segment) of the first k-block by division, then running counters: no divisions in the loops
       const int per_img = P.H * P.segs_w;
       int n = kb0 / per_img;
@@ -118,7 +135,13 @@ local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_co
         if (++sg == P.segs_w) { sg = 0; if (++q == P.H) { q = 0; ++n; } }
         unsigned char* st = raw_ring + (size_t)s * P.raw_bytes;
         if (P.dbg & 1) { mbar_arrive(&raw_full[s]); continue; }
-        mbar_arrive_expect_tx(&raw_full[s], xraw_bytes + KPC * T * 64);
+        if constexpr (FL) {
+          mbar_arrive_expect_tx(&raw_full[s], xraw_bytes + KPC * T * 64 + FL_SX_BYTES + fl_sy_bytes(T));
+          tma_load_4d(st + fl_sx(T), &F.sx, &raw_full[s], c0 - 4, qc, 0, nc);
+          tma_load_4d(st + fl_sx(T) + 256, &F.sy, &raw_full[s], c0, qc + PAD - (T - 1), 0, P.B + nc);
+        } else {
+          mbar_arrive_expect_tx(&raw_full[s], xraw_bytes + KPC * T * 64);
+        }
         tma_load_4d(st, &mapx, &raw_full[s], c0 - 4, qc, 0, nc);
         tma_load_4d(st + 3072, &mapy, &raw_full[s], c0, qc + PAD - (T - 1), 0, nc);
         TRACE(0, 2);
@@ -194,6 +217,11 @@ local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_co
         float xv[PXB];
 #pragma unroll
         for (int p = 0; p < PXB; ++p) xv[p] = xs[p];
+        if constexpr (FL) {
+          const float* sm = reinterpret_cast<const float*>(raw + fl_sx(T)) + (dx + 4 - PAD);      // m, then r at + XRW
+#pragma unroll
+          for (int p = 0; p < PXB; ++p) xv[p] = __expf(__fmul_rn(xv[p], F.inv_temp) - sm[p]) * sm[XRW + p];
+        }
         unsigned char* a32 = op + (mt * 2) * ATILE + r * 64;
         unsigned char* a16 = a32 + ATILE;
 #pragma unroll
@@ -214,7 +242,17 @@ local_joint_tcp_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_co
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           const int off = (c ^ sw) << 4;
-          const float4 t = *reinterpret_cast<const float4*>(raw + 3072 + nrow * 64 + off);
+          float4 t = *reinterpret_cast<const float4*>(raw + 3072 + nrow * 64 + off);
+          if constexpr (FL) {
+            // box row nrow = (channel, y row r); channels >= K were zero-filled logits: their p must be 0, not exp(-m) r
+            const int r = nrow % T;
+            const float* sm = reinterpret_cast<const float*>(raw + fl_sx(T) + 256) + r * PXB + 4 * c;   // m; r at + T*PXB
+            const bool live = nrow < T * P.K;
+            t.x = live ? __expf(__fmul_rn(t.x, F.inv_temp) - sm[0]) * sm[T * PXB + 0] : 0.f;
+            t.y = live ? __expf(__fmul_rn(t.y, F.inv_temp) - sm[1]) * sm[T * PXB + 1] : 0.f;
+            t.z = live ? __expf(__fmul_rn(t.z, F.inv_temp) - sm[2]) * sm[T * PXB + 2] : 0.f;
+            t.w = live ? __expf(__fmul_rn(t.w, F.inv_temp) - sm[3]) * sm[T * PXB + 3] : 0.f;
+          }
           *reinterpret_cast<float4*>(b32 + off) = t;
           yv[4 * c] = t.x; yv[4 * c + 1] = t.y; yv[4 * c + 2] = t.z; yv[4 * c + 3] = t.w;
         }
@@ -298,10 +336,11 @@ reduce_packed_kernel(const float* __restrict__ partial, int ncta, int slot_float
   }
 }
 
-template <int T>
-static int launch(const CUtensorMap& mx, const CUtensorMap& my, const Params& P, int grid, size_t smem, cudaStream_t st) {
-  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tcp_kernel<T>), (int)(SMEM_LIMIT)));
-  local_joint_tcp_kernel<T><<<grid, NTHREADS, smem, st>>>(mx, my, P);
+template <int T, bool FL>
+static int launch(const CUtensorMap& mx, const CUtensorMap& my, const Params& P, const FLParams& F, int grid, size_t smem,
+                  cudaStream_t st) {
+  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tcp_kernel<T, FL>), (int)(SMEM_LIMIT)));
+  local_joint_tcp_kernel<T, FL><<<grid, NTHREADS, smem, st>>>(mx, my, P, F);
   IIC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -314,23 +353,34 @@ size_t local_joint_tcp_slot_floats(int K, int pad) {
   return (size_t)((T * K + 127) / 128) * 128 * (T * fwdtcp::KPC);
 }
 
-int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_floats, SlotInfo* slots, cudaStream_t st) {
+// stats == nullptr: probabilities; else logits with the per-pixel (m, r) of local_logit_stats_kernel in `stats`
+static int tcp_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, size_t partial_floats,
+                   SlotInfo* slots, cudaStream_t st) {
   using namespace fwdtcp;
   const int B = m.B, K = m.K, H = m.H, W = m.W;
   const size_t slot_floats = local_joint_tcp_slot_floats(K, m.pad);
   if (slot_floats == 0 || W % PXB != 0) return -1;
   const int T = 2 * m.pad + 1;
   const int nmt = (T * K + 127) / 128, nb = T * KPC;
+  const bool fl = stats != nullptr;
   CUtensorMap mx, my;
   if (!make_map_4d(&mx, m.x, m, XRW, 1, KPC)) return -1;
   if (!make_map_4d(&my, m.y, m, PXB, T, KPC, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
+  FLParams F{};
+  F.inv_temp = inv_temp;
+  if (fl) {
+    const long long hw = (long long)H * W;
+    if (!make_map_4d(&F.sx, stats, 2 * B, 2, H, W, 2 * hw, hw, W, XRW, 1, 2)) return -1;
+    if (!make_map_4d(&F.sy, stats, 2 * B, 2, H, W, 2 * hw, hw, W, PXB, T, 2)) return -1;
+  }
   const long long nkb = (long long)B * H * (W / PXB);
   long long grid = m.sms;
   if ((long long)(partial_floats / slot_floats) < grid) grid = (long long)(partial_floats / slot_floats);
   if (grid > nkb) grid = nkb;
   if (grid < 1) return -1;
   const int op_bytes = (nmt * 2 * ATILE + 2 * nb * 64 + 1023) & ~1023;
-  const int raw_bytes = (3072 + KPC * T * 64 + 1023) & ~1023;
+  const int raw_used = fl ? fl_sx(T) + 256 + fl_sy_bytes(T) : 3072 + KPC * T * 64;
+  const int raw_bytes = (raw_used + 1023) & ~1023;
   int nop = (SMEM_LIMIT - 1024 - NRAW * raw_bytes) / op_bytes;
   if (nop > 8) nop = 8;
   if (tc::bringup_env("IIC_TC_NOP", nop) < nop) nop = tc::bringup_env("IIC_TC_NOP", nop);   // experiments (bring-up builds only)
@@ -339,10 +389,21 @@ int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_float
   Params P{B, H, W, K, W / PXB, nmt, nb, op_bytes, raw_bytes, nop,
            tc::bringup_env("IIC_TC_SEG", SEG_KB_DEFAULT),
            tc::bringup_env("IIC_TC_DBG", 0), partial};
-  const int rc = T == 3 ? launch<3>(mx, my, P, (int)grid, smem, st) : launch<7>(mx, my, P, (int)grid, smem, st);
+  int rc;
+  if (fl) rc = T == 3 ? launch<3, true>(mx, my, P, F, (int)grid, smem, st) : launch<7, true>(mx, my, P, F, (int)grid, smem, st);
+  else rc = T == 3 ? launch<3, false>(mx, my, P, F, (int)grid, smem, st) : launch<7, false>(mx, my, P, F, (int)grid, smem, st);
   if (rc) return rc;
   *slots = SlotInfo{SLOT_PACKED, (int)grid, (long long)slot_floats, nb};
   return 0;
+}
+
+int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_floats, SlotInfo* slots, cudaStream_t st) {
+  return tcp_try(m, nullptr, 1.f, partial, partial_floats, slots, st);
+}
+
+int local_joint_tcp_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, size_t partial_floats,
+                           SlotInfo* slots, cudaStream_t st) {
+  return tcp_try(m, stats, inv_temp, partial, partial_floats, slots, st);
 }
 
 }  // namespace iic

@@ -43,6 +43,9 @@ int local_joint_tc_try(const LocalMaps& m, float* partial, int max_ctas, SlotInf
 int local_joint_tcj10_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, int* flags, int* checked,
                           int from_logits, float inv_temp, cudaStream_t st);
 int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_floats, SlotInfo* slots, cudaStream_t st);
+// its from-logits form: `stats` holds the per-pixel (m, r) of both maps (local_logit_stats, local_logits.cu)
+int local_joint_tcp_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, size_t partial_floats,
+                           SlotInfo* slots, cudaStream_t st);
 // floats of one slot of the packed tensor-core joint (0 when it does not cover (K, pad)); the workspace is sized for it
 size_t local_joint_tcp_slot_floats(int K, int pad);
 namespace fwdtcp {
@@ -58,11 +61,23 @@ int local_bwd_fast_try(const LocalMaps& m, const float* Wx, const float* Wy, con
                        float inv_temp, cudaStream_t st);
 int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st);
 int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st);
+int local_bwd_tcrb_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                          cudaStream_t st);
+// the tcrb family's work split (false: not covered) and its padding-1 gate ("enough row blocks to fill the SMs")
+bool local_bwd_tcrb_plan(int B, int K, int H, int W, int pad, int* PW, int* npanel, int* R, int* n_items);
+bool local_bwd_tcrb_p1_gate(int n_items, int sms);
 int local_bwd_tcrb10_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, cudaStream_t st);
 int local_bwd_tcrb10h_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, int from_logits,
                           float inv_temp, cudaStream_t st);
 // bytes of the weight image in the coefficient buffers' tail (0 when the family does not cover (K, pad))
 size_t local_bwd_tc_image_bytes(int K, int pad);      // K = 128, padding 1
 size_t local_bwd_tcrb_image_bytes(int K, int pad);    // 16 <= K <= 24, padding 1 or 3
+
+// ---- from logits, 16 <= K <= 24 (local_logits.cu) ----
+// THE rule that decides whether such a term runs fused (tcp joint + tcrb backward on logits): used by both entry points
+// and by iic_local_from_logits_covered
+bool local_fl_tc_covered(const LocalMaps& m);
+// (m, r) of every pixel of both maps into stats = [2B][2][H][W] (x at n, y at B + n)
+int local_logit_stats(const LocalMaps& m, float inv_temp, float* stats, cudaStream_t st);
 
 }  // namespace iic

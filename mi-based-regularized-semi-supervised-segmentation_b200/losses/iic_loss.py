@@ -22,7 +22,7 @@ from torch import Tensor, nn
 
 from .. import checks
 from ..ops import (FusedShapeUnsupported, GlobalIICFunction, GlobalTerm, JointFunction, LocalIICFunction,
-                   LocalIICLogitsFunction, LocalTerm, iic_terms)
+                   LocalIICLogitsFunction, LocalTerm, from_logits_covered, iic_terms)
 
 
 def _pair(x):
@@ -126,8 +126,11 @@ class IIDSegmentationSmallPathLoss(IIDSegmentationLoss):
         fused into the joint kernel and their backward into the gradient kernel, so the probability maps are
         never written to memory.  The gradient is returned with respect to the logits.
 
-        The fused kernels cover the udaiic decoder shapes (padding 1, 10 clusters, one patch, width a multiple
-        of 4 and at most 248); any other shape applies the softmax first and takes the probability path."""
+        The fused kernels cover one patch (the patch at least the map) and
+          * 10 clusters: padding 1, width a multiple of 4 and at most 248 (the udaiic decoder shapes);
+          * 16 to 24 clusters (the reference's 20): padding 3, or padding 1 on maps with enough row blocks to fill the
+            GPU; width a multiple of 16.
+        Both need 16-byte aligned rows.  Any other shape applies the softmax first and takes the probability path."""
         assert logits_out.shape == logits_tf_out.shape, (logits_out.shape, logits_tf_out.shape)
         assert logits_out.requires_grad and logits_tf_out.requires_grad        # :110
         h, w = logits_out.shape[2], logits_out.shape[3]
@@ -143,18 +146,28 @@ class IIDSegmentationSmallPathLoss(IIDSegmentationLoss):
         return self((logits_out / T).softmax(1), (logits_tf_out / T).softmax(1))
 
 
-def iic_losses(calls):
+def iic_losses(calls, from_logits: bool = False, T: float = 1.0):
     """Evaluate many loss calls of one iteration TOGETHER: ``calls`` is a sequence of ``(criterion, x_out, x_tf_out)`` or
     ``(criterion, x_out, x_tf_out, mask)`` with ``criterion`` an :class:`IIDLoss`, :class:`IIDSegmentationLoss` or
     :class:`IIDSegmentationSmallPathLoss` instance; the result is the list ``[criterion(x_out, x_tf_out), ...]`` -- same
     values, same autograd behaviour -- but computed with one joint kernel per call and ONE finish launch for all of
     them (csrc/finish.cu): one slot reduction, one epilogue and, under ``set_data_parallel(True)``, ONE exchange of all
     joints.  This is the batched form of the (feature layer x sub-head) loop of ``IICTrainEpocher.regularization``
-    (semi_seg/epocher.py:249-277), where the reference issues S x L separate calls."""
+    (semi_seg/epocher.py:249-277), where the reference issues S x L separate calls.
+
+    ``from_logits=True``: every ``x_out`` / ``x_tf_out`` is a cluster head's LOGITS and the result is that of the calls
+    on ``softmax(x / T, 1)`` (the heads' ``SoftmaxWithT``, contrastyou/trainer/_utils.py:15-23).  Local terms whose shape
+    the fused kernels cover (:func:`from_logits_covered`, see :meth:`IIDSegmentationSmallPathLoss.from_logits`) take the
+    softmax inside their kernels; the others, and the global terms' (N, K) rows, get ``torch.softmax`` first.  Gradients
+    are with respect to the logits.  Masks are not accepted with ``from_logits``."""
     terms, post = [], []
+    inv_t = 1.0 / float(T)
     for c in calls:
         crit, x, y = c[0], c[1], c[2]
         mask = c[3] if len(c) > 3 else None
+        if from_logits and mask is not None:
+            raise ValueError("iic_losses(from_logits=True): masks are not supported; apply the softmax and pass the "
+                             "probabilities with the mask")
         if isinstance(crit, IIDSegmentationLoss):
             assert x.requires_grad and y.requires_grad                   # iic_loss.py:110
             if mask is not None:
@@ -165,10 +178,20 @@ def iic_losses(calls):
                 patch, step = crit._patch_size, crit._step_size
             else:
                 patch, step = (h, w), (h, w)
+            if from_logits:
+                one_patch = patch[0] >= h and patch[1] >= w
+                if one_patch and from_logits_covered(x, y, crit.padding):
+                    terms.append(LocalTerm(x, y, None, crit.padding, (h, w), (h, w), crit.lamda, logits=True,
+                                           inv_temperature=inv_t))
+                    post.append(None)
+                    continue
+                x, y = (x / T).softmax(1), (y / T).softmax(1)          # on the autograd tape, before the batched call
             terms.append(LocalTerm(x, y, mask, crit.padding, patch, step, crit.lamda))
             post.append(None)
         elif isinstance(crit, IIDLoss):
             assert x.dim() == 2 and y.shape == x.shape, (x.shape, y.shape)
+            if from_logits:
+                x, y = (x / T).softmax(1), (y / T).softmax(1)
             terms.append(GlobalTerm(x, y, crit.lamb, True))
             post.append(crit)
         else:

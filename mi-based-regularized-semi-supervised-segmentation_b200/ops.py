@@ -279,6 +279,40 @@ def _local_backward_logits(lx, ly, Wx, Wy, grad, pad, inv_temperature):
     return gx, gy
 
 
+def from_logits_covered(lx: torch.Tensor, ly: torch.Tensor, pad: int) -> bool:
+    """Whether a one-patch local term on the logit maps `lx`, `ly` runs with the cluster head's softmax fused into its
+    kernels (include/iic_b200.h: iic_local_from_logits_covered, the rule the kernels themselves follow); False means
+    the caller applies the softmax and takes the probability path."""
+    if not (lx.is_cuda and ly.is_cuda and lx.dtype == torch.float32 and ly.dtype == torch.float32):
+        return False
+    if lx.dim() != 4 or lx.shape != ly.shape or lx.stride(-1) != 1 or ly.stride(-1) != 1:
+        return False
+    lib = _lib.load()
+    B, K, H, W = lx.shape
+    rc = lib.iic_local_from_logits_covered(lx.device.index or 0, lx.data_ptr(), lx.stride(0), lx.stride(1), lx.stride(2),
+                                           ly.data_ptr(), ly.stride(0), ly.stride(1), ly.stride(2), B, K, H, W, int(pad))
+    if rc < 0:
+        _lib.check(rc, "iic_local_from_logits_covered")
+    return rc == 1
+
+
+def _local_backward_logits_stats_into(lx, ly, stats, Wx, Wy, grad, pad, inv_temperature, gx, gy):
+    """Backward of a fused from-logits term whose forward wrote `stats` (None on the K = 10 shapes)."""
+    lib = _lib.load()
+    lx, ly = _logit_maps(lx, ly)
+    B, K, H, W = lx.shape
+    grad = grad.to(torch.float32).reshape(())
+    with torch.cuda.device(lx.device):
+        rc = lib.iic_local_backward_from_logits_stats(lx.data_ptr(), lx.stride(0), lx.stride(1), lx.stride(2),
+                                                      ly.data_ptr(), ly.stride(0), ly.stride(1), ly.stride(2),
+                                                      B, K, H, W, pad, float(inv_temperature), _ptr(stats), Wx.data_ptr(),
+                                                      Wy.data_ptr(), grad.data_ptr(), gx.data_ptr(), gy.data_ptr(),
+                                                      gx.stride(0), gy.stride(0), _stream(lx.device))
+    if rc == _lib.UNSUPPORTED:
+        raise FusedShapeUnsupported(lib.iic_b200_last_error().decode())
+    _lib.check(rc, "iic_local_backward_from_logits_stats")
+
+
 def _global_joint(x, y, check_simplex=False):
     lib = _lib.load()
     _require_cuda_f32("x_out", x)
@@ -745,16 +779,20 @@ def _finish_terms(terms, check_simplex):
                 x, y = _w_contig(t.x), _w_contig(t.y)
                 B, K, H, W = x.shape
                 info = _lib.SlotInfo()
+                stats = None
                 if t.logits:
-                    nbytes = max(lib.iic_b200_sm_count(dev.index or 0) * 9 * K * K * 4, 4)
+                    nbytes = max(lib.iic_local_joint_from_logits_workspace_bytes(dev.index or 0, B, K, H, W, t.pad), 4)
                     ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-                    rc = lib.iic_local_joint_from_logits(x.data_ptr(), x.stride(0), x.stride(1), x.stride(2),
-                                                         y.data_ptr(), y.stride(0), y.stride(1), y.stride(2),
-                                                         B, K, H, W, t.pad, t.inv_temperature, None, ws.data_ptr(), nbytes,
-                                                         C.byref(info), _stream(dev))
+                    if 16 <= K <= 24:
+                        # per-pixel softmax statistics (m, r) of both maps, written by the joint, read by the backward
+                        stats = torch.empty(lib.iic_local_logit_stats_floats(B, H, W), dtype=torch.float32, device=dev)
+                    rc = lib.iic_local_joint_from_logits_stats(x.data_ptr(), x.stride(0), x.stride(1), x.stride(2),
+                                                               y.data_ptr(), y.stride(0), y.stride(1), y.stride(2),
+                                                               B, K, H, W, t.pad, t.inv_temperature, _ptr(stats), None,
+                                                               ws.data_ptr(), nbytes, C.byref(info), _stream(dev))
                     if rc == _lib.UNSUPPORTED:
                         raise FusedShapeUnsupported(lib.iic_b200_last_error().decode())
-                    _lib.check(rc, "iic_local_joint_from_logits")
+                    _lib.check(rc, "iic_local_joint_from_logits_stats")
                     npatch, m = 1, None
                 else:
                     m, msn, msc, msh = _mask_args(t.mask, x)
@@ -786,8 +824,8 @@ def _finish_terms(terms, check_simplex):
                 it.epilogue_workspace = st.epilogue_ws(K, t.pad, npatch, dev).data_ptr()      # used when the epilogue is not fused
                 it.loss_out, it.Wx, it.Wy = loss_buf[lo:].data_ptr(), Wx.data_ptr(), Wy.data_ptr()
                 E = npatch * T * T * K * K
-                recs.append(dict(kind="local", x=x, y=y, mask=m, Wx=Wx, Wy=Wy, loss=loss_buf[lo], K=K, T=T, npatch=npatch,
-                                 joff=E_total, E=E))
+                recs.append(dict(kind="local", x=x, y=y, mask=m, Wx=Wx, Wy=Wy, stats=stats, loss=loss_buf[lo], K=K, T=T,
+                                 npatch=npatch, joff=E_total, E=E))
                 keep.append(ws)
                 lo += 1
             else:
@@ -915,13 +953,14 @@ class IICTermsFunction(torch.autograd.Function):
             if r["kind"] == "local":
                 outs.append(r["loss"])
                 saved += [r["x"], r["y"], r["Wx"], r["Wy"]] + ([r["mask"]] if r["mask"] is not None else [])
+                saved += [r["stats"]] if r.get("stats") is not None else []
             else:
                 outs += [r["loss"], r["loss_nl"], r["P"]]
                 saved += [r["x"], r["y"], r["J"]]
         ctx.save_for_backward(*saved)
         ctx.meta = [(t.__class__, getattr(t, "pad", None), getattr(t, "patch", None), getattr(t, "step", None),
                      getattr(t, "logits", False), getattr(t, "inv_temperature", 1.0), getattr(t, "lamb", None),
-                     getattr(t, "symmetric", True), r.get("mask") is not None, r.get("npatch", 1))
+                     getattr(t, "symmetric", True), r.get("mask") is not None, r.get("npatch", 1), r.get("stats") is not None)
                     for t, r in zip(terms, recs)]
         ctx.slots = slots
         ctx.src_meta = [(tuple(s_.shape), s_.device) for s_ in sources]
@@ -992,7 +1031,7 @@ class IICTermsFunction(torch.autograd.Function):
         for m in ctx.meta:
             offs.append((si_, gi))
             if m[0] is LocalTerm:
-                si_ += 4 + (1 if m[8] else 0)
+                si_ += 4 + (1 if m[8] else 0) + (1 if m[10] else 0)
                 gi += 1
             else:
                 si_ += 3
@@ -1002,7 +1041,7 @@ class IICTermsFunction(torch.autograd.Function):
             # global terms first: their targets are allocated (and zero-filled where needed) on the main stream before the fork
             order.sort(key=lambda t_: ctx.meta[t_][0] is LocalTerm)
         for ti in order:
-            cls, pad, patch, step, logits, inv_t, lamb, symmetric, has_mask, npatch = ctx.meta[ti]
+            cls, pad, patch, step, logits, inv_t, lamb, symmetric, has_mask, npatch, has_stats = ctx.meta[ti]
             si_, gi = offs[ti]
             if cls is LocalTerm:
                 if use_side and side is None and gjobs:
@@ -1011,12 +1050,13 @@ class IICTermsFunction(torch.autograd.Function):
                     side.wait_stream(main)        # fork: upstream gradients and the global targets' zero fills are queued on main
                 x, y, Wx, Wy = sv[si_:si_ + 4]
                 mask = sv[si_ + 4] if has_mask else None
+                stats = sv[si_ + 4 + (1 if has_mask else 0)] if has_stats else None
                 g = grads[gi]
                 if g is None:
                     continue
                 (gx, ax), (gy, ay) = target(2 * ti, x), target(2 * ti + 1, y)
                 if logits:
-                    _local_backward_logits_into(x, y, Wx, Wy, g.contiguous(), pad, inv_t, gx, gy)
+                    _local_backward_logits_stats_into(x, y, stats, Wx, Wy, g.contiguous(), pad, inv_t, gx, gy)
                 else:
                     _local_backward_into(x, y, mask, Wx, Wy, g.contiguous(), pad, patch[0], patch[1], step[0], step[1], gx, gy)
             else:
@@ -1109,20 +1149,24 @@ class LocalIICFunction(torch.autograd.Function):
 class LocalIICLogitsFunction(torch.autograd.Function):
     """LocalIICFunction applied to softmax(logits / T, dim=1) of both maps, with the softmax and its
     backward fused into the joint and gradient kernels (contrastyou/trainer/_utils.py:15-23,137-168 feeding
-    iic_loss.py:107-149); one patch = the whole map.  Raises FusedShapeUnsupported for other shapes."""
+    iic_loss.py:107-149); one patch = the whole map.  Raises FusedShapeUnsupported for other shapes.  For 16 <= K <= 24
+    the forward also writes the per-pixel softmax statistics of both maps, kept with Wx / Wy for the backward."""
 
     @staticmethod
     def forward(ctx, lx, ly, pad, lamda, inv_temperature):
         t = LocalTerm(lx, ly, None, pad, lx.shape[2:], lx.shape[2:], lamda, logits=True, inv_temperature=inv_temperature)
         (r,) = _finish_terms([t], False)
-        ctx.save_for_backward(r["x"], r["y"], r["Wx"], r["Wy"])
+        ctx.save_for_backward(r["x"], r["y"], r["Wx"], r["Wy"], r["stats"])
         ctx.cfg = (pad, inv_temperature)
         return r["loss"]
 
     @staticmethod
     def backward(ctx, grad):
-        lx, ly, Wx, Wy = ctx.saved_tensors
-        gx, gy = ops.local_backward_logits(lx, ly, Wx, Wy, grad.contiguous(), *ctx.cfg)
+        lx, ly, Wx, Wy, stats = ctx.saved_tensors
+        B, K, H, W = lx.shape
+        gx = torch.empty((B, K, H, W), dtype=torch.float32, device=lx.device)
+        gy = torch.empty((B, K, H, W), dtype=torch.float32, device=lx.device)
+        _local_backward_logits_stats_into(lx, ly, stats, Wx, Wy, grad.contiguous(), ctx.cfg[0], ctx.cfg[1], gx, gy)
         return gx, gy, None, None, None
 
 

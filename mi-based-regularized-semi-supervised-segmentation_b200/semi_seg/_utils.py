@@ -108,19 +108,20 @@ def combine_iic_losses(losses_per_layer: Sequence[Sequence[Tensor]], feature_imp
 
 
 def iic_regularization(prob_pairs_per_layer: Sequence[Sequence], criteria: Sequence[nn.Module],
-                       feature_importance: Sequence[float]):
+                       feature_importance: Sequence[float], from_logits: bool = False, T: float = 1.0):
     """The value ``IICTrainEpocher.regularization`` computes (semi_seg/epocher.py:249-277) from the cluster heads' outputs:
     ``prob_pairs_per_layer[l]`` is the list of ``(prob1, prob2)`` pairs of layer ``l`` (one per sub-head, epocher.py:
     269-273), ``criteria[l]`` that layer's loss module (``IICLossWrapper[l]``).  All S x L loss calls go through
     :func:`iic_losses` -- one finish launch, one multi-GPU exchange -- and are combined by :func:`combine_iic_losses`
-    (``average_iter`` over sub-heads, ``weighted_average_iter`` over layers).  Returns ``(reg_loss, per_layer_losses)``."""
+    (``average_iter`` over sub-heads, ``weighted_average_iter`` over layers).  Returns ``(reg_loss, per_layer_losses)``.
+    ``from_logits=True``: the pairs are the heads' logits, as for :func:`iic_losses`."""
     assert len(prob_pairs_per_layer) == len(criteria) == len(feature_importance)
     calls, counts = [], []
     for pairs, crit in zip(prob_pairs_per_layer, criteria):
         pairs = list(pairs)
         counts.append(len(pairs))
         calls += [(crit, a, b) for a, b in pairs]
-    flat = iic_losses(calls)
+    flat = iic_losses(calls, from_logits=from_logits, T=T)
     per_layer, k = [], 0
     for c in counts:
         per_layer.append([l[0] if isinstance(l, tuple) else l for l in flat[k:k + c]])
