@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IIC_B200_ABI_VERSION 7
+#define IIC_B200_ABI_VERSION 8
 
 /* flag bits written (OR-ed) into the int* `flags` words by the kernels */
 #define IIC_FLAG_NAN_LOSS 1      /* iic_loss.py:147-148,184-185 -> RuntimeError on the host  */
@@ -161,8 +161,9 @@ int iic_local_backward_from_logits(const float* lx, long long x_sn, long long x_
                                    const float* Wx, const float* Wy, const float* grad_loss,
                                    float* g_lx, float* g_ly, long long gx_sn, long long gy_sn, void* stream);
 
-/* The same for the reference's default cluster count (16 <= K <= 24, padding 1 or 3; ABI 7).  Its tensor-core kernels
- * stage 8-channel slices and never hold a whole pixel, so a first pass writes per pixel of both maps
+/* The same for the reference's default cluster count (16 <= K <= 24, padding 1 or 3; ABI 7) and for the wide heads
+ * (K == 128, padding 1; ABI 8).  Their tensor-core kernels stage 8-channel slices or single channel rows and never hold
+ * a whole pixel, so a first pass writes per pixel of both maps
  *   m = max_k(l_k * inv_temperature),  r = 1 / sum_k exp(l_k * inv_temperature - m)
  * into the caller's `stats` buffer (iic_local_logit_stats_floats floats, 16-byte aligned: [2B][2][H][W], planes m and r,
  * lx at samples 0..B-1, ly at B..2B-1), and the kernels use p = exp(l * inv_temperature - m) * r.  The caller keeps
@@ -171,13 +172,16 @@ int iic_local_backward_from_logits(const float* lx, long long x_sn, long long x_
  *                                       strides as for the calls), 0 when the caller must apply the softmax and use
  *                                       the probability entry points; the ONE rule both calls follow.  16 <= K <= 24:
  *                                       padding 3, or padding 1 with enough row blocks to fill the SMs; W % 16 == 0;
- *                                       16-byte aligned rows; tensor-core and TMA kernels not switched off.  K == 10:
- *                                       the shapes of iic_local_joint_from_logits above.
+ *                                       16-byte aligned rows; tensor-core and TMA kernels not switched off.  K == 128:
+ *                                       padding 1; W % 16 == 0 and W <= 248; 16-byte aligned rows; tensor-core and TMA
+ *                                       kernels not switched off.  K == 10: the shapes of iic_local_joint_from_logits
+ *                                       above.
  *   iic_local_joint_from_logits_workspace_bytes   the workspace of the joint (per-SM slots of the kernel it selects)
  *   iic_local_joint_from_logits_stats   as iic_local_joint_from_logits, also writing stats; on a K == 10 shape it is
  *                                       that call (stats untouched, may be NULL); IIC_UNSUPPORTED when not covered
- *   iic_local_backward_from_logits_stats  its backward, reading stats; Wx / Wy are writable because the K = 20 kernels
- *                                       lay their weight images into the buffers' tails (iic_local_coeff_floats) */
+ *   iic_local_backward_from_logits_stats  its backward, reading stats; Wx / Wy are writable because the K = 20 and
+ *                                       K = 128 kernels lay their weight images into the buffers' tails
+ *                                       (iic_local_coeff_floats) */
 size_t iic_local_logit_stats_floats(int B, int H, int W);
 size_t iic_local_joint_from_logits_workspace_bytes(int device, int B, int K, int H, int W, int pad);
 int iic_local_from_logits_covered(int device, const float* lx, long long x_sn, long long x_sc, long long x_sh,
@@ -217,6 +221,15 @@ int iic_global_backward(const float* x, long long x_sn, const float* y, long lon
                         long long N, int K, const double* J, double lamb, int symmetric,
                         const float* g_loss, const float* g_no_lamb, const float* gP,
                         float* gx, float* gy, long long gx_sn, long long gy_sn, void* stream);
+/* The same when x and y are the cluster head's LOGITS and J is the joint of softmax(x * inv_temperature) and
+ * softmax(y * inv_temperature) (an IIC_ITEM_GLOBAL_LOGITS term of iic_finish; ABI 8): the gradients are with respect to
+ * the logits, d l_k = inv_temperature * p_k * (dp_k - sum_c dp_c p_c) per row, with p computed exactly as the finish
+ * launch computed it.  K <= 128. */
+int iic_global_backward_from_logits(const float* x, long long x_sn, const float* y, long long y_sn,
+                                    long long N, int K, const double* J, double lamb, int symmetric,
+                                    float inv_temperature, const float* g_loss, const float* g_no_lamb,
+                                    const float* gP, float* gx, float* gy, long long gx_sn, long long gy_sn,
+                                    void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * iic_finish: ONE launch between the joint kernels and the backward kernels of one or many IIC terms -- the (layer,
@@ -234,8 +247,11 @@ int iic_global_backward(const float* x, long long x_sn, const float* y, long lon
  * ---------------------------------------------------------------------------------------------- */
 #define IIC_ITEM_LOCAL 0
 #define IIC_ITEM_GLOBAL_ROWS 1
+#define IIC_ITEM_GLOBAL_LOGITS 2    /* global term on logit rows: the joint of softmax(x * inv_temperature) and
+                                       softmax(y * inv_temperature), each row normalised inside the launch (no simplex
+                                       check: a softmax row is one); N <= 4096, K <= 128; ABI 8 */
 typedef struct iic_finish_item {
-  int kind;                       /* IIC_ITEM_LOCAL or IIC_ITEM_GLOBAL_ROWS */
+  int kind;                       /* IIC_ITEM_LOCAL, IIC_ITEM_GLOBAL_ROWS or IIC_ITEM_GLOBAL_LOGITS */
   int K;
   double lamda;                   /* lamda of IIDSegmentationLoss / lamb of IIDLoss */
   /* local term: the slots left by iic_local_joint_partials and its geometry */
@@ -255,6 +271,7 @@ typedef struct iic_finish_item {
   float* Wx;
   float* Wy;
   float* P_out;
+  float inv_temperature;          /* IIC_ITEM_GLOBAL_LOGITS: 1 / T of the head's softmax */
 } iic_finish_item;
 size_t iic_finish_workspace_bytes(void);
 int iic_finish(const iic_finish_item* items_host, int n_items, double* J_all, long long E_total, int* flags,

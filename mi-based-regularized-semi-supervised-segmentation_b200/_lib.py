@@ -10,13 +10,14 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libiic_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 FLAG_NAN_LOSS = 1
 FLAG_NOT_SIMPLEX = 2
 FLAG_BAD_LABEL = 4
 FLAG_XCHG_TIMEOUT = 8
 ITEM_LOCAL = 0
 ITEM_GLOBAL_ROWS = 1
+ITEM_GLOBAL_LOGITS = 2
 UNSUPPORTED = 3
 FLIP_H = 1      # axis 1 of a (C, H, W) sample
 FLIP_W = 2      # axis 2
@@ -63,6 +64,8 @@ PROTOTYPES = {
     "iic_global_joint": (_i, [_p, _ll, _p, _ll, _ll, _i, _p, _p, _sz, _p, _p]),
     "iic_global_epilogue": (_i, [_p, _i, _d, _i, _p, _p, _p, _p]),
     "iic_global_backward": (_i, [_p, _ll, _p, _ll, _ll, _i, _p, _d, _i, _p, _p, _p, _p, _p, _ll, _ll, _p]),
+    "iic_global_backward_from_logits": (_i, [_p, _ll, _p, _ll, _ll, _i, _p, _d, _i, C.c_float, _p, _p, _p, _p, _p, _ll,
+                                             _ll, _p]),
     "iic_uda_workspace_bytes": (_sz, [_i]),
     "iic_uda_forward": (_i, [_p, _p, _ll, _i, _ll, _i, _d, _p, _i, _p, _p, _i, _p, _p]),
     "iic_uda_backward": (_i, [_p, _p, _ll, _i, _ll, _i, _d, _p, _i, _p, _p, _p]),
@@ -95,7 +98,7 @@ class FinishItem(C.Structure):
                 ("pad", _i), ("n_patches", _i), ("epilogue_workspace", _p),
                 ("x", _p), ("x_sn", _ll), ("y", _p), ("y_sn", _ll), ("N", _ll),
                 ("symmetric", _i), ("check_simplex", _i),
-                ("loss_out", _p), ("Wx", _p), ("Wy", _p), ("P_out", _p)]
+                ("loss_out", _p), ("Wx", _p), ("Wy", _p), ("P_out", _p), ("inv_temperature", C.c_float)]
 
 
 _lib = None

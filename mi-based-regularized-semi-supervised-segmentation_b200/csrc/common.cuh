@@ -182,4 +182,29 @@ __device__ __forceinline__ double block_min_nan(double v, bool has_nan, double* 
   return scratch[32];
 }
 
+// ---- the cluster head's softmax from per-pixel / per-row statistics ---------------------------------------
+// p = softmax(l * inv_temp) from m = max_k(l_k * inv_temp) and r = 1 / sum_k exp(l_k * inv_temp - m): the product is
+// rounded on its own (__fmul_rn, never contracted into an FMA), so every kernel that converts the same logit gets the
+// same bits.  r = 0 (a TMA zero fill outside the map) gives p = 0.
+__device__ __forceinline__ float logit_p(float l, float inv_temp, float m, float r) {
+  return __expf(__fmul_rn(l, inv_temp) - m) * r;
+}
+
+// (m, r) of one row of K logits, held by the 32 lanes of a warp (lane k takes k, k + 32, ...): the max is exact, the
+// sum adds each lane's terms in index order and then the lanes in a fixed butterfly, so every lane gets the same bits
+// and every caller that uses this function gets the same (m, r).
+__device__ __forceinline__ void warp_row_softmax_stats(const float* __restrict__ row, int K, float inv_temp, float* m_out,
+                                                       float* r_out) {
+  const int lane = threadIdx.x & 31;
+  float mx = -INFINITY;
+  for (int k = lane; k < K; k += 32) mx = fmaxf(mx, __fmul_rn(row[k], inv_temp));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  float s = 0.f;
+  for (int k = lane; k < K; k += 32) s += __expf(__fmul_rn(row[k], inv_temp) - mx);
+  s = warp_sum(s);
+  *m_out = mx;
+  *r_out = 1.f / s;
+}
+
 }  // namespace iic

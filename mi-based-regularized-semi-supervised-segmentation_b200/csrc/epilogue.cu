@@ -138,12 +138,17 @@ constexpr int GLOBAL_BWD_STAGE_FLOATS = 2048;      // rows of x (and of y) stage
 // Every CTA rebuilds GJ = d(objective)/dJ in shared memory, then produces a slab of rows of gx = y GJ^T and gy = x GJ.
 // The joint is read from global memory ONCE (symmetrised into shared memory); the kernel is a chain of small dependent
 // phases, so every phase that went back to global memory for J cost a memory latency (19k cycles at (32, 10) before).
+// From-logits form (FL): x and y are logit rows and J the joint of their softmax(l * inv_temp) (iic_finish's
+// IIC_ITEM_GLOBAL_LOGITS).  One warp per row recomputes p of both rows with the finish launch's own functions
+// (warp_row_softmax_stats, logit_p: the same bits), forms dp = GJ p and applies the softmax adjoint
+// inv_temp * p * (dp - <dp, p>) to both rows.
+template <bool FL>
 __global__ void __launch_bounds__(256) global_backward_kernel(
     const float* __restrict__ x, long long x_sn, const float* __restrict__ y, long long y_sn, long long N,
     int K, const double* __restrict__ J, double lamb, int symmetric, const float* __restrict__ g_loss,
     const float* __restrict__ g_no_lamb, const float* __restrict__ gP, float* __restrict__ gx,
     float* __restrict__ gy, long long gx_sn, long long gy_sn,
-    long long rows_per_cta) {
+    long long rows_per_cta, float inv_temp) {
   extern __shared__ __align__(16) double sm[];
   double* scratch = sm;            // 33
   double* pi = sm + 40;            // K
@@ -163,7 +168,7 @@ __global__ void __launch_bounds__(256) global_backward_kernel(
   // A small slab (config 2: 32 rows of 10) is staged in shared memory now, so that its global-memory latency overlaps the
   // epilogue phases below instead of sitting in the row loop (K dependent loads per output there: ~6000 clk at K = 10).
   const long long slab = (r1 - r0) * K;
-  const bool staged_rows = slab <= GLOBAL_BWD_STAGE_FLOATS;
+  const bool staged_rows = !FL && slab <= GLOBAL_BWD_STAGE_FLOATS;     // (FL: rows_s holds per-warp p rows)
   if (staged_rows)
     for (long long e = tid; e < slab; e += nt) {
       const long long n = r0 + e / K;
@@ -213,6 +218,51 @@ __global__ void __launch_bounds__(256) global_backward_kernel(
     GJ[e] = (float)v;
   }
   __syncthreads();
+  if constexpr (FL) {
+    const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
+    float* px = rows_s + (size_t)wid * 2 * K;        // this warp's p rows of x and y
+    float* py = px + K;
+    for (long long n = r0 + wid; n < r1; n += nw) {
+      const float* xr = x + n * x_sn;
+      const float* yr = y + n * y_sn;
+      float mx, rx, my, ry;
+      warp_row_softmax_stats(xr, K, inv_temp, &mx, &rx);
+      warp_row_softmax_stats(yr, K, inv_temp, &my, &ry);
+      for (int k = lane; k < K; k += 32) {
+        px[k] = logit_p(xr[k], inv_temp, mx, rx);
+        py[k] = logit_p(yr[k], inv_temp, my, ry);
+      }
+      __syncwarp();
+      // dp of the row (lane c takes channels c, c + 32, ...: K <= 128), then the two dot products
+      float ax[4], ay[4];
+      float dx = 0.f, dy = 0.f;
+#pragma unroll
+      for (int h = 0; h < 4; ++h) {
+        const int c = lane + 32 * h;
+        ax[h] = 0.f; ay[h] = 0.f;
+        if (c < K) {
+          for (int q = 0; q < K; ++q) {
+            ax[h] = fmaf(GJ[(size_t)c * K + q], py[q], ax[h]);
+            ay[h] = fmaf(GJ[(size_t)q * K + c], px[q], ay[h]);
+          }
+          dx = fmaf(ax[h], px[c], dx);
+          dy = fmaf(ay[h], py[c], dy);
+        }
+      }
+      dx = warp_sum(dx);
+      dy = warp_sum(dy);
+#pragma unroll
+      for (int h = 0; h < 4; ++h) {
+        const int c = lane + 32 * h;
+        if (c < K) {
+          gx[n * gx_sn + c] = inv_temp * px[c] * (ax[h] - dx);
+          gy[n * gy_sn + c] = inv_temp * py[c] * (ay[h] - dy);
+        }
+      }
+      __syncwarp();                                  // px / py are rewritten for the next row
+    }
+    return;
+  }
   // gx[n][i] = sum_j GJ[i][j] y[n][j] ; gy[n][j] = sum_i GJ[i][j] x[n][i]
   const long long total = (r1 - r0) * K;
   for (long long e = tid; e < total; e += nt) {
@@ -334,12 +384,35 @@ extern "C" int iic_global_backward(const float* x, long long x_sn, const float* 
   long long rpc;
   const int ctas = global_grid(current_device(), N, &rpc);
   const size_t smem = (40 + 4 * (size_t)K + (size_t)K * K) * sizeof(double) + ((size_t)K * K + 2 * GLOBAL_BWD_STAGE_FLOATS) * sizeof(float);
-  auto kern = global_backward_kernel;
+  auto kern = global_backward_kernel<false>;
   // opted in once per device, for the largest K the entry point takes (128)
   if (smem > 48 * 1024) IIC_CHECK_RC(ensure_dyn_smem((const void*)kern, (int)((40 + 4 * 128 + 128 * 128) * sizeof(double) + (128 * 128 + 2 * GLOBAL_BWD_STAGE_FLOATS) * sizeof(float))));
   if (gx_sn <= 0) gx_sn = K;            // 0 = dense rows
   if (gy_sn <= 0) gy_sn = K;
-  kern<<<ctas, 256, smem, st>>>(x, x_sn, y, y_sn, N, K, J, lamb, symmetric, g_loss, g_no_lamb, gP, gx, gy, gx_sn, gy_sn, rpc);
+  kern<<<ctas, 256, smem, st>>>(x, x_sn, y, y_sn, N, K, J, lamb, symmetric, g_loss, g_no_lamb, gP, gx, gy, gx_sn, gy_sn, rpc,
+                                1.f);
+  IIC_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int iic_global_backward_from_logits(const float* x, long long x_sn, const float* y, long long y_sn,
+                                               long long N, int K, const double* J, double lamb, int symmetric,
+                                               float inv_temperature, const float* g_loss, const float* g_no_lamb,
+                                               const float* gP, float* gx, float* gy, long long gx_sn, long long gy_sn,
+                                               void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  IIC_REQUIRE(x && y && J && gx && gy, "iic_global_backward_from_logits: null pointer");
+  IIC_REQUIRE(N > 0 && K > 0 && K <= 128, "iic_global_backward_from_logits: bad sizes N=%lld K=%d", N, K);
+  long long rpc;
+  const int ctas = global_grid(current_device(), N, &rpc);
+  // the probability form's layout; its row stage holds the 8 warps' p rows (2 * 8 * 128 <= 2 * GLOBAL_BWD_STAGE_FLOATS)
+  const size_t smem = (40 + 4 * (size_t)K + (size_t)K * K) * sizeof(double) + ((size_t)K * K + 2 * GLOBAL_BWD_STAGE_FLOATS) * sizeof(float);
+  auto kern = global_backward_kernel<true>;
+  if (smem > 48 * 1024) IIC_CHECK_RC(ensure_dyn_smem((const void*)kern, (int)((40 + 4 * 128 + 128 * 128) * sizeof(double) + (128 * 128 + 2 * GLOBAL_BWD_STAGE_FLOATS) * sizeof(float))));
+  if (gx_sn <= 0) gx_sn = K;            // 0 = dense rows
+  if (gy_sn <= 0) gy_sn = K;
+  kern<<<ctas, 256, smem, st>>>(x, x_sn, y, y_sn, N, K, J, lamb, symmetric, g_loss, g_no_lamb, gP, gx, gy, gx_sn, gy_sn, rpc,
+                                inv_temperature);
   IIC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

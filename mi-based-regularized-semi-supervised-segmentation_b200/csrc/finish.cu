@@ -2,7 +2,8 @@
 // launch --
 //   phase 1 (all CTAs)   fixed-order fp64 reduction of the joint kernels' per-CTA partial slots into the joints J
 //                        (what reduce_partials_kernel / reduce_packed_kernel do per term), the small global joints
-//                        x^T y computed directly from the (N, K) rows (contrastyou/losses/iic_loss.py:88-89); under data
+//                        x^T y computed directly from the (N, K) rows (contrastyou/losses/iic_loss.py:88-89) -- or from
+//                        the cluster head's logits, each row turned into softmax(l * inv_temp) on the way; under data
 //                        parallelism every value is also stored into this rank's slot of every peer's exchange buffer;
 //   phase 2 (last CTA)   [data parallel: publish the sequence number to every peer, wait for theirs, add the ranks'
 //                        slots in rank order -- csrc/xchg.cu's protocol, ONE exchange for all terms of the iteration]
@@ -30,6 +31,9 @@ constexpr int FIN_SMALL_UNITS = 32;        // the last CTA runs the epilogues it
 constexpr int FIN_BIG_MAX_UNITS = 16384;   // displacement units of one batched epilogue launch (workspace: one double each)
 constexpr size_t FIN_WS_TICKETS = 64;      // workspace: [0] phase-1 ticket, [1] rank-sum ticket; per-term tickets from here
 constexpr size_t FIN_WS_LOSSES = 256;      // workspace: unit losses from here
+constexpr int FIN_GLOBAL_LOGITS_MAX_N = 4096;    // rows of a global term from logits (ops.py: GLOBAL_ROWS_MAX)
+constexpr int FIN_GL_EPT = 8;              // joint entries per thread and pass of a global term from logits
+constexpr int FIN_PST_FLOATS = FIN_WARPS * 3 * FIN_MAX_K * 2;   // p rows staged by a global term from logits (wscratch)
 
 struct FinItem {
   const float* slots;            // local terms: per-CTA partial joints
@@ -43,9 +47,11 @@ struct FinItem {
   float* P_out;                  // global: (K, K) float32, nullable
   long long E;                   // local n_patches*T*T*K*K; global K*K
   long long slot_stride;
-  int kind;                      // IIC_ITEM_LOCAL / IIC_ITEM_GLOBAL_ROWS
+  int kind;                      // IIC_ITEM_LOCAL / IIC_ITEM_GLOBAL_ROWS (also for IIC_ITEM_GLOBAL_LOGITS: see inv_temp)
   int layout, n_slots, nb;
   int K, T, n_patches, symmetric, check_simplex;
+  float inv_temp;                // > 0: a global term whose x / y hold logits, its joint that of softmax(l * inv_temp);
+                                 // 0: probability rows.  (In the padding before lamda: the struct keeps its layout.)
   double lamda;
 };
 
@@ -160,6 +166,73 @@ __device__ void global_rows_unit(const FinBatch& B, const FinItem& it, double* s
       if (!(fabsf(sum - 1.f) <= 1e-4f + 1e-4f * 1.f)) bad = true;
     }
     if (bad) atomicOr(B.flags, IIC_FLAG_NOT_SIMPLEX);
+  }
+}
+
+// The same joint from LOGIT rows: the rows are turned into p = softmax(l * inv_temp) chunk by chunk (one warp per row,
+// warp_row_softmax_stats + logit_p: the p global_backward_kernel<true> recomputes, bit for bit) into `pst`, then
+// accumulated in fp64 in a fixed order as above -- group g takes the rows n = g mod G of every chunk in increasing n.
+// With one group (K > 32) a thread holds at most FIN_GL_EPT entries, so K*K > FIN_GL_EPT * 1024 (K > 90) takes more than
+// one pass over the rows (finish_kernel runs at 64 registers per thread: with 8 accumulators ptxas reports 68 / 60 bytes
+// of spill stores / loads, against 44 / 40 without this unit and 140 / 184 with 16).  No simplex assertion: a softmax
+// row is a simplex by construction.
+__device__ void global_logit_rows_unit(const FinBatch& B, const FinItem& it, double* scratch /* FIN_WARPS*33 doubles */,
+                                       float* pst /* FIN_PST_FLOATS */, int par) {
+  const int K = it.K, KK = K * K;
+  const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  int G = FIN_THREADS / KK;
+  if (G > FIN_WARPS * 33 / KK) G = FIN_WARPS * 33 / KK;
+  if (G < 1) G = 1;
+  const int g = threadIdx.x / KK;                         // G == 1: group 0 holds entries e = tid + q * FIN_THREADS
+  const int e0 = G == 1 ? threadIdx.x : threadIdx.x - g * KK;
+  const int rows_per_chunk = FIN_PST_FLOATS / (2 * K);
+  const int per_pass = G == 1 ? FIN_GL_EPT * FIN_THREADS : KK;
+  for (int eb = 0; eb < KK; eb += per_pass) {
+    double acc[FIN_GL_EPT];
+#pragma unroll
+    for (int q = 0; q < FIN_GL_EPT; ++q) acc[q] = 0.0;
+    __syncthreads();                                      // pst and scratch are reused from the previous unit / pass
+    for (long long n0 = 0; n0 < it.N; n0 += rows_per_chunk) {
+      const int nr = (int)(it.N - n0 < rows_per_chunk ? it.N - n0 : rows_per_chunk);
+      for (int rr = wid; rr < 2 * nr; rr += FIN_WARPS) {  // x rows of the chunk at pst[0 .. nr*K), then its y rows
+        const float* row = rr < nr ? it.x + (n0 + rr) * it.x_sn : it.y + (n0 + rr - nr) * it.y_sn;
+        float m, r;
+        warp_row_softmax_stats(row, K, it.inv_temp, &m, &r);
+        for (int k = lane; k < K; k += 32) pst[rr * K + k] = logit_p(row[k], it.inv_temp, m, r);
+      }
+      __syncthreads();
+      const float* px = pst;
+      const float* py = pst + (size_t)nr * K;
+      if (g < G) {
+        const int nfirst = (int)((g - n0 % G + G) % G);
+#pragma unroll
+        for (int q = 0; q < FIN_GL_EPT; ++q) {
+          const int e = eb + e0 + q * FIN_THREADS;
+          if ((q == 0 || G == 1) && e < KK) {
+            const int i = e / K, j = e - i * K;
+            double a = acc[q];
+            for (int n = nfirst; n < nr; n += G) a += (double)px[n * K + i] * (double)py[n * K + j];
+            acc[q] = a;
+          }
+        }
+      }
+      __syncthreads();
+    }
+    if (G == 1) {
+#pragma unroll
+      for (int q = 0; q < FIN_GL_EPT; ++q) {
+        const int e = eb + e0 + q * FIN_THREADS;
+        if (g == 0 && e < KK) store_joint(B, it, e, acc[q], par);
+      }
+    } else {
+      if (g < G) scratch[g * KK + e0] = acc[0];
+      __syncthreads();
+      if (threadIdx.x < KK) {
+        double t = 0.0;
+        for (int q = 0; q < G; ++q) t += scratch[q * KK + threadIdx.x];
+        store_joint(B, it, threadIdx.x, t, par);
+      }
+    }
   }
 }
 
@@ -324,8 +397,12 @@ __global__ void __launch_bounds__(FIN_THREADS, 1) finish_kernel(const __grid_con
       long long first = blockIdx.x - (base % gridDim.x);
       if (first < 0) first += gridDim.x;
       for (long long u = first; u < nu; u += gridDim.x) {
-        if (it.kind == IIC_ITEM_GLOBAL_ROWS) global_rows_unit(B, it, &sm[0][0], par);
-        else reduce_unit(B, it, u, sm, par);
+        if (it.kind == IIC_ITEM_GLOBAL_ROWS) {
+          if (it.inv_temp > 0.f) global_logit_rows_unit(B, it, &sm[0][0], reinterpret_cast<float*>(&wscratch[0][0]), par);
+          else global_rows_unit(B, it, &sm[0][0], par);
+        } else {
+          reduce_unit(B, it, u, sm, par);
+        }
       }
       base += nu;
     }
@@ -591,9 +668,15 @@ extern "C" int iic_finish(const iic_finish_item* items_host, int n_items, double
   for (int i = 0; i < n_items; ++i) {
     const iic_finish_item& s = items_host[i];
     FinItem& d = B.it[i];
-    IIC_REQUIRE(s.kind == IIC_ITEM_LOCAL || s.kind == IIC_ITEM_GLOBAL_ROWS, "iic_finish: term %d has unknown kind %d", i, s.kind);
+    IIC_REQUIRE(s.kind == IIC_ITEM_LOCAL || s.kind == IIC_ITEM_GLOBAL_ROWS || s.kind == IIC_ITEM_GLOBAL_LOGITS,
+                "iic_finish: term %d has unknown kind %d", i, s.kind);
     IIC_REQUIRE(s.K > 0, "iic_finish: term %d has K = %d", i, s.K);
-    d.kind = s.kind;
+    // a global term from logits is a global term whose phase-1 unit applies the softmax first
+    const bool logits = s.kind == IIC_ITEM_GLOBAL_LOGITS;
+    IIC_REQUIRE(!logits || (s.inv_temperature > 0.f && s.inv_temperature <= 3.0e38f),
+                "iic_finish: global term %d from logits needs a positive, finite inv_temperature", i);
+    d.kind = logits ? IIC_ITEM_GLOBAL_ROWS : s.kind;
+    d.inv_temp = logits ? s.inv_temperature : 0.f;
     d.K = s.K;
     d.lamda = s.lamda;
     d.J = J_all + off;
@@ -617,12 +700,15 @@ extern "C" int iic_finish(const iic_finish_item* items_host, int n_items, double
     } else {
       IIC_REQUIRE(s.x && s.y && s.N > 0, "iic_finish: global term %d is malformed", i);
       IIC_REQUIRE(s.K <= FIN_MAX_K * 4 && s.N <= (1 << 20), "iic_finish: global term %d too large for the direct joint", i);
+      IIC_REQUIRE(!logits || s.N <= FIN_GLOBAL_LOGITS_MAX_N,
+                  "iic_finish: global term %d from logits has %lld rows (at most %d; apply the softmax first)", i, s.N,
+                  FIN_GLOBAL_LOGITS_MAX_N);
       d.x = s.x; d.y = s.y; d.x_sn = s.x_sn; d.y_sn = s.y_sn; d.N = s.N;
       d.T = 1;
       d.n_patches = 1;
       d.E = (long long)s.K * s.K;
       d.symmetric = s.symmetric;
-      d.check_simplex = s.check_simplex;
+      d.check_simplex = logits ? 0 : s.check_simplex;
       d.P_out = s.P_out;
       epi_units += 1;
     }

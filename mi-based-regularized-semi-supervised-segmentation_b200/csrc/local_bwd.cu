@@ -313,8 +313,9 @@ extern "C" int iic_local_backward_from_logits(const float* lx, long long x_sn, l
 }
 
 // Backward of iic_local_joint_from_logits_stats: the stats are the ones its forward wrote.  16 <= K <= 24 where
-// local_fl_tc_covered holds: row-block tensor-core sweeps on the logits (their weight images go into the tails of Wx / Wy,
-// hence float*); the K = 10 shapes as iic_local_backward_from_logits.
+// local_fl_tc_covered holds: row-block tensor-core sweeps on the logits; K = 128 where local_fl_tc128_covered holds: the
+// tc sweeps on the logits (both lay their weight images into the tails of Wx / Wy, hence float*); the K = 10 shapes as
+// iic_local_backward_from_logits.
 extern "C" int iic_local_backward_from_logits_stats(const float* lx, long long x_sn, long long x_sc, long long x_sh,
                                                     const float* ly, long long y_sn, long long y_sc, long long y_sh,
                                                     int B, int K, int H, int W, int pad, float inv_temperature,
@@ -326,15 +327,17 @@ extern "C" int iic_local_backward_from_logits_stats(const float* lx, long long x
   const int sms = sm_count_cached(current_device());
   IIC_REQUIRE(sms > 0, "iic_local_backward_from_logits_stats: no device");
   const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
-  if (!local_fl_tc_covered(m))
+  const bool wide = local_fl_tc128_covered(m);
+  if (!wide && !local_fl_tc_covered(m))
     return iic_local_backward_from_logits(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, inv_temperature, Wx,
                                           Wy, grad_loss, g_lx, g_ly, gx_sn, gy_sn, stream);
   IIC_REQUIRE(stats, "iic_local_backward_from_logits_stats: null stats");
   if (gx_sn <= 0) gx_sn = (long long)K * H * W;
   if (gy_sn <= 0) gy_sn = (long long)K * H * W;
   const LocalGrads gr{grad_loss, g_lx, g_ly, gx_sn, gy_sn};
-  const int rc = local_bwd_tcrb_fl_try(m, stats, inv_temperature, Wx, Wy, gr, st);
+  const int rc = wide ? local_bwd_tc_fl_try(m, stats, inv_temperature, Wx, Wy, gr, st)
+                      : local_bwd_tcrb_fl_try(m, stats, inv_temperature, Wx, Wy, gr, st);
   if (rc > 0) return rc;
-  IIC_REQUIRE(rc == 0, "iic_local_backward_from_logits_stats: the row-block tensor-core backward refused a covered shape");
+  IIC_REQUIRE(rc == 0, "iic_local_backward_from_logits_stats: the tensor-core backward refused a covered shape");
   return 0;
 }

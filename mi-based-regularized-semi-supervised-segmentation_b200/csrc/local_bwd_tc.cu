@@ -25,6 +25,16 @@
 //              chunk; bf16: chunk 0 = al, chunk 1 = ah of the 8 channels)
 //   warps 1-2  MMA issuers (one lane each, one output row each): 9 taps x 2 tiles x 2 MMAs per slice and row
 //   warps 8-11 epilogue after the 16th slice: tcgen05.ld (lane = pixel, columns = channels), scale by g, coalesced stores
+//
+// From-logits form (FL, the cluster head's SoftmaxWithT fused): the maps hold logits.  Once per item the TMA warp also
+// stages the (m, r) of the item's four source rows (local_logit_stats_kernel, local_logits.cu; one 8 KB buffer behind
+// the raw ring, freed by the transform after the item's last slice), and the transform converts each 8-channel slice to
+// p = exp(l * inv_temp - m) * r (logit_p, common.cuh; r = 0 in the TMA zero fill outside the map, so p stays 0 there).
+// The epilogue holds all 128 accumulator channels g_o of its pixel (lane = pixel) and applies the softmax adjoint
+//   d logit_o = inv_temp * p_o * (g_o - sum_k g_k p_k)
+// in two passes over TMEM: the first forms the dot product, the second the gradient; p is recomputed in the second from
+// the OUTPUT pixel's logits and (m, r) with the same instructions, so both passes see the same p.  The item's output
+// logits are pulled into L2 while its MMAs run.
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -50,6 +60,10 @@ constexpr int NW = 6;
 constexpr int RAW_HALF_MAX = SL * 2 * 256 * 4;   // 16384 (8 ch x 2 rows x up to 256 px)
 constexpr int SMEM_BYTES = NA * A_SLOT + NW * W_TILE + 2 * RAW_HALF_MAX + 1024;
 constexpr int NTHREADS = 384;
+// FL: behind the raw ring, the item's stats [2 planes][4 rows][W + 8] and the two barriers of that buffer
+constexpr int FL_STATS_MAX = 2 * 4 * 256 * 4;    // 8192
+constexpr int FL_SMEM_BYTES = SMEM_BYTES + FL_STATS_MAX + 16;
+static_assert((NA * A_SLOT + NW * W_TILE + 2 * RAW_HALF_MAX) % 128 == 0, "the stats buffer is a TMA destination");
 
 
 struct Params {
@@ -60,6 +74,16 @@ struct Params {
   float* out;                   // (B, 128, H, W), channel planes dense
   long long out_sn;             // sample stride of `out` in elements
   int dbg;                      // bring-up switches (IIC_TC_DBG): 1 no source loads, 2 no weight loads, 4 no transform, 8 no stores
+};
+
+// the from-logits form's extra arguments (unused by the probability instantiation)
+struct FLParams {
+  CUtensorMap stats;            // the (2B, 2, H, W) stats tensor, box [2][4][W + 8]: x stats at n, y stats at B + n
+  int src_n;                    // stats sample offset of the source map (B for y, 0 for x)
+  float inv_temp;
+  const float* lout;            // logits of the OUTPUT map (its gradient is `out`), strides below
+  long long l_sn, l_sc, l_sh;
+  const float* sout;            // its (m, r) planes: sample n at sout + n * 2HW
 };
 
 // Wc[cin][tap][128] (iic_local_epilogue) -> operand image: the fp32 tile and the bf16 correction tile [wh | wl]
@@ -77,8 +101,9 @@ __global__ void weight_image_kernel(const float* __restrict__ Wc, float* __restr
   reinterpret_cast<uint4*>(dst)[3 * KC + o] = pack8<true>(v);      // wl (pairs with ah)
 }
 
+template <bool FL>
 __global__ void __launch_bounds__(NTHREADS, 1)
-local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
+local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P, const __grid_constant__ FLParams F) {
   extern __shared__ __align__(1024) unsigned char smem_dyn[];
   __shared__ __align__(8) uint64_t raw_full[2], raw_empty[2], a_full[NA], a_empty[NA], w_full[NW], w_empty[NW], accum_full, tmem_empty;
   __shared__ uint32_t tmem_base_s;
@@ -94,8 +119,12 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
   const int SW = P.W + 8;                                  // staged columns: -4 .. W+3
   const int raw_half_bytes = SL * 2 * SW * 4;
   const int ntile = P.W > 128 ? 2 : 1;
+  // FL: the item's stats and their full / empty barriers (dynamic shared memory: the probability form keeps its layout)
+  float* fl_stats = reinterpret_cast<float*>(raw_ring + 2 * RAW_HALF_MAX);
+  uint64_t* fl_bar = reinterpret_cast<uint64_t*>(raw_ring + 2 * RAW_HALF_MAX + FL_STATS_MAX);
 
   if (threadIdx.x == 0) {
+    if constexpr (FL) { mbar_init(&fl_bar[0], 1); mbar_init(&fl_bar[1], 4); }
     for (int s = 0; s < 2; ++s) { mbar_init(&raw_full[s], 1); mbar_init(&raw_empty[s], 4); }
     for (int s = 0; s < NA; ++s) { mbar_init(&a_full[s], 4); mbar_init(&a_empty[s], 2); }
     for (int s = 0; s < NW; ++s) { mbar_init(&w_full[s], 1); mbar_init(&w_empty[s], 2); }
@@ -116,9 +145,15 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
     // ===== TMA producer: source rows =====
     if (lane == 0) {
       tma_prefetch_desc(&maps);
+      if constexpr (FL) tma_prefetch_desc(&F.stats);
       for (int i = 0; i < nit; ++i) {
         const int item = it0 + i;
         const int n = item / pairs, r = (item - n * pairs) * 2;
+        if constexpr (FL) {                                 // the four source rows' (m, r), once per item
+          if (i >= 1) mbar_wait(&fl_bar[1], ((unsigned)i & 1u) ^ 1u, 9);
+          mbar_arrive_expect_tx(&fl_bar[0], 2 * 4 * SW * 4);
+          tma_load_4d(fl_stats, &F.stats, &fl_bar[0], -4, r - 1, 0, F.src_n + n);
+        }
         for (int js = 0; js < NSL; ++js) {
           const int t = i * NSL + js;
 #pragma unroll
@@ -214,6 +249,9 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
       const int a = t % NA;
       if (t >= NA) mbar_wait(&a_empty[a], ((unsigned)(t / NA) & 1u) ^ 1u, 3);
       unsigned char* ahi = a_ring + (size_t)a * A_SLOT;
+      if constexpr (FL) {
+        if (t % NSL == 0) mbar_wait(&fl_bar[0], (unsigned)(t / NSL) & 1u, 10);      // the item's stats
+      }
 #pragma unroll 1
       for (int h = 0; h < 2; ++h) {
         mbar_wait(&raw_full[h], (unsigned)t & 1u, 4);
@@ -225,6 +263,11 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
 #pragma unroll
           for (int c = 0; c < SL; ++c) v[c] = raw[(c * 2 + row) * SW + px];
           const int q = 2 * h + row;
+          if constexpr (FL) {
+            const float mx = fl_stats[q * SW + px], rr = fl_stats[(4 + q) * SW + px];     // m [4][SW], then r [4][SW]
+#pragma unroll
+            for (int c = 0; c < SL; ++c) v[c] = logit_p(v[c], F.inv_temp, mx, rr);
+          }
           const int off = ((q * 2) * APX + px + 4) * 16;                 // staged pixel px is column px - 4
           *reinterpret_cast<float4*>(ahi + off) = make_float4(v[0], v[1], v[2], v[3]);
           *reinterpret_cast<float4*>(ahi + off + APX * 16) = make_float4(v[4], v[5], v[6], v[7]);
@@ -237,6 +280,9 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> tensor-core reads
       __syncwarp();
       if (lane == 0) mbar_arrive(&a_full[a]);
+      if constexpr (FL) {
+        if (t % NSL == NSL - 1 && lane == 0) mbar_arrive(&fl_bar[1]);             // done with the item's stats
+      }
     }
   } else if (wid >= 8) {
     // ===== epilogue =====
@@ -247,8 +293,78 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
       const int item = it0 + i;
       const int n = item / pairs, r = (item - n * pairs) * 2;
       const int nrow = (r + 1 < P.H) ? 2 : 1;
+      if constexpr (FL) {
+        // while the MMAs run: pull the item's output logits and stats into L2 (128-byte lines, all epilogue lanes)
+        const int lines = (P.W * 4 + 127) / 128;
+        const int per_plane = nrow * lines;
+        for (int e = threadIdx.x - 256; e < (KC + 2) * per_plane; e += 128) {
+          const int ch = e / per_plane, rem = e - ch * per_plane, row = rem / lines, ln = rem - row * lines;
+          const float* src = ch < KC ? F.lout + (size_t)n * F.l_sn + (size_t)ch * F.l_sc + (size_t)(r + row) * F.l_sh
+                                     : F.sout + ((size_t)n * 2 + (ch - KC)) * plane + (size_t)(r + row) * P.W;
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(src + ln * 32));
+        }
+      }
       mbar_wait(&accum_full, (unsigned)i & 1u, 8);
       asm volatile("tcgen05.fence::after_thread_sync;");
+      if constexpr (FL) {
+        for (int orow = 0; orow < nrow; ++orow)
+          for (int mt = 0; mt < ntile; ++mt) {
+            const int c = mt * 128 + q4 * 32 + lane;
+            const bool live = c < P.W && !(P.dbg & 8);
+            const int row = r + orow;
+            float* dst = P.out + (size_t)n * P.out_sn + (size_t)row * P.W + c;
+            const float* lp = F.lout + (size_t)n * F.l_sn + (size_t)row * F.l_sh + c;
+            const float* sp = F.sout + (size_t)n * 2 * plane + (size_t)row * P.W + c;
+            const float mx = live ? __ldg(sp) : 0.f, rr = live ? __ldg(sp + plane) : 0.f;
+            float dot = 0.f;
+            // pass 1: sum_k g_k p_k over the four 32-channel chunks, in channel order
+#pragma unroll 1
+            for (int ch = 0; ch < KC / 32; ++ch) {
+              uint32_t v[32];
+              const uint32_t taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(orow * 2 + mt) * KC + ch * 32;
+              asm volatile(
+                  "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+                  "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+                  "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                    "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+                    "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+                    "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+                  : "r"(taddr));
+              asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+              if (live) {
+#pragma unroll
+                for (int o = 0; o < 32; ++o) {
+                  const float pr = logit_p(__ldg(lp + (size_t)(ch * 32 + o) * F.l_sc), F.inv_temp, mx, rr);
+                  dot = fmaf(g * __uint_as_float(v[o]), pr, dot);
+                }
+              }
+            }
+            // pass 2: the gradient, channel by channel
+#pragma unroll 1
+            for (int ch = 0; ch < KC / 32; ++ch) {
+              uint32_t v[32];
+              const uint32_t taddr = tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(orow * 2 + mt) * KC + ch * 32;
+              asm volatile(
+                  "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+                  "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+                  "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                    "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+                    "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+                    "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+                  : "r"(taddr));
+              asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+              if (live) {
+#pragma unroll
+                for (int o = 0; o < 32; ++o) {
+                  const float pr = logit_p(__ldg(lp + (size_t)(ch * 32 + o) * F.l_sc), F.inv_temp, mx, rr);
+                  dst[(size_t)(ch * 32 + o) * plane] = F.inv_temp * pr * (g * __uint_as_float(v[o]) - dot);
+                }
+              }
+            }
+          }
+      } else {
       for (int orow = 0; orow < nrow; ++orow)
         for (int mt = 0; mt < ntile; ++mt) {
           const int c = mt * 128 + q4 * 32 + lane;
@@ -273,6 +389,7 @@ local_bwd_tc_kernel(const __grid_constant__ CUtensorMap maps, const Params P) {
             }
           }
         }
+      }
       asm volatile("tcgen05.fence::before_thread_sync;");
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty);
@@ -289,17 +406,32 @@ size_t local_bwd_tc_image_bytes(int K, int pad) {
   return (K == bwdtc::KC && pad == 1) ? (size_t)bwdtc::NSL * 9 * bwdtc::W_TILE : 0;
 }
 
-int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
+// stats == nullptr: probabilities; else logits with the per-pixel (m, r) of local_logit_stats_kernel in `stats`
+static int tc_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                  cudaStream_t st) {
   using namespace bwdtc;
   const int B = m.B, K = m.K, H = m.H, W = m.W, pad = m.pad, sms = m.sms;
   if (K != KC || pad != 1 || W % 4 != 0 || W > MAXW || W < 8) return -1;
+  const bool fl = stats != nullptr;
   CUtensorMap mx, my;
   if (!make_map_4d(&mx, m.x, m, W + 8, 2, SL)) return -1;
   if (!make_map_4d(&my, m.y, m, W + 8, 2, SL)) return -1;
+  const long long hw = (long long)H * W;
+  FLParams Fgx{}, Fgy{};
+  if (fl) {
+    if (!make_map_4d(&Fgx.stats, stats, 2 * B, 2, H, W, 2 * hw, hw, W, W + 8, 4, 2)) return -1;
+    Fgy.stats = Fgx.stats;
+    // dL/dx: source y (stats at B + n), output x;  dL/dy: source x, output y
+    Fgx.src_n = B; Fgx.inv_temp = inv_temp; Fgx.lout = m.x.p; Fgx.l_sn = m.x.sn; Fgx.l_sc = m.x.sc; Fgx.l_sh = m.x.sh;
+    Fgx.sout = stats;
+    Fgy.src_n = 0; Fgy.inv_temp = inv_temp; Fgy.lout = m.y.p; Fgy.l_sn = m.y.sn; Fgy.l_sc = m.y.sc; Fgy.l_sh = m.y.sh;
+    Fgy.sout = stats + 2 * B * hw;
+  }
   // the weight image lives in the tail of the caller's coefficient buffer (common.cuh)
   float* img_x = Wx + local_coeff_image_offset(K, pad, 1);
   float* img_y = Wy + local_coeff_image_offset(K, pad, 1);
-  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tc_kernel), (int)(SMEM_BYTES)));
+  if (fl) IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tc_kernel<true>), (int)(FL_SMEM_BYTES)));
+  else IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_bwd_tc_kernel<false>), (int)(SMEM_BYTES)));
   const int n_items = B * ((H + 1) / 2);
   const int grid = n_items < sms ? n_items : sms;
   const int wthreads = NSL * 9 * KC;
@@ -308,11 +440,25 @@ int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads&
   IIC_CHECK_CUDA(cudaGetLastError());
   const int dbg = tc::bringup_env("IIC_TC_DBG", 0);
   Params Pgx{B, H, W, n_items, img_x, g.grad_loss, g.gx, g.gx_sn, dbg};     // dL/dx from y
-  local_bwd_tc_kernel<<<grid, NTHREADS, SMEM_BYTES, st>>>(my, Pgx);
   Params Pgy{B, H, W, n_items, img_y, g.grad_loss, g.gy, g.gy_sn, dbg};     // dL/dy from x
-  local_bwd_tc_kernel<<<grid, NTHREADS, SMEM_BYTES, st>>>(mx, Pgy);
+  if (fl) {
+    local_bwd_tc_kernel<true><<<grid, NTHREADS, FL_SMEM_BYTES, st>>>(my, Pgx, Fgx);
+    local_bwd_tc_kernel<true><<<grid, NTHREADS, FL_SMEM_BYTES, st>>>(mx, Pgy, Fgy);
+  } else {
+    local_bwd_tc_kernel<false><<<grid, NTHREADS, SMEM_BYTES, st>>>(my, Pgx, Fgx);
+    local_bwd_tc_kernel<false><<<grid, NTHREADS, SMEM_BYTES, st>>>(mx, Pgy, Fgy);
+  }
   IIC_CHECK_CUDA(cudaGetLastError());
   return 0;
+}
+
+int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st) {
+  return tc_try(m, nullptr, 1.f, Wx, Wy, g, st);
+}
+
+int local_bwd_tc_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                        cudaStream_t st) {
+  return tc_try(m, stats, inv_temp, Wx, Wy, g, st);
 }
 
 }  // namespace iic

@@ -569,8 +569,8 @@ extern "C" int iic_local_joint_from_logits(const float* lx, long long x_sn, long
 }
 
 // Fused cluster-head softmax + local joint with caller-owned per-pixel stats: 16 <= K <= 24 where local_fl_tc_covered
-// holds (stats pass, then the packed tensor-core joint on the logits); the K = 10 shapes of iic_local_joint_from_logits
-// as there (stats untouched)
+// holds (stats pass, then the packed tensor-core joint on the logits), K = 128 where local_fl_tc128_covered holds (stats
+// pass, then the tc joint on the logits); the K = 10 shapes of iic_local_joint_from_logits as there (stats untouched)
 extern "C" int iic_local_joint_from_logits_stats(const float* lx, long long x_sn, long long x_sc, long long x_sh,
                                                  const float* ly, long long y_sn, long long y_sc, long long y_sh,
                                                  int B, int K, int H, int W, int pad, float inv_temperature, float* stats,
@@ -582,11 +582,30 @@ extern "C" int iic_local_joint_from_logits_stats(const float* lx, long long x_sn
   const int sms = sm_count_cached(current_device());
   IIC_REQUIRE(sms > 0, "iic_local_joint_from_logits_stats: no device");
   const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
-  if (!local_fl_tc_covered(m))
+  const bool wide = local_fl_tc128_covered(m);
+  if (!wide && K == 128) {
+    // (the workspace was sized for the tc joint's slots, not for the per-SM slots the K = 10 entry checks first)
+    set_error("iic_local_joint_from_logits_stats: K = 128 is fused at padding 1, W %% 16 == 0, W <= 248, 16-byte aligned "
+              "rows; apply the softmax and call iic_local_joint");
+    return IIC_UNSUPPORTED;
+  }
+  if (!wide && !local_fl_tc_covered(m))
     return iic_local_joint_from_logits(lx, x_sn, x_sc, x_sh, ly, y_sn, y_sc, y_sh, B, K, H, W, pad, inv_temperature, J_out,
                                        workspace, workspace_bytes, info_host, stream);
   IIC_REQUIRE(stats && (reinterpret_cast<uintptr_t>(stats) & 15) == 0,
               "iic_local_joint_from_logits_stats: stats must be a 16-byte aligned buffer of iic_local_logit_stats_floats");
+  if (wide) {
+    const int max_ctas = local_fl_tc128_slots(sms);
+    const size_t need = (size_t)max_ctas * 9 * K * K * sizeof(float);
+    IIC_REQUIRE(workspace_bytes >= need, "iic_local_joint_from_logits_stats: workspace too small (%zu < %zu)",
+                workspace_bytes, need);
+    if (int e = local_logit_stats(m, inv_temperature, stats, st)) return e;
+    SlotInfo slots{};
+    const int rc = local_joint_tc_fl_try(m, stats, inv_temperature, (float*)workspace, max_ctas, &slots, st);
+    if (rc > 0) return rc;
+    IIC_REQUIRE(rc == 0, "iic_local_joint_from_logits_stats: the tensor-core joint refused a covered shape");
+    return reduce_or_describe_slots(slots, (const float*)workspace, 3, K, 1, J_out, info_host, st);
+  }
   const size_t need = (size_t)sms * local_joint_tcp_slot_floats(K, pad) * sizeof(float);
   IIC_REQUIRE(workspace_bytes >= need, "iic_local_joint_from_logits_stats: workspace too small (%zu < %zu)",
               workspace_bytes, need);

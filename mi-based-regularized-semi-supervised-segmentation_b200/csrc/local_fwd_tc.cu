@@ -25,6 +25,12 @@
 // reduce_partials_kernel (local_fwd.cu) adds the slots in fp64 in a fixed order and undoes the permutation.
 // To bound the fp32 accumulation run in TMEM the k-blocks are processed in segments: after each segment the
 // accumulators are drained into the slot (first segment stores, later ones add).
+//
+// From-logits form (FL, the cluster head's SoftmaxWithT fused): x and y hold logits and local_logit_stats_kernel
+// (local_logits.cu) has written each pixel's (m, r).  The TMA warp also stages the stats of the k-block's 28 x columns
+// and 16 y pixels behind the y box, and the transform converts every logit it uses to p = exp(l * inv_temp - m) * r
+// (logit_p, common.cuh) before the fp32 / bf16 split.  Outside the map the TMA zero fill gives r = 0, so p = 0 there
+// (the conv padding), not softmax(0) = 1/K.
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -54,6 +60,13 @@ constexpr int NTHREADS = 384;                   // 4 control warps + two transfo
 // bias of about -1.4e-7 per 8-pixel slice that is (measured) uniform over the entries of J to 0.4 % of itself -- the
 // normalisation of iic_loss.py:129 removes a uniform factor.  32 k-blocks = 512 pixels bound it at 1e-5.
 constexpr int SEG_KB_DEFAULT = 32;
+// FL: a raw slot also holds the staged stats after RAW_BYTES: x [2][XRW] (m, r), then y [2][PXB] 256 bytes on (a TMA
+// destination must be 128-byte aligned); slots stay 1024-byte aligned (the y box is swizzled)
+constexpr int FL_SX = RAW_BYTES, FL_SY = RAW_BYTES + 256;
+constexpr int FL_STATS_BYTES = 2 * XRW * 4 + 2 * PXB * 4;         // 352 bytes copied
+constexpr int FL_RAW_STRIDE = (FL_SY + 2 * PXB * 4 + 1023) & ~1023;
+constexpr int FL_SMEM_BYTES = NRAW * FL_RAW_STRIDE + NOP * OP_BYTES + 1024;
+static_assert(FL_SX % 128 == 0 && FL_SY % 128 == 0 && FL_RAW_STRIDE % 1024 == 0, "TMA destinations must stay aligned");
 
 
 struct Params {
@@ -63,8 +76,21 @@ struct Params {
   int dbg;                      // bring-up switches (IIC_TC_DBG): 1 no loads, 4 no transform
 };
 
+// the from-logits form's extra arguments (unused by the probability instantiation)
+struct FLParams {
+  CUtensorMap sx, sy;           // the (2B, 2, H, W) stats tensor: x stats at n, y stats at B + n
+  float inv_temp;
+};
+
+// bytes between raw-ring slots (a namespace-scope function rather than a constexpr local, which can change the
+// probability instantiation's register assignment)
+template <bool FL>
+__device__ constexpr int raw_stride() { return FL ? FL_RAW_STRIDE : RAW_BYTES; }
+
+template <bool FL>
 __global__ void __launch_bounds__(NTHREADS, 1)
-local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_constant__ CUtensorMap mapy, const Params P) {
+local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_constant__ CUtensorMap mapy, const Params P,
+                      const __grid_constant__ FLParams F) {
   extern __shared__ __align__(1024) unsigned char smem_dyn[];
   __shared__ __align__(8) uint64_t raw_full[NRAW], raw_empty[NRAW], op_full[NOP], op_empty[NOP], accum_bar, drained_bar;
   __shared__ uint32_t tmem_base_s;
@@ -101,6 +127,7 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
     if (lane == 0) {
       tma_prefetch_desc(&mapx);
       tma_prefetch_desc(&mapy);
+      if constexpr (FL) { tma_prefetch_desc(&F.sx); tma_prefetch_desc(&F.sy); }
       // (image, row, segment) of the first k-block by division, then running counters: a division by a runtime value
       // costs this single-lane loop ~100 clk per k-block
       const int per_img = P.H * P.segs_w;
@@ -112,9 +139,15 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
         if (k >= NRAW) mbar_wait(&raw_empty[s], ((unsigned)(k / NRAW) & 1u) ^ 1u, 1);
         const int c0 = sg * PXB, uc = u, nc = n;
         if (++sg == P.segs_w) { sg = 0; if (++u == P.H) { u = 0; ++n; } }
-        unsigned char* st = raw_ring + (size_t)s * RAW_BYTES;
+        unsigned char* st = raw_ring + (size_t)s * raw_stride<FL>();
         if (P.dbg & 1) { mbar_arrive(&raw_full[s]); continue; }
-        mbar_arrive_expect_tx(&raw_full[s], RAW_BYTES);
+        if constexpr (FL) {
+          mbar_arrive_expect_tx(&raw_full[s], RAW_BYTES + FL_STATS_BYTES);
+          tma_load_4d(st + FL_SX, &F.sx, &raw_full[s], c0 - 4, uc + dy - 1, 0, nc);
+          tma_load_4d(st + FL_SY, &F.sy, &raw_full[s], c0, uc, 0, P.B + nc);
+        } else {
+          mbar_arrive_expect_tx(&raw_full[s], RAW_BYTES);
+        }
         tma_load_4d(st, &mapx, &raw_full[s], c0 - 4, uc + dy - 1, 0, nc);
         tma_load_4d(st + XRAW_BYTES, &mapy, &raw_full[s], c0, uc, 0, nc);
       }
@@ -167,7 +200,7 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
       const int s = k % NRAW, o = k % NOP;
       mbar_wait(&raw_full[s], (unsigned)(k / NRAW) & 1u, 3);
       if (k >= NOP) mbar_wait(&op_empty[o], ((unsigned)(k / NOP) & 1u) ^ 1u, 2);
-      const unsigned char* raw = raw_ring + (size_t)s * RAW_BYTES;
+      const unsigned char* raw = raw_ring + (size_t)s * raw_stride<FL>();
       unsigned char* op = smem + (size_t)o * OP_BYTES;
       if (!(P.dbg & 4)) {
         float v[XRU];
@@ -176,6 +209,13 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
         for (int q = 0; q < XRU / 4; ++q) {
           const float4 t = xr[q];
           v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
+        }
+        if constexpr (FL) {
+          // staged columns 3 .. 19 (group 0: shifts 0, 1) or 5 .. 20 (group 1: shift 2) are read; m [XRW], then r [XRW]
+          const float* sm = reinterpret_cast<const float*>(raw + FL_SX);
+#pragma unroll
+          for (int q = 3; q <= 20; ++q)
+            if (grp == 1 ? q >= 5 : q <= 19) v[q] = logit_p(v[q], F.inv_temp, sm[q], sm[XRW + q]);
         }
 #pragma unroll
         for (int dx = 0; dx < 3; ++dx) {
@@ -199,7 +239,14 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           const int off = r * 64 + ((c ^ sw) << 4);
-          const float4 t = *reinterpret_cast<const float4*>(raw + XRAW_BYTES + off);
+          float4 t = *reinterpret_cast<const float4*>(raw + XRAW_BYTES + off);
+          if constexpr (FL) {
+            const float* sm = reinterpret_cast<const float*>(raw + FL_SY) + 4 * c;            // m [PXB], then r [PXB]
+            t.x = logit_p(t.x, F.inv_temp, sm[0], sm[PXB + 0]);
+            t.y = logit_p(t.y, F.inv_temp, sm[1], sm[PXB + 1]);
+            t.z = logit_p(t.z, F.inv_temp, sm[2], sm[PXB + 2]);
+            t.w = logit_p(t.w, F.inv_temp, sm[3], sm[PXB + 3]);
+          }
           *reinterpret_cast<float4*>(op + 3 * TILE_BYTES + off) = t;
           yv[4 * c] = t.x; yv[4 * c + 1] = t.y; yv[4 * c + 2] = t.z; yv[4 * c + 3] = t.w;
         }
@@ -283,25 +330,49 @@ local_joint_tc_kernel(const __grid_constant__ CUtensorMap mapx, const __grid_con
 
 }  // namespace fwdtc
 
-int local_joint_tc_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st) {
+// stats == nullptr: probabilities; else logits with the per-pixel (m, r) of local_logit_stats_kernel in `stats`
+static int tc_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, int max_ctas, SlotInfo* slots,
+                  cudaStream_t st) {
   using namespace fwdtc;
   const int B = m.B, H = m.H, W = m.W;
   if (m.K != KC || m.pad != 1 || W % PXB != 0 || max_ctas < 1) return -1;
+  const bool fl = stats != nullptr;
   CUtensorMap mx, my;
   if (!make_map_4d(&mx, m.x, m, XRW, 1, KC)) return -1;
   if (!make_map_4d(&my, m.y, m, PXB, 1, KC, CU_TENSOR_MAP_SWIZZLE_64B)) return -1;
+  FLParams F{};
+  F.inv_temp = inv_temp;
+  if (fl) {
+    const long long hw = (long long)H * W;
+    if (!make_map_4d(&F.sx, stats, 2 * B, 2, H, W, 2 * hw, hw, W, XRW, 1, 2)) return -1;
+    if (!make_map_4d(&F.sy, stats, 2 * B, 2, H, W, 2 * hw, hw, W, PXB, 1, 2)) return -1;
+  }
   const long long nkb = (long long)B * H * (W / PXB);
   int gx = m.sms / 3;                                 // three displacement rows per share of the pixels
   if (gx > max_ctas) gx = max_ctas;
   if (gx > nkb) gx = (int)nkb;
   if (gx < 1) gx = 1;
-  IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tc_kernel), (int)(SMEM_BYTES)));
   Params P{B, H, W, W / PXB, partial, tc::bringup_env("IIC_TC_SEG", SEG_KB_DEFAULT),
            tc::bringup_env("IIC_TC_DBG", 0)};
-  local_joint_tc_kernel<<<dim3(gx, 3), NTHREADS, SMEM_BYTES, st>>>(mx, my, P);
+  if (fl) {
+    IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tc_kernel<true>), (int)(FL_SMEM_BYTES)));
+    local_joint_tc_kernel<true><<<dim3(gx, 3), NTHREADS, FL_SMEM_BYTES, st>>>(mx, my, P, F);
+  } else {
+    IIC_CHECK_RC(ensure_dyn_smem((const void*)(local_joint_tc_kernel<false>), (int)(SMEM_BYTES)));
+    local_joint_tc_kernel<false><<<dim3(gx, 3), NTHREADS, SMEM_BYTES, st>>>(mx, my, P, F);
+  }
   IIC_CHECK_CUDA(cudaGetLastError());
   *slots = SlotInfo{SLOT_TC128, gx, (long long)9 * KC * KC, 0};
   return 0;
+}
+
+int local_joint_tc_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st) {
+  return tc_try(m, nullptr, 1.f, partial, max_ctas, slots, st);
+}
+
+int local_joint_tc_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, int max_ctas,
+                          SlotInfo* slots, cudaStream_t st) {
+  return tc_try(m, stats, inv_temp, partial, max_ctas, slots, st);
 }
 
 }  // namespace iic

@@ -40,6 +40,9 @@ int local_joint_fast_try(const LocalMaps& m, float* partial, int max_ctas, SlotI
                          int from_logits, float inv_temp, cudaStream_t st);
 int local_joint_fast7_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st);
 int local_joint_tc_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, cudaStream_t st);
+// its from-logits form (K = 128): `stats` holds the per-pixel (m, r) of both maps (local_logit_stats, local_logits.cu)
+int local_joint_tc_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* partial, int max_ctas,
+                          SlotInfo* slots, cudaStream_t st);
 int local_joint_tcj10_try(const LocalMaps& m, float* partial, int max_ctas, SlotInfo* slots, int* flags, int* checked,
                           int from_logits, float inv_temp, cudaStream_t st);
 int local_joint_tcp_try(const LocalMaps& m, float* partial, size_t partial_floats, SlotInfo* slots, cudaStream_t st);
@@ -60,6 +63,8 @@ int local_bwd_tma_try(const LocalMaps& m, const float* Wx, const float* Wy, cons
 int local_bwd_fast_try(const LocalMaps& m, const float* Wx, const float* Wy, const LocalGrads& g, int from_logits,
                        float inv_temp, cudaStream_t st);
 int local_bwd_tc_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st);
+int local_bwd_tc_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
+                        cudaStream_t st);
 int local_bwd_tcrb_try(const LocalMaps& m, float* Wx, float* Wy, const LocalGrads& g, cudaStream_t st);
 int local_bwd_tcrb_fl_try(const LocalMaps& m, const float* stats, float inv_temp, float* Wx, float* Wy, const LocalGrads& g,
                           cudaStream_t st);
@@ -73,10 +78,13 @@ int local_bwd_tcrb10h_try(const LocalMaps& m, const float* Wx, const float* Wy, 
 size_t local_bwd_tc_image_bytes(int K, int pad);      // K = 128, padding 1
 size_t local_bwd_tcrb_image_bytes(int K, int pad);    // 16 <= K <= 24, padding 1 or 3
 
-// ---- from logits, 16 <= K <= 24 (local_logits.cu) ----
-// THE rule that decides whether such a term runs fused (tcp joint + tcrb backward on logits): used by both entry points
-// and by iic_local_from_logits_covered
+// ---- from logits with per-pixel stats: 16 <= K <= 24 and K = 128 (local_logits.cu) ----
+// THE rules that decide whether such a term runs fused, used by both entry points and by iic_local_from_logits_covered:
+// 16 <= K <= 24 (tcp joint + tcrb backward on logits) and K = 128 (tc joint + tc backward on logits)
 bool local_fl_tc_covered(const LocalMaps& m);
+bool local_fl_tc128_covered(const LocalMaps& m);
+// joints the wide heads' from-logits joint may spread over (its grid is SMs / 3 shares x 3 displacement rows)
+int local_fl_tc128_slots(int sms);
 // (m, r) of every pixel of both maps into stats = [2B][2][H][W] (x at n, y at B + n)
 int local_logit_stats(const LocalMaps& m, float inv_temp, float* stats, cudaStream_t st);
 

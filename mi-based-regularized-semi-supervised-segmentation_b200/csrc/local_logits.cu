@@ -1,9 +1,9 @@
-// The cluster head's softmax fused into the local IIC term for the reference's default cluster count (16 <= K <= 24,
-// contrastyou/trainer/_utils.py:15-23,137-168 feeding iic_loss.py:107-149): per-pixel softmax statistics, the coverage
-// rule and the size queries of the from-logits entry points.
+// The cluster head's softmax fused into the local IIC term for the reference's default cluster count (16 <= K <= 24)
+// and the wide heads (K = 128, padding 1; contrastyou/trainer/_utils.py:15-23,137-168 feeding iic_loss.py:107-149):
+// per-pixel softmax statistics, the coverage rules and the size queries of the from-logits entry points.
 //
-// The tensor-core kernels of this K range never hold all K channels of a pixel at once (the row-block backward stages
-// 8-channel slices), so they cannot normalise by themselves.  One streaming pass writes, per pixel of both maps,
+// The tensor-core kernels of these K never hold all K channels of a pixel at once while they stage it (8-channel
+// slices, or one channel row per thread), so they cannot normalise by themselves.  One streaming pass writes, per pixel of both maps,
 //   m = max_k (l_k * inv_temp)      r = 1 / sum_k exp(l_k * inv_temp - m)
 // and every consumer computes p = exp(l * inv_temp - m) * r with the same fp32 product l * inv_temp (__fmul_rn: never
 // contracted into an FMA).  (m, r) rather than one log-sum-exp: with T = 0.1 the scaled logits reach a few hundred, and
@@ -78,6 +78,18 @@ bool local_fl_tc_covered(const LocalMaps& m) {
   return true;
 }
 
+// K = 128 from logits is fused (tc joint + tc backward, both converting logits with the stats) when: padding 1;
+// W % 16 == 0 (the joint's 16-pixel k-blocks); 8 <= W <= 248 (the backward stages W + 8 columns in one TMA box);
+// 16-byte aligned rows of both maps; the tensor-core and TMA kernels not switched off.
+bool local_fl_tc128_covered(const LocalMaps& m) {
+  if (options().no_tc || options().no_tma) return false;
+  if (m.K != 128 || m.pad != 1) return false;
+  if (m.B < 1 || m.H < 1 || m.W < 16 || m.W % 16 != 0 || m.W > 248 || m.sms < 1) return false;
+  return rows16(m.x) && rows16(m.y);
+}
+
+int local_fl_tc128_slots(int sms) { return sms / 3 > 0 ? sms / 3 : 1; }
+
 // the K = 10 fused kernels' shapes, as include/iic_b200.h states them (local_fwd_fast3.inc, local_bwd_fast.cu)
 static bool fl10_covered(const LocalMaps& m) {
   return m.K == 10 && m.pad == 1 && m.W % 4 == 0 && m.W >= 4 && m.W <= 248 && rows16(m.x) && rows16(m.y);
@@ -97,6 +109,8 @@ extern "C" size_t iic_local_joint_from_logits_workspace_bytes(int device, int B,
   if (sms <= 0 || B <= 0 || K <= 0 || H <= 0 || W <= 0) return 0;
   const size_t tcp = local_joint_tcp_slot_floats(K, pad);
   if (tcp) return (size_t)sms * tcp * sizeof(float);
+  // K = 128: one [9][128][128] slot per share of the tc joint
+  if (K == 128 && pad == 1) return (size_t)local_fl_tc128_slots(sms) * 9 * K * K * sizeof(float);
   return (size_t)sms * 9 * K * K * sizeof(float);
 }
 
@@ -109,5 +123,5 @@ extern "C" int iic_local_from_logits_covered(int device, const float* lx, long l
     return -1;
   }
   const LocalMaps m{{lx, x_sn, x_sc, x_sh}, {ly, y_sn, y_sc, y_sh}, B, K, H, W, pad, sms};
-  return (local_fl_tc_covered(m) || fl10_covered(m)) ? 1 : 0;
+  return (local_fl_tc_covered(m) || local_fl_tc128_covered(m) || fl10_covered(m)) ? 1 : 0;
 }

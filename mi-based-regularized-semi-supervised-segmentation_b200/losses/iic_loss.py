@@ -22,7 +22,7 @@ from torch import Tensor, nn
 
 from .. import checks
 from ..ops import (FusedShapeUnsupported, GlobalIICFunction, GlobalTerm, JointFunction, LocalIICFunction,
-                   LocalIICLogitsFunction, LocalTerm, from_logits_covered, iic_terms)
+                   LocalIICLogitsFunction, LocalTerm, from_logits_covered, global_logits_covered, iic_terms)
 
 
 def _pair(x):
@@ -50,6 +50,21 @@ class IIDLoss(nn.Module):
                                                             checks.want_simplex_kernels())
         checks.finish(x_out.device, loss, "x_out / x_tf_out not normalized.")
         return loss, loss_no_lamb, p_i_j
+
+    def from_logits(self, logits_out: Tensor, logits_tf_out: Tensor, T: float = 1.0):
+        """``IIDLoss.forward(softmax(logits_out / T, 1), softmax(logits_tf_out / T, 1))`` -- the (N, K) rows of a
+        ``ClusterHead`` before its ``SoftmaxWithT`` (contrastyou/trainer/_utils.py:15-23, ``ClusterHead.logits()``) --
+        with the softmax inside the joint launch and its backward inside the gradient kernel.  Returns the same
+        ``(loss, loss_no_lamb, p_i_j)``; the gradients are with respect to the logits.  Covered: N <= 4096 rows and
+        K <= 128 clusters, float32 CUDA rows with unit inner stride (sub-head views of a wider head output included);
+        anything else applies the softmax first."""
+        assert logits_out.dim() == 2 and logits_tf_out.shape == logits_out.shape, (logits_out.shape, logits_tf_out.shape)
+        if global_logits_covered(logits_out, logits_tf_out):
+            t = GlobalTerm(logits_out, logits_tf_out, self.lamb, True, logits=True, inv_temperature=1.0 / float(T))
+            (r,) = iic_terms([t])
+            checks.finish(logits_out.device, r[0])
+            return r
+        return IIDLoss.forward(self, (logits_out / T).softmax(1), (logits_tf_out / T).softmax(1))
 
 
 def compute_joint(x_out: Tensor, x_tf_out: Tensor, symmetric=True) -> Tensor:
@@ -129,7 +144,8 @@ class IIDSegmentationSmallPathLoss(IIDSegmentationLoss):
         The fused kernels cover one patch (the patch at least the map) and
           * 10 clusters: padding 1, width a multiple of 4 and at most 248 (the udaiic decoder shapes);
           * 16 to 24 clusters (the reference's 20): padding 3, or padding 1 on maps with enough row blocks to fill the
-            GPU; width a multiple of 16.
+            GPU; width a multiple of 16;
+          * 128 clusters (the wide heads): padding 1, width a multiple of 16 and at most 248.
         Both need 16-byte aligned rows.  Any other shape applies the softmax first and takes the probability path."""
         assert logits_out.shape == logits_tf_out.shape, (logits_out.shape, logits_tf_out.shape)
         assert logits_out.requires_grad and logits_tf_out.requires_grad        # :110
@@ -158,8 +174,9 @@ def iic_losses(calls, from_logits: bool = False, T: float = 1.0):
     ``from_logits=True``: every ``x_out`` / ``x_tf_out`` is a cluster head's LOGITS and the result is that of the calls
     on ``softmax(x / T, 1)`` (the heads' ``SoftmaxWithT``, contrastyou/trainer/_utils.py:15-23).  Local terms whose shape
     the fused kernels cover (:func:`from_logits_covered`, see :meth:`IIDSegmentationSmallPathLoss.from_logits`) take the
-    softmax inside their kernels; the others, and the global terms' (N, K) rows, get ``torch.softmax`` first.  Gradients
-    are with respect to the logits.  Masks are not accepted with ``from_logits``."""
+    softmax inside their kernels, and so do global terms of at most 4096 rows and 128 clusters (the finish launch
+    normalises their rows, see :meth:`IIDLoss.from_logits`); the others get ``torch.softmax`` first.  Gradients are with
+    respect to the logits.  Masks are not accepted with ``from_logits``."""
     terms, post = [], []
     inv_t = 1.0 / float(T)
     for c in calls:
@@ -190,6 +207,10 @@ def iic_losses(calls, from_logits: bool = False, T: float = 1.0):
             post.append(None)
         elif isinstance(crit, IIDLoss):
             assert x.dim() == 2 and y.shape == x.shape, (x.shape, y.shape)
+            if from_logits and global_logits_covered(x, y):
+                terms.append(GlobalTerm(x, y, crit.lamb, True, logits=True, inv_temperature=inv_t))
+                post.append(crit)
+                continue
             if from_logits:
                 x, y = (x / T).softmax(1), (y / T).softmax(1)
             terms.append(GlobalTerm(x, y, crit.lamb, True))

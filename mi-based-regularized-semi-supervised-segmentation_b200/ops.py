@@ -373,6 +373,27 @@ def _global_backward_into(x, y, J, lamb, symmetric, g_loss, g_no_lamb, gP, gx, g
     _lib.check(rc, "iic_global_backward")
 
 
+def _global_backward_logits_into(x, y, J, lamb, symmetric, inv_temperature, g_loss, g_no_lamb, gP, gx, gy):
+    """_global_backward_into for a global term from logits (x, y the logit rows, J the joint of their softmax): the
+    gradients are with respect to the logits."""
+    lib = _lib.load()
+    x, y = _w_contig(x), _w_contig(y)
+    N, K = x.shape
+    assert gx.shape == x.shape and gy.shape == x.shape and gx.stride(1) == 1 and gy.stride(1) == 1
+    if g_loss is not None:
+        g_loss = g_loss.to(torch.float32).reshape(())
+    if g_no_lamb is not None:
+        g_no_lamb = g_no_lamb.to(torch.float32).reshape(())
+    if gP is not None:
+        gP = gP.to(torch.float32).contiguous()
+    with torch.cuda.device(x.device):
+        rc = lib.iic_global_backward_from_logits(x.data_ptr(), x.stride(0), y.data_ptr(), y.stride(0), N, K, J.data_ptr(),
+                                                 float(lamb), int(symmetric), float(inv_temperature), _ptr(g_loss),
+                                                 _ptr(g_no_lamb), _ptr(gP), gx.data_ptr(), gy.data_ptr(), gx.stride(0),
+                                                 gy.stride(0), _stream(x.device))
+    _lib.check(rc, "iic_global_backward_from_logits")
+
+
 def _as_oci(t: torch.Tensor) -> Tuple[int, int, int]:
     outer, C = t.shape[0], t.shape[1]
     inner = 1
@@ -732,15 +753,33 @@ class LocalTerm:
 
 
 class GlobalTerm:
-    """One global IIC call: IIDLoss / compute_joint on (N, K) rows."""
-    __slots__ = ("x", "y", "lamb", "symmetric", "want_losses")
+    """One global IIC call: IIDLoss / compute_joint on (N, K) rows; `logits` = the rows are the cluster head's logits and
+    the softmax(rows * inv_temperature) is applied inside the finish launch and the backward kernel (at most
+    GLOBAL_ROWS_MAX rows and GLOBAL_LOGITS_MAX_K clusters: global_logits_covered)."""
+    __slots__ = ("x", "y", "lamb", "symmetric", "want_losses", "logits", "inv_temperature")
 
-    def __init__(self, x, y, lamb=1.0, symmetric=True, want_losses=True):
+    def __init__(self, x, y, lamb=1.0, symmetric=True, want_losses=True, logits=False, inv_temperature=1.0):
         self.x, self.y, self.lamb, self.symmetric, self.want_losses = x, y, float(lamb), bool(symmetric), bool(want_losses)
+        self.logits, self.inv_temperature = bool(logits), float(inv_temperature)
 
 
 MAX_TERMS_PER_FINISH = 32
 GLOBAL_ROWS_MAX = 4096          # larger (N, K) inputs take the multi-CTA global joint kernel instead of iic_finish
+GLOBAL_LOGITS_MAX_K = 128       # widest global term the finish launch takes from logits
+
+
+def global_logits_covered(x: torch.Tensor, y: torch.Tensor) -> bool:
+    """Whether a global term on the (N, K) logit rows `x`, `y` runs with the softmax inside the finish launch and the
+    backward kernel (include/iic_b200.h: IIC_ITEM_GLOBAL_LOGITS); False means the caller applies the softmax first."""
+    return (x.is_cuda and y.is_cuda and x.dtype == torch.float32 and y.dtype == torch.float32 and x.dim() == 2
+            and x.shape == y.shape and 0 < x.shape[0] <= GLOBAL_ROWS_MAX and 0 < x.shape[1] <= GLOBAL_LOGITS_MAX_K)
+
+
+def _keeps_logit_stats(K: int) -> bool:
+    """Whether a from-logits local term with K clusters may keep per-pixel softmax statistics from its forward to its
+    backward: the tensor-core kernels of 16 <= K <= 24 and K = 128 do (local_logits.cu); the K = 10 kernels hold whole
+    pixels and normalise by themselves.  Whether a given shape uses the buffer is the library's coverage rule."""
+    return 16 <= K <= 24 or K == 128
 
 
 def _world():
@@ -783,7 +822,7 @@ def _finish_terms(terms, check_simplex):
                 if t.logits:
                     nbytes = max(lib.iic_local_joint_from_logits_workspace_bytes(dev.index or 0, B, K, H, W, t.pad), 4)
                     ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-                    if 16 <= K <= 24:
+                    if _keeps_logit_stats(K):
                         # per-pixel softmax statistics (m, r) of both maps, written by the joint, read by the backward
                         stats = torch.empty(lib.iic_local_logit_stats_floats(B, H, W), dtype=torch.float32, device=dev)
                     rc = lib.iic_local_joint_from_logits_stats(x.data_ptr(), x.stride(0), x.stride(1), x.stride(2),
@@ -836,7 +875,11 @@ def _finish_terms(terms, check_simplex):
                 x, y = _w_contig(t.x), _w_contig(t.y)
                 N, K = x.shape
                 P = torch.empty((K, K), dtype=torch.float32, device=dev)
-                it.kind, it.K, it.lamda = _lib.ITEM_GLOBAL_ROWS, K, t.lamb
+                if t.logits and not (0 < N <= GLOBAL_ROWS_MAX and K <= GLOBAL_LOGITS_MAX_K):
+                    raise ValueError(f"iic_b200: global term from logits of shape {tuple(x.shape)} is not covered "
+                                     f"(N <= {GLOBAL_ROWS_MAX}, K <= {GLOBAL_LOGITS_MAX_K}); apply the softmax first")
+                it.kind, it.K, it.lamda = _lib.ITEM_GLOBAL_LOGITS if t.logits else _lib.ITEM_GLOBAL_ROWS, K, t.lamb
+                it.inv_temperature = t.inv_temperature if t.logits else 0.0
                 it.x, it.x_sn, it.y, it.y_sn, it.N = x.data_ptr(), x.stride(0), y.data_ptr(), y.stride(0), N
                 it.symmetric, it.check_simplex = int(t.symmetric), int(bool(check_simplex))
                 it.loss_out, it.P_out = loss_buf[lo:].data_ptr(), P.data_ptr()
@@ -1066,25 +1109,25 @@ class IICTermsFunction(torch.autograd.Function):
                     continue
                 (gx, ax), (gy, ay) = target(2 * ti, x), target(2 * ti + 1, y)
                 if use_side:
-                    gjobs.append((x, y, J, lamb, symmetric, g1, g2, gP, gx, gy, ax, ay))
+                    gjobs.append((x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy, ax, ay))
                     continue
-                _global_backward_into(x, y, J.view(x.shape[1], x.shape[1]), lamb, symmetric, g1, g2, gP, gx, gy)
+                _global_backward_any(x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy)
             if ax is not None:
                 ax += gx
             if ay is not None:
                 ay += gy
         if gjobs:
             if side is None:                      # no local term had a gradient after all: plain launches
-                for (x, y, J, lamb, symmetric, g1, g2, gP, gx, gy, ax, ay) in gjobs:
-                    _global_backward_into(x, y, J.view(x.shape[1], x.shape[1]), lamb, symmetric, g1, g2, gP, gx, gy)
+                for (x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy, ax, ay) in gjobs:
+                    _global_backward_any(x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy)
                     if ax is not None:
                         ax += gx
                     if ay is not None:
                         ay += gy
             else:
                 with torch.cuda.stream(side):
-                    for (x, y, J, lamb, symmetric, g1, g2, gP, gx, gy, ax, ay) in gjobs:
-                        _global_backward_into(x, y, J.view(x.shape[1], x.shape[1]), lamb, symmetric, g1, g2, gP, gx, gy)
+                    for (x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy, ax, ay) in gjobs:
+                        _global_backward_any(x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy)
                         if ax is not None:
                             deferred.append((ax, gx))
                         if ay is not None:
@@ -1095,12 +1138,26 @@ class IICTermsFunction(torch.autograd.Function):
         return (None, None, None, *[G[i] if any_grad[i] else None for i in range(n_src)])
 
 
+def _global_backward_any(x, y, J, lamb, symmetric, logits, inv_t, g1, g2, gP, gx, gy):
+    """The gradient kernel of one global term of an IICTermsFunction: from its rows, or from its logits."""
+    Jm = J.view(x.shape[1], x.shape[1])
+    if logits:
+        _global_backward_logits_into(x, y, Jm, lamb, symmetric, inv_t, g1, g2, gP, gx, gy)
+    else:
+        _global_backward_into(x, y, Jm, lamb, symmetric, g1, g2, gP, gx, gy)
+
+
 def iic_terms(terms, check_simplex=False):
     """Evaluate many IIC terms together; returns a list with, per term, the loss (LocalTerm) or the tuple
     (loss, loss_no_lamb, P) (GlobalTerm).  Global terms with more than GLOBAL_ROWS_MAX rows and batches beyond
-    MAX_TERMS_PER_FINISH are split off transparently."""
+    MAX_TERMS_PER_FINISH are split off transparently; a global term from logits that the finish launch does not cover
+    (global_logits_covered) gets torch.softmax(rows * inv_temperature) first."""
     terms = list(terms)
     out = [None] * len(terms)
+    for i, t in enumerate(terms):
+        if isinstance(t, GlobalTerm) and t.logits and not global_logits_covered(t.x, t.y):
+            terms[i] = GlobalTerm((t.x * t.inv_temperature).softmax(1), (t.y * t.inv_temperature).softmax(1), t.lamb,
+                                  t.symmetric, t.want_losses)
     batch = [i for i, t in enumerate(terms) if isinstance(t, LocalTerm) or t.x.shape[0] <= GLOBAL_ROWS_MAX]
     for i, t in enumerate(terms):
         if i not in batch:
@@ -1150,7 +1207,8 @@ class LocalIICLogitsFunction(torch.autograd.Function):
     """LocalIICFunction applied to softmax(logits / T, dim=1) of both maps, with the softmax and its
     backward fused into the joint and gradient kernels (contrastyou/trainer/_utils.py:15-23,137-168 feeding
     iic_loss.py:107-149); one patch = the whole map.  Raises FusedShapeUnsupported for other shapes.  For 16 <= K <= 24
-    the forward also writes the per-pixel softmax statistics of both maps, kept with Wx / Wy for the backward."""
+    and K = 128 the forward also writes the per-pixel softmax statistics of both maps, kept with Wx / Wy for the
+    backward."""
 
     @staticmethod
     def forward(ctx, lx, ly, pad, lamda, inv_temperature):

@@ -29,6 +29,9 @@ class IIDLoss(_IIDLoss):
     def forward(self, x_out: Tensor, x_tf_out: Tensor):
         return super().forward(x_out, x_tf_out)[0]
 
+    def from_logits(self, logits_out: Tensor, logits_tf_out: Tensor, T: float = 1.0):
+        return super().from_logits(logits_out, logits_tf_out, T)[0]
+
 
 def _nlist(n):
     def parse(x):

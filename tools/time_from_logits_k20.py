@@ -1,4 +1,5 @@
-"""Times the softmax-fused local term for 16 <= K <= 24 against torch.softmax + the probability path, in CUDA graphs,
+"""Times the softmax-fused local term (16 <= K <= 24, and K = 128 at padding 1) against torch.softmax + the probability
+path, in CUDA graphs,
 with inputs rotated over enough copies that the working set exceeds the 126 MB L2:
 
   forward   fused: stats pass + from-logits joint + finish     fallback: torch softmax x2 + joint + finish
@@ -8,6 +9,7 @@ with inputs rotated over enough copies that the working set exceeds the 126 MB L
             output, fwd + bwd, against softmax + iic_losses
 
     python tools/time_from_logits_k20.py --shape 8,20,224,224 --pad 3 [--T 1.0] [--step]
+    python tools/time_from_logits_k20.py --shape 32,128,224,224 --pad 1        (the wide heads, BASELINE config 5)
 
 Prints the GPU name and power limit with the numbers, and which path the fused side took (the coverage query)."""
 import argparse
