@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IIC_B200_ABI_VERSION 8
+#define IIC_B200_ABI_VERSION 9
 
 /* flag bits written (OR-ed) into the int* `flags` words by the kernels */
 #define IIC_FLAG_NAN_LOSS 1      /* iic_loss.py:147-148,184-185 -> RuntimeError on the host  */
@@ -283,7 +283,9 @@ int iic_finish(const iic_finish_item* items_host, int n_items, double* J_all, lo
  * elements; kind 1 = KL_div(reduction="mean") (dc2:deepclustering2/loss/kl_losses.py:107-126):
  * sum_c -t*log((p+eps)/(t+eps)) * w_c, mean over outer*inner.  Call site semi_seg/epocher.py:221-224.
  * from_logits != 0: prob/target hold logits and the channel softmax (epocher.py:222-223) is fused in;
- * the gradient is then w.r.t. the prob logits.  The gradient flows to `prob` only.
+ * the gradient is then w.r.t. the prob logits.  The gradient flows to `prob` only.  1 <= C <= 256: up to
+ * 8 channels a thread holds all channels of its pixels, from 9 the channels of a pixel are spread over the
+ * warps of a CTA (DESIGN.md section 4.5).
  * ---------------------------------------------------------------------------------------------- */
 size_t iic_uda_workspace_bytes(int device);
 int iic_uda_forward(const float* prob, const float* target, long long outer, int C, long long inner,
@@ -303,7 +305,7 @@ int iic_uda_backward(const float* prob, const float* target, long long outer, in
  *          (dc2:deepclustering2/meters2/individual_meters/general_dice_meter.py:41-95):
  *          dice_out[0][o][c] = #pixels(argmax == c and label == c)       (_intersaction)
  *          dice_out[1][o][c] = #pixels(argmax == c) + #pixels(label == c) (_union)
- * logits (outer, C, inner) contiguous float32, C <= 8; labels (outer, inner) contiguous int64 class
+ * logits (outer, C, inner) contiguous float32, 1 <= C <= 256; labels (outer, inner) contiguous int64 class
  * indices; weight (nullable) C floats, already normalised as at kl_losses.py:100.  A label outside
  * [0, C) sets IIC_FLAG_BAD_LABEL and contributes nothing.  workspace >= iic_sup_workspace_bytes,
  * zero-initialised once by the caller.  The backward writes d loss / d logits (dense, same layout).
@@ -328,7 +330,7 @@ int iic_sup_backward(const float* logits, const long long* labels, long long out
  *   iic_uda_flip_forward  iic_uda_forward(prob, flip(target)) without materialising flip(target): the UDA
  *   iic_uda_flip_backward term of semi_seg/epocher.py:221-224 on `unlabel_tf_logits` and the unflipped
  *                         `unlabel_logits` (epocher.py:160-161 fused away).  kind / eps / from_logits as for
- *                         iic_uda_forward (no class weights, no simplex pass); C <= 8.  workspace >=
+ *                         iic_uda_forward (no class weights, no simplex pass); 1 <= C <= 256.  workspace >=
  *                         iic_uda_flip_workspace_bytes, zero-initialised once by the caller.
  * ---------------------------------------------------------------------------------------------- */
 #define IIC_FLIP_H 1

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libiic_b200.so")
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 FLAG_NAN_LOSS = 1
 FLAG_NOT_SIMPLEX = 2
 FLAG_BAD_LABEL = 4

@@ -196,6 +196,111 @@ __global__ void __launch_bounds__(256, NC <= 4 ? 3 : 2) uda_flip_bwd_kernel(
   }
 }
 
+// ---- wide-class path (9 <= C <= 256): the channels of a pixel spread over the 8 warps of a CTA (pixel_common.cuh) ----
+// grid (gx, outer); a tile is 32 pixel groups of one sample's plane, each read through the sample's flips as above.
+template <int V, int CW, bool FROM_LOGITS>
+__global__ void __launch_bounds__(256, CW >= 32 ? 1 : 2) uda_flip_fwd_wide_kernel(
+    const float* __restrict__ prob, const float* __restrict__ target, const unsigned char* __restrict__ flips, int C,
+    int H, int W, int kind, float eps, double denom, float* __restrict__ loss_out, int* __restrict__ flags,
+    FlipWorkspace* ws) {
+  __shared__ float2 red_p[2][WIDE_WARPS * 32 * V], red_t[2][WIDE_WARPS * 32 * V];
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  const long long o = blockIdx.y, inner = (long long)H * W;
+  const unsigned f = flips[o];
+  const bool fh = f & IIC_FLIP_H, fw = f & IIC_FLIP_W;
+  const float* pb = prob + o * C * inner;
+  const float* tb = target + o * C * inner;
+  double local = 0.0;
+  const long long ngroups = inner / V, ntiles = (ngroups + 31) / 32;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane;
+    const bool live = q < ngroups;
+    long long off_s, off_t;
+    flip_offsets<V>(q, H, W, fh, fw, &off_s, &off_t);
+    float p[CW][V], t[CW][V];
+    wide_load<V, CW>(pb + off_s, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, p);
+    wide_load<V, CW>(tb + off_t, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, t);
+    if (fw) reverse_group<V, CW>(t);
+    if (FROM_LOGITS) {
+      int arg[V];
+      wide_softmax<V, CW>(p, c0, red_p[it], nullptr, arg);
+      wide_softmax<V, CW>(t, c0, red_t[it], nullptr, arg);
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      float v = 0.f;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        if (c0 + j < C) {
+          if (kind == 0) { const float d = p[j][e] - t[j][e]; v = fmaf(d, d, v); }
+          else v += -t[j][e] * logf((p[j][e] + eps) / (t[j][e] + eps));
+        }
+      }
+      if (live) local += v;
+    }
+  }
+  wide_loss_combine(local, denom, &ws->ticket, reinterpret_cast<double*>(ws + 1), loss_out, flags);
+}
+
+template <int V, int CW, bool FROM_LOGITS>
+__global__ void __launch_bounds__(256, CW >= 32 ? 1 : 2) uda_flip_bwd_wide_kernel(
+    const float* __restrict__ prob, const float* __restrict__ target, const unsigned char* __restrict__ flips, int C,
+    int H, int W, int kind, float eps, float inv_denom, const float* __restrict__ grad_loss,
+    float* __restrict__ grad_prob) {
+  __shared__ float2 red_p[2][WIDE_WARPS * 32 * V], red_t[2][WIDE_WARPS * 32 * V];
+  __shared__ float red_d[2][WIDE_WARPS * 32 * V];
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  const long long o = blockIdx.y, inner = (long long)H * W;
+  const unsigned f = flips[o];
+  const bool fh = f & IIC_FLIP_H, fw = f & IIC_FLIP_W;
+  const float* pb = prob + o * C * inner;
+  const float* tb = target + o * C * inner;
+  float* gb = grad_prob + o * C * inner;
+  const float g = (grad_loss ? __ldg(grad_loss) : 1.f) * inv_denom;
+  const long long ngroups = inner / V, ntiles = (ngroups + 31) / 32;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane;
+    const bool live = q < ngroups;
+    long long off_s, off_t;
+    flip_offsets<V>(q, H, W, fh, fw, &off_s, &off_t);
+    float p[CW][V], t[CW][V];
+    wide_load<V, CW>(pb + off_s, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, p);
+    wide_load<V, CW>(tb + off_t, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, t);
+    if (fw) reverse_group<V, CW>(t);
+    if (FROM_LOGITS) {
+      int arg[V];
+      wide_softmax<V, CW>(p, c0, red_p[it], nullptr, arg);
+      wide_softmax<V, CW>(t, c0, red_t[it], nullptr, arg);
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      float dot = 0.f;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        float gp = 0.f;
+        if (c0 + j < C) {
+          gp = (kind == 0) ? 2.f * (p[j][e] - t[j][e]) * g : -t[j][e] / (p[j][e] + eps) * g;
+          dot = fmaf(gp, p[j][e], dot);
+        }
+        t[j][e] = gp;                          // reuse as the gradient w.r.t. the probabilities
+      }
+      if (FROM_LOGITS) red_d[it][(threadIdx.x >> 5) * 32 * V + lane * V + e] = dot;
+    }
+    if (FROM_LOGITS) {
+      __syncthreads();
+#pragma unroll
+      for (int e = 0; e < V; ++e) {
+        const float dot = wide_warp_sum<V>(red_d[it], lane * V + e);
+#pragma unroll
+        for (int j = 0; j < CW; ++j) t[j][e] = p[j][e] * (t[j][e] - dot);   // softmax adjoint
+      }
+    }
+    wide_store<V, CW>(gb + off_s, inner, c0, C, live, t);
+  }
+}
+
 static bool flip_vec_ok(const void* a, const void* b, const void* c, int W) {
   if (W % 4 != 0) return false;
   return ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c)) & 15) == 0;
@@ -250,12 +355,26 @@ extern "C" int iic_uda_flip_forward(const float* prob, const float* target, cons
   IIC_REQUIRE(prob && target && flips && loss_out && flags && workspace, "iic_uda_flip_forward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && H > 0 && W > 0, "iic_uda_flip_forward: empty tensor");
   IIC_REQUIRE(outer <= 65535, "iic_uda_flip_forward: outer=%lld > 65535 samples unsupported", outer);
-  IIC_REQUIRE(C <= SUP_CMAX, "iic_uda_flip_forward: C=%d > %d channels unsupported", C, SUP_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_uda_flip_forward: C=%d > %d channels unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(kind == 0 || kind == 1, "iic_uda_flip_forward: kind must be 0 (mse) or 1 (kl)");
   cudaStream_t st = (cudaStream_t)stream;
   const long long inner = (long long)H * W, total = outer * inner;
   const double denom = kind == 0 ? (double)total * C : (double)total;
   const bool vec = flip_vec_ok(prob, target, prob, W);
+  if (C > SUP_CMAX) {
+    const long long ntiles = (inner / (vec ? 4 : 1) + 31) / 32;
+#define IIC_FLIP_FWD_WIDE(VV, CW)                                                                                   \
+    do {                                                                                                            \
+      const auto kern = from_logits ? uda_flip_fwd_wide_kernel<VV, CW, true> : uda_flip_fwd_wide_kernel<VV, CW, false>; \
+      const dim3 wgrid(pixel_ctas_per_sample(outer, ntiles * 256, wide_ctas_per_sm(kern)), (unsigned)outer);         \
+      kern<<<wgrid, 256, 0, st>>>(prob, target, flips, C, H, W, kind, (float)eps, denom, loss_out, flags,           \
+                                  (FlipWorkspace*)workspace);                                                       \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_FLIP_FWD_WIDE);
+#undef IIC_FLIP_FWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   const dim3 grid(pixel_ctas_per_sample(outer, vec ? inner / 4 : inner, C <= 4 ? 3 : 2), (unsigned)outer);
 #define IIC_FLIP_FWD(VV, NN, FL)                                                                              \
   uda_flip_fwd_kernel<VV, NN, FL><<<grid, 256, 0, st>>>(prob, target, flips, C, H, W, kind, (float)eps, denom, \
@@ -272,12 +391,25 @@ extern "C" int iic_uda_flip_backward(const float* prob, const float* target, con
   IIC_REQUIRE(prob && target && flips && grad_prob, "iic_uda_flip_backward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && H > 0 && W > 0, "iic_uda_flip_backward: empty tensor");
   IIC_REQUIRE(outer <= 65535, "iic_uda_flip_backward: outer=%lld > 65535 samples unsupported", outer);
-  IIC_REQUIRE(C <= SUP_CMAX, "iic_uda_flip_backward: C=%d > %d channels unsupported", C, SUP_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_uda_flip_backward: C=%d > %d channels unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(kind == 0 || kind == 1, "iic_uda_flip_backward: kind must be 0 (mse) or 1 (kl)");
   cudaStream_t st = (cudaStream_t)stream;
   const long long inner = (long long)H * W, total = outer * inner;
   const float inv_denom = (float)(1.0 / (kind == 0 ? (double)total * C : (double)total));
   const bool vec = flip_vec_ok(prob, target, grad_prob, W);
+  if (C > SUP_CMAX) {
+    const long long ntiles = (inner / (vec ? 4 : 1) + 31) / 32;
+#define IIC_FLIP_BWD_WIDE(VV, CW)                                                                                   \
+    do {                                                                                                            \
+      const auto kern = from_logits ? uda_flip_bwd_wide_kernel<VV, CW, true> : uda_flip_bwd_wide_kernel<VV, CW, false>; \
+      const dim3 wgrid(pixel_ctas_per_sample(outer, ntiles * 256, wide_ctas_per_sm(kern)), (unsigned)outer);         \
+      kern<<<wgrid, 256, 0, st>>>(prob, target, flips, C, H, W, kind, (float)eps, inv_denom, grad_loss, grad_prob); \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_FLIP_BWD_WIDE);
+#undef IIC_FLIP_BWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   const dim3 grid(pixel_ctas_per_sample(outer, vec ? inner / 4 : inner, C <= 4 ? 3 : 2), (unsigned)outer);
 #define IIC_FLIP_BWD(VV, NN, FL)                                                                                  \
   uda_flip_bwd_kernel<VV, NN, FL><<<grid, 256, 0, st>>>(prob, target, flips, C, H, W, kind, (float)eps, inv_denom, \

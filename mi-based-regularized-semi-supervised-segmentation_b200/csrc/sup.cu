@@ -170,6 +170,129 @@ __global__ void __launch_bounds__(256, NC <= 4 ? 3 : 2) sup_bwd_kernel(const flo
   }
 }
 
+// ---- wide-class path (9 <= C <= 256): the channels of a pixel spread over the 8 warps of a CTA (pixel_common.cuh) ----
+// grid (gx, outer) as above; a CTA walks the tiles of its sample.  The warp that holds the labelled class adds the
+// pixel's loss term.  Dice: the warps holding a pixel's argmax and label class count it into 2*C shared-memory
+// counters, added to dice_out with integer atomics at the end (order-independent, so bit-exact).
+template <int V, int CW>
+__global__ void __launch_bounds__(256, CW * V >= 32 ? 1 : 2) sup_fwd_wide_kernel(const float* __restrict__ logits,
+                                                           const long long* __restrict__ labels, int C, long long inner,
+                                                           float eps, const float* __restrict__ weight, double denom,
+                                                           float* __restrict__ loss_out, long long* __restrict__ dice_out,
+                                                           int* __restrict__ flags, SupWorkspace* ws) {
+  __shared__ float2 red[2][WIDE_WARPS * 32 * V];
+  __shared__ int red_arg[2][WIDE_WARPS * 32 * V];
+  __shared__ unsigned int s_cnt[2][WIDE_CMAX];                    // [intersection, union][class]
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  const long long o = blockIdx.y, outer = gridDim.y;
+  const float* lg = logits + o * C * inner;
+  const long long* lb = labels + o * inner;
+  for (int k = threadIdx.x; k < 2 * WIDE_CMAX; k += blockDim.x) (&s_cnt[0][0])[k] = 0u;
+  __syncthreads();
+  double local = 0.0;
+  bool bad = false;
+  const long long ngroups = inner / V, ntiles = (ngroups + 31) / 32;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane;
+    const bool live = q < ngroups;
+    float x[CW][V];
+    long long l[V];
+    wide_load<V, CW>(lg + q * V, inner, c0, C, live, -INFINITY, x);
+    if (live) sup_load_labels<V>(lb + q * V, l);
+#pragma unroll
+    for (int e = 0; e < V; ++e) if (!live) l[e] = -1;
+    int arg[V];
+    wide_softmax<V, CW>(x, c0, red[it], red_arg[it], arg);
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      const bool ok = (l[e] >= 0 && l[e] < C);
+      bad |= live && !ok;
+      const int li = ok ? (int)l[e] : -1, ai = live ? arg[e] : -1;   // a lane past the end has l = -1
+      float pl = 1.f;
+      bool own = false;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        if (c0 + j == li) { pl = x[j][e]; own = true; }
+      }
+      if (dice_out != nullptr) {
+        if (own) {
+          atomicAdd(&s_cnt[1][li], 1u);
+          if (ai == li) atomicAdd(&s_cnt[0][li], 1u);
+        }
+        if (ai >= c0 && ai < c0 + CW) atomicAdd(&s_cnt[1][ai], 1u);
+      }
+      // -target * log((prob + eps) / (target + eps)) * weight with target = 1 (kl_losses.py:114-118)
+      if (own) local += -logf((pl + eps) / (1.f + eps)) * (weight ? __ldg(weight + li) : 1.f);
+    }
+  }
+  if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(flags, IIC_FLAG_BAD_LABEL);
+  if (dice_out != nullptr) {
+    __syncthreads();
+    for (int k = threadIdx.x; k < 2 * C; k += blockDim.x) {
+      const int which = k / C, c = k - which * C;
+      const unsigned v = s_cnt[which][c];
+      // dice_out[which][sample][class]
+      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(dice_out) + ((long long)which * outer + o) * C + c,
+                       (unsigned long long)v);
+    }
+  }
+  wide_loss_combine(local, denom, &ws->ticket, reinterpret_cast<double*>(ws + 1), loss_out, flags);
+}
+
+// softmax adjoint with the dot sum_k gp_k p_k = gp_l p_l supplied by the warp that holds the label
+template <int V, int CW>
+__global__ void __launch_bounds__(256, CW * V >= 32 ? 1 : 2) sup_bwd_wide_kernel(const float* __restrict__ logits,
+                                                           const long long* __restrict__ labels, int C, long long inner,
+                                                           float eps, const float* __restrict__ weight, float inv_denom,
+                                                           const float* __restrict__ grad_loss,
+                                                           float* __restrict__ grad_logits) {
+  __shared__ float2 red[2][WIDE_WARPS * 32 * V];
+  __shared__ float red_d[2][WIDE_WARPS * 32 * V];
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  const long long o = blockIdx.y;
+  const float* lg = logits + o * C * inner;
+  const long long* lb = labels + o * inner;
+  float* gl = grad_logits + o * C * inner;
+  const float g = (grad_loss ? __ldg(grad_loss) : 1.f) * inv_denom;
+  const long long ngroups = inner / V, ntiles = (ngroups + 31) / 32;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane;
+    const bool live = q < ngroups;
+    float x[CW][V];
+    long long l[V];
+    wide_load<V, CW>(lg + q * V, inner, c0, C, live, -INFINITY, x);
+    if (live) sup_load_labels<V>(lb + q * V, l);
+#pragma unroll
+    for (int e = 0; e < V; ++e) if (!live) l[e] = -1;
+    int arg[V];
+    wide_softmax<V, CW>(x, c0, red[it], nullptr, arg);
+    int li[V];
+    float gpl[V];
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      li[e] = (live && l[e] >= 0 && l[e] < C) ? (int)l[e] : -1;
+      float pl = 0.f;
+      bool own = false;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        if (c0 + j == li[e]) { pl = x[j][e]; own = true; }
+      }
+      gpl[e] = own ? -(weight ? __ldg(weight + li[e]) : 1.f) / (pl + eps) * g : 0.f;
+      red_d[it][(threadIdx.x >> 5) * 32 * V + lane * V + e] = gpl[e] * pl;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      const float dot = wide_warp_sum<V>(red_d[it], lane * V + e);
+#pragma unroll
+      for (int j = 0; j < CW; ++j) x[j][e] = x[j][e] * ((c0 + j == li[e] ? gpl[e] : 0.f) - dot);
+    }
+    wide_store<V, CW>(gl + q * V, inner, c0, C, live, x);
+  }
+}
+
 static bool sup_vec_ok(const void* a, const void* b, const void* c, long long inner) {
   if (inner % 4 != 0) return false;
   return ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c)) & 15) == 0;
@@ -193,11 +316,26 @@ extern "C" int iic_sup_forward(const float* logits, const long long* labels, lon
   IIC_REQUIRE(logits && labels && loss_out && flags && workspace, "iic_sup_forward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && inner > 0, "iic_sup_forward: empty tensor");
   IIC_REQUIRE(outer <= 65535, "iic_sup_forward: outer=%lld > 65535 samples unsupported", outer);
-  IIC_REQUIRE(C <= SUP_CMAX, "iic_sup_forward: C=%d > %d classes unsupported", C, SUP_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_sup_forward: C=%d > %d classes unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(eps > 0.0, "iic_sup_forward: eps must be > 0 (the reference's loss is NaN at eps = 0)");
   cudaStream_t st = (cudaStream_t)stream;
   if (dice_out) IIC_CHECK_CUDA(cudaMemsetAsync(dice_out, 0, (size_t)2 * outer * C * sizeof(long long), st));
   const double denom = (double)outer * (double)inner;
+  if (C > SUP_CMAX) {
+    const bool vec = wide_vec_ok(logits, labels, logits, inner);
+    const long long ntiles = (inner / (vec ? 4 : 1) + 31) / 32;
+#define IIC_SUP_FWD_WIDE(VV, CW)                                                                                    \
+    do {                                                                                                            \
+      const auto kern = sup_fwd_wide_kernel<VV, CW>;                                                                \
+      const dim3 wgrid(pixel_ctas_per_sample(outer, ntiles * 256, wide_ctas_per_sm(kern)), (unsigned)outer);         \
+      kern<<<wgrid, 256, 0, st>>>(logits, labels, C, inner, (float)eps, weight, denom, loss_out, dice_out, flags,    \
+                                  (SupWorkspace*)workspace);                                                        \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_SUP_FWD_WIDE);
+#undef IIC_SUP_FWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   const bool vec = sup_vec_ok(logits, labels, logits, inner);
   const dim3 grid(pixel_ctas_per_sample(outer, vec ? inner / 4 : inner, C <= 4 ? 3 : 2), (unsigned)outer);
 #define IIC_SUP_FWD(VV, NN)                                                                                      \
@@ -216,10 +354,24 @@ extern "C" int iic_sup_backward(const float* logits, const long long* labels, lo
   IIC_REQUIRE(logits && labels && grad_logits, "iic_sup_backward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && inner > 0, "iic_sup_backward: empty tensor");
   IIC_REQUIRE(outer <= 65535, "iic_sup_backward: outer=%lld > 65535 samples unsupported", outer);
-  IIC_REQUIRE(C <= SUP_CMAX, "iic_sup_backward: C=%d > %d classes unsupported", C, SUP_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_sup_backward: C=%d > %d classes unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(eps > 0.0, "iic_sup_backward: eps must be > 0");
   cudaStream_t st = (cudaStream_t)stream;
   const float inv_denom = (float)(1.0 / ((double)outer * (double)inner));
+  if (C > SUP_CMAX) {
+    const bool vec = wide_vec_ok(logits, labels, grad_logits, inner);
+    const long long ntiles = (inner / (vec ? 4 : 1) + 31) / 32;
+#define IIC_SUP_BWD_WIDE(VV, CW)                                                                                    \
+    do {                                                                                                            \
+      const auto kern = sup_bwd_wide_kernel<VV, CW>;                                                                \
+      const dim3 wgrid(pixel_ctas_per_sample(outer, ntiles * 256, wide_ctas_per_sm(kern)), (unsigned)outer);         \
+      kern<<<wgrid, 256, 0, st>>>(logits, labels, C, inner, (float)eps, weight, inv_denom, grad_loss, grad_logits); \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_SUP_BWD_WIDE);
+#undef IIC_SUP_BWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   const bool vec = sup_vec_ok(logits, labels, grad_logits, inner);
   const dim3 grid(pixel_ctas_per_sample(outer, vec ? inner / 4 : inner, C <= 4 ? 3 : 2), (unsigned)outer);
 #define IIC_SUP_BWD(VV, NN)                                                                                      \

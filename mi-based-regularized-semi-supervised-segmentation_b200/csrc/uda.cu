@@ -7,6 +7,7 @@
 // consecutive floats per channel: fully coalesced.  With from_logits the two channel softmaxes of
 // epocher.py:222-223 are computed in registers and never touch HBM.
 #include "common.cuh"
+#include "pixel_common.cuh"
 
 namespace iic {
 
@@ -280,6 +281,126 @@ __global__ void __launch_bounds__(256) uda_bwd_vec_kernel(const float* __restric
   }
 }
 
+// ---- wide-class UDA path (9 <= C <= 256): the channels of a pixel spread over the 8 warps of a CTA -------------------
+// (pixel_common.cuh).  A tile is 32 consecutive pixel groups of the flattened outer*inner map (V = 4 needs
+// inner % 4 == 0, so a group never straddles two samples); a 1-D grid of at most 8 CTAs per SM walks the tiles.  Each
+// input byte is read once per pass; the softmaxes, the simplex sums and the adjoint's dot are merged in shared memory.
+template <int V, int CW, bool FROM_LOGITS>
+__global__ void __launch_bounds__(256, CW >= 32 ? 1 : 2) uda_fwd_wide_kernel(const float* __restrict__ prob,
+                                                           const float* __restrict__ target, long long outer, int C,
+                                                           long long inner, int kind, float eps,
+                                                           const float* __restrict__ weight, double denom,
+                                                           float* __restrict__ loss_out, int* __restrict__ flags,
+                                                           int check_simplex, UdaWorkspace* ws) {
+  __shared__ float2 red_p[2][WIDE_WARPS * 32 * V], red_t[2][WIDE_WARPS * 32 * V];
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  float wt[CW];
+#pragma unroll
+  for (int j = 0; j < CW; ++j) wt[j] = (weight && c0 + j < C) ? __ldg(weight + c0 + j) : 1.f;
+  const long long ngroups = outer * inner / V, ntiles = (ngroups + 31) / 32;
+  double local = 0.0;
+  bool bad = false;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane, px = q * V;
+    const bool live = q < ngroups;
+    const long long o = px / inner, base = o * C * inner + (px - o * inner);
+    float p[CW][V], t[CW][V];
+    wide_load<V, CW>(prob + base, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, p);
+    wide_load<V, CW>(target + base, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, t);
+    if (FROM_LOGITS) {
+      int arg[V];
+      wide_softmax<V, CW>(p, c0, red_p[it], nullptr, arg);
+      wide_softmax<V, CW>(t, c0, red_t[it], nullptr, arg);
+    }
+    float sp[V], st[V];
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      float v = 0.f;
+      sp[e] = 0.f; st[e] = 0.f;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        if (c0 + j < C) {
+          sp[e] += p[j][e]; st[e] += t[j][e];
+          if (kind == 0) { const float d = p[j][e] - t[j][e]; v = fmaf(d, d, v); }
+          else v += -t[j][e] * logf((p[j][e] + eps) / (t[j][e] + eps)) * wt[j];
+        }
+      }
+      if (live) local += v;
+    }
+    if (check_simplex && !FROM_LOGITS) {
+      float2* red = red_p[it];
+#pragma unroll
+      for (int e = 0; e < V; ++e) red[(threadIdx.x >> 5) * 32 * V + lane * V + e] = make_float2(sp[e], st[e]);
+      __syncthreads();
+#pragma unroll
+      for (int e = 0; e < V; ++e) {
+        float2 s = red[lane * V + e];
+#pragma unroll
+        for (int w = 1; w < WIDE_WARPS; ++w) { s.x += red[w * 32 * V + lane * V + e].x; s.y += red[w * 32 * V + lane * V + e].y; }
+        if (live && (!(fabsf(s.x - 1.f) <= 2e-4f) || !(fabsf(s.y - 1.f) <= 2e-4f))) bad = true;
+      }
+    }
+  }
+  if (check_simplex && __any_sync(0xffffffffu, bad) && lane == 0) atomicOr(flags, IIC_FLAG_NOT_SIMPLEX);
+  wide_loss_combine(local, denom, &ws->ticket, reinterpret_cast<double*>(ws + 1), loss_out, flags);
+}
+
+template <int V, int CW, bool FROM_LOGITS>
+__global__ void __launch_bounds__(256, CW >= 32 ? 1 : 2) uda_bwd_wide_kernel(const float* __restrict__ prob,
+                                                           const float* __restrict__ target, long long outer, int C,
+                                                           long long inner, int kind, float eps,
+                                                           const float* __restrict__ weight, float inv_denom,
+                                                           const float* __restrict__ grad_loss,
+                                                           float* __restrict__ grad_prob) {
+  __shared__ float2 red_p[2][WIDE_WARPS * 32 * V], red_t[2][WIDE_WARPS * 32 * V];
+  __shared__ float red_d[2][WIDE_WARPS * 32 * V];
+  const int lane = threadIdx.x & 31, c0 = (threadIdx.x >> 5) * CW;
+  const float g = (grad_loss ? __ldg(grad_loss) : 1.f) * inv_denom;
+  float wt[CW];
+#pragma unroll
+  for (int j = 0; j < CW; ++j) wt[j] = (weight && c0 + j < C) ? __ldg(weight + c0 + j) : 1.f;
+  const long long ngroups = outer * inner / V, ntiles = (ngroups + 31) / 32;
+  int it = 0;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it ^= 1) {
+    const long long q = tile * 32 + lane, px = q * V;
+    const bool live = q < ngroups;
+    const long long o = px / inner, base = o * C * inner + (px - o * inner);
+    float p[CW][V], t[CW][V];
+    wide_load<V, CW>(prob + base, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, p);
+    wide_load<V, CW>(target + base, inner, c0, C, live, FROM_LOGITS ? -INFINITY : 0.f, t);
+    if (FROM_LOGITS) {
+      int arg[V];
+      wide_softmax<V, CW>(p, c0, red_p[it], nullptr, arg);
+      wide_softmax<V, CW>(t, c0, red_t[it], nullptr, arg);
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+      float dot = 0.f;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        float gp = 0.f;
+        if (c0 + j < C) {
+          gp = (kind == 0) ? 2.f * (p[j][e] - t[j][e]) * g : -t[j][e] / (p[j][e] + eps) * wt[j] * g;
+          dot = fmaf(gp, p[j][e], dot);
+        }
+        t[j][e] = gp;                      // reuse as the gradient w.r.t. the probabilities
+      }
+      if (FROM_LOGITS) red_d[it][(threadIdx.x >> 5) * 32 * V + lane * V + e] = dot;
+    }
+    if (FROM_LOGITS) {
+      __syncthreads();
+#pragma unroll
+      for (int e = 0; e < V; ++e) {
+        const float dot = wide_warp_sum<V>(red_d[it], lane * V + e);
+#pragma unroll
+        for (int j = 0; j < CW; ++j) t[j][e] = p[j][e] * (t[j][e] - dot);   // softmax adjoint
+      }
+    }
+    wide_store<V, CW>(grad_prob + base, inner, c0, C, live, t);
+  }
+}
+
 static bool uda_vec_ok(const void* a, const void* b, const void* c, long long outer, int C, long long inner) {
   if (C < 2 || C > 4) return false;
   if (inner % 4 != 0) return false;
@@ -324,13 +445,28 @@ extern "C" int iic_uda_forward(const float* prob, const float* target, long long
                                void* workspace, void* stream) {
   IIC_REQUIRE(prob && target && loss_out && flags && workspace, "iic_uda_forward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && inner > 0, "iic_uda_forward: empty tensor");
-  IIC_REQUIRE(C <= UDA_CMAX, "iic_uda_forward: C=%d > %d channels unsupported", C, UDA_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_uda_forward: C=%d > %d channels unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(kind == 0 || kind == 1, "iic_uda_forward: kind must be 0 (mse) or 1 (kl)");
   const long long total = outer * inner;
   const int grid = uda_grid(total);
   // MSELoss: mean over all elements; KL_div "mean": mean over outer*inner after the channel sum
   const double denom = kind == 0 ? (double)total * C : (double)total;
   cudaStream_t st = (cudaStream_t)stream;
+  if (C > UDA_CMAX) {
+    const bool vec = wide_vec_ok(prob, target, prob, inner);
+    const long long ntiles = (total / (vec ? 4 : 1) + 31) / 32;
+#define IIC_UDA_FWD_WIDE(VV, CW)                                                                                  \
+    do {                                                                                                          \
+      const auto kern = from_logits ? uda_fwd_wide_kernel<VV, CW, true> : uda_fwd_wide_kernel<VV, CW, false>;     \
+      kern<<<wide_grid(kern, ntiles), 256, 0, st>>>(prob, target, outer, C, inner, kind, (float)eps, \
+                                                                   weight, denom, loss_out, flags, check_simplex,   \
+                                                                   (UdaWorkspace*)workspace);                       \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_UDA_FWD_WIDE);
+#undef IIC_UDA_FWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   if (uda_vec_ok(prob, target, prob, outer, C, inner)) {
     const unsigned nquads = (unsigned)(total / 4), inner4 = (unsigned)(inner / 4);
     const int vgrid = uda_grid(total / 4);
@@ -358,12 +494,26 @@ extern "C" int iic_uda_backward(const float* prob, const float* target, long lon
                                 int from_logits, const float* grad_loss, float* grad_prob, void* stream) {
   IIC_REQUIRE(prob && target && grad_prob, "iic_uda_backward: null pointer");
   IIC_REQUIRE(outer > 0 && C > 0 && inner > 0, "iic_uda_backward: empty tensor");
-  IIC_REQUIRE(C <= UDA_CMAX, "iic_uda_backward: C=%d > %d channels unsupported", C, UDA_CMAX);
+  IIC_REQUIRE(C <= WIDE_CMAX, "iic_uda_backward: C=%d > %d channels unsupported", C, WIDE_CMAX);
   IIC_REQUIRE(kind == 0 || kind == 1, "iic_uda_backward: kind must be 0 (mse) or 1 (kl)");
   const long long total = outer * inner;
   const int grid = uda_grid(total);
   const float inv_denom = (float)(1.0 / (kind == 0 ? (double)total * C : (double)total));
   cudaStream_t st = (cudaStream_t)stream;
+  if (C > UDA_CMAX) {
+    const bool vec = wide_vec_ok(prob, target, grad_prob, inner);
+    const long long ntiles = (total / (vec ? 4 : 1) + 31) / 32;
+#define IIC_UDA_BWD_WIDE(VV, CW)                                                                                  \
+    do {                                                                                                          \
+      const auto kern = from_logits ? uda_bwd_wide_kernel<VV, CW, true> : uda_bwd_wide_kernel<VV, CW, false>;     \
+      kern<<<wide_grid(kern, ntiles), 256, 0, st>>>(prob, target, outer, C, inner, kind, (float)eps, \
+                                                                   weight, inv_denom, grad_loss, grad_prob);        \
+    } while (0)
+    IIC_WIDE_DISPATCH(vec, C, IIC_UDA_BWD_WIDE);
+#undef IIC_UDA_BWD_WIDE
+    IIC_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   if (uda_vec_ok(prob, target, grad_prob, outer, C, inner)) {
     const unsigned nquads = (unsigned)(total / 4), inner4 = (unsigned)(inner / 4);
     const int vgrid = uda_grid(total / 4);
