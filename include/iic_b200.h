@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IIC_B200_ABI_VERSION 9
+#define IIC_B200_ABI_VERSION 10
 
 /* flag bits written (OR-ed) into the int* `flags` words by the kernels */
 #define IIC_FLAG_NAN_LOSS 1      /* iic_loss.py:147-148,184-185 -> RuntimeError on the host  */
@@ -309,6 +309,18 @@ int iic_uda_backward(const float* prob, const float* target, long long outer, in
  * indices; weight (nullable) C floats, already normalised as at kl_losses.py:100.  A label outside
  * [0, C) sets IIC_FLAG_BAD_LABEL and contributes nothing.  workspace >= iic_sup_workspace_bytes,
  * zero-initialised once by the caller.  The backward writes d loss / d logits (dense, same layout).
+ *
+ * The _ignore pair adds an ignore label (torch's `ignore_index`; Cityscapes / VOC void = 255):
+ *   - a pixel whose label equals ignore_index (any value, also one inside [0, C)) adds nothing to the
+ *     loss, gets an exactly zero gradient and is left out of dice_out (neither its argmax nor its label
+ *     is counted); it never sets IIC_FLAG_BAD_LABEL;
+ *   - n = #pixels whose label is not ignore_index, counted on the device by the forward into *n_valid
+ *     (1 int64, overwritten); the loss is the sum above over those pixels divided by n, with or without
+ *     weights (KL_div's mean, not torch's division by the summed weights); n = 0 gives a loss of 0.0,
+ *     a zero gradient and no IIC_FLAG_NAN_LOSS;
+ *   - any other label outside [0, C) behaves as above and counts in n;
+ *   - the backward reads n from the n_valid the forward wrote (stream order), so neither call
+ *     synchronises the host and a graph replay may see a different n each time.
  * ---------------------------------------------------------------------------------------------- */
 size_t iic_sup_workspace_bytes(int device, long long outer);
 int iic_sup_forward(const float* logits, const long long* labels, long long outer, int C, long long inner,
@@ -317,6 +329,12 @@ int iic_sup_forward(const float* logits, const long long* labels, long long oute
 int iic_sup_backward(const float* logits, const long long* labels, long long outer, int C, long long inner,
                      double eps, const float* weight, const float* grad_loss, float* grad_logits,
                      void* stream);
+int iic_sup_forward_ignore(const float* logits, const long long* labels, long long outer, int C, long long inner,
+                           double eps, const float* weight, long long ignore_index, float* loss_out,
+                           long long* dice_out, long long* n_valid, int* flags, void* workspace, void* stream);
+int iic_sup_backward_ignore(const float* logits, const long long* labels, long long outer, int C,
+                            long long inner, double eps, const float* weight, long long ignore_index,
+                            const long long* n_valid, const float* grad_loss, float* grad_logits, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Per-sample flip alignment (SURVEY.md section 8f row 2).  The reference aligns the two views with

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libiic_b200.so")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 FLAG_NAN_LOSS = 1
 FLAG_NOT_SIMPLEX = 2
 FLAG_BAD_LABEL = 4
@@ -72,6 +72,8 @@ PROTOTYPES = {
     "iic_sup_workspace_bytes": (_sz, [_i, _ll]),
     "iic_sup_forward": (_i, [_p, _p, _ll, _i, _ll, _d, _p, _p, _p, _p, _p, _p]),
     "iic_sup_backward": (_i, [_p, _p, _ll, _i, _ll, _d, _p, _p, _p, _p]),
+    "iic_sup_forward_ignore": (_i, [_p, _p, _ll, _i, _ll, _d, _p, _ll, _p, _p, _p, _p, _p, _p]),
+    "iic_sup_backward_ignore": (_i, [_p, _p, _ll, _i, _ll, _d, _p, _ll, _p, _p, _p, _p]),
     "iic_flip_batch": (_i, [_p, _p, _p, _ll, _i, _i, _i, _p]),
     "iic_uda_flip_workspace_bytes": (_sz, [_i, _ll]),
     "iic_uda_flip_forward": (_i, [_p, _p, _p, _ll, _i, _i, _i, _i, _d, _i, _p, _p, _p, _p]),

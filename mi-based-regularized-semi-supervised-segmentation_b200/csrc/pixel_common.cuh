@@ -211,17 +211,42 @@ __device__ __forceinline__ void wide_softmax(float (&x)[CW][V], int c0, float2* 
   }
 }
 
+// Ignore-label forms of the supervised kernels: the CTA's count of pixels that are not ignored, from the per-thread
+// counts (warp sums into one shared counter; integer, so exact).  Every thread calls it and gets the count.
+__device__ __forceinline__ unsigned long long cta_count(unsigned int n_local) {
+  __shared__ unsigned long long s_n;
+  if (threadIdx.x == 0) s_n = 0ull;
+  __syncthreads();
+  const unsigned int w = __reduce_add_sync(0xffffffffu, n_local);
+  if ((threadIdx.x & 31) == 0) atomicAdd(&s_n, (unsigned long long)w);
+  __syncthreads();
+  return s_n;
+}
+
+// The mean's denominator in the ignore-label forms: the device-side count n of pixels that are not ignored, complete
+// once the last CTA holds its ticket; the mean of an empty set is 0 (not NaN).
+__device__ __forceinline__ double mean_over_valid(double sum, const long long* n_valid) {
+  const long long n = *reinterpret_cast<const volatile long long*>(n_valid);
+  return n > 0 ? sum / (double)n : 0.0;
+}
+
 // Per-CTA fp64 partial of the loss into partial[linear CTA index]; the last CTA to take a ticket adds the partials in a
 // fixed order (thread t takes t, t + 256, ... then a fixed-shape block reduction) and writes sum / denom.  The ticket
-// resets itself.  Deterministic for a given grid.
+// resets itself.  Deterministic for a given grid.  IGN (the ignore-label forms): each CTA adds its count of pixels that
+// are not ignored (`n_local` per thread) to *n_valid before its ticket, and the last CTA divides by the final count
+// instead of `denom` (mean_over_valid).
+template <bool IGN = false>
 __device__ __forceinline__ void wide_loss_combine(double local, double denom, unsigned int* ticket, double* partial,
-                                                  float* __restrict__ loss_out, int* __restrict__ flags) {
+                                                  float* __restrict__ loss_out, int* __restrict__ flags,
+                                                  unsigned int n_local = 0u, long long* n_valid = nullptr) {
   __shared__ double scratch[40];
   __shared__ bool is_last;
+  const unsigned long long cta_n = IGN ? cta_count(n_local) : 0ull;
   const double bsum = block_sum(local, scratch);
   const unsigned int ncta = gridDim.x * gridDim.y;
   if (threadIdx.x == 0) {
     partial[blockIdx.y * gridDim.x + blockIdx.x] = bsum;
+    if (IGN && cta_n) atomicAdd(reinterpret_cast<unsigned long long*>(n_valid), cta_n);
     __threadfence();
     is_last = (atomicAdd(ticket, 1u) == ncta - 1);
   }
@@ -233,7 +258,7 @@ __device__ __forceinline__ void wide_loss_combine(double local, double denom, un
     for (unsigned int b = threadIdx.x; b < ncta; b += blockDim.x) tsum += pp[b];
     double tot = block_sum(tsum, scratch);
     if (threadIdx.x == 0) {
-      tot /= denom;
+      tot = IGN ? mean_over_valid(tot, n_valid) : tot / denom;
       loss_out[0] = (float)tot;
       if (tot != tot) atomicOr(flags, IIC_FLAG_NAN_LOSS);
       *ticket = 0;

@@ -12,6 +12,7 @@ what the ``sup_dice`` meter needs (epocher.py:183-184).
 """
 from __future__ import annotations
 
+import numbers
 from typing import List, Optional, Union
 
 import torch
@@ -115,7 +116,7 @@ def _normalised_weight(weight) -> Optional[Tensor]:
 
 
 def sup_kl_from_logits(logits: Tensor, target: Tensor, weight: Union[List[float], Tensor] = None,
-                       eps: float = 1e-16, return_dice: bool = False):
+                       eps: float = 1e-16, return_dice: bool = False, ignore_index: Optional[int] = None):
     """``KL_div(weight=weight, eps=eps)(logits.softmax(1), class2one_hot(target, C))`` without the
     probability map or the one-hot tensor (semi_seg/epocher.py:165-166; dc2:loss/kl_losses.py:107-126).
 
@@ -123,13 +124,29 @@ def sup_kl_from_logits(logits: Tensor, target: Tensor, weight: Union[List[float]
     With ``return_dice`` the call also returns ``(intersection, union)``, the two (B, C) int64 tensors
     ``UniversalDice.add(logits.max(1)[1], target)`` would append (dc2:general_dice_meter.py:41-95), counted in
     the same pass.  A label outside [0, C) raises AssertionError like ``class2one_hot`` (per the check mode).
+
+    ``ignore_index`` (an int, e.g. 255 for the Cityscapes / VOC void label, or torch's -100; a value inside [0, C)
+    drops that class): pixels labelled with it add nothing to the loss, get a zero gradient and are left out of the
+    Dice counts.  The loss is the sum over the other n pixels divided by n, also with ``weight``: this is
+    ``KL_div``'s mean over the kept pixels, not ``F.cross_entropy``'s division by the summed weights of the kept
+    labels.  n is counted on the GPU (no host synchronisation, so a CUDA graph can replay the call with a different
+    number of ignored pixels); when every pixel is ignored the loss is 0 and the gradient is zero.  Any other label
+    outside [0, C) still raises, and counts in n.
     """
+    if ignore_index is not None:
+        if isinstance(ignore_index, bool) or not isinstance(ignore_index, numbers.Integral):
+            raise TypeError(f"sup_kl_from_logits: ignore_index must be None or an int, got "
+                            f"{type(ignore_index).__name__}")
+        ignore_index = int(ignore_index)
+        if not -2 ** 63 <= ignore_index < 2 ** 63:
+            raise ValueError(f"sup_kl_from_logits: ignore_index={ignore_index} is not an int64 label")
     if target.dim() == logits.dim() and target.shape[1] == 1:
         target = target.squeeze(1)
     assert not target.requires_grad
     if not eps > 0:
         raise ValueError("sup_kl_from_logits needs eps > 0 (the reference's loss is NaN at eps = 0)")
-    loss, dice = SupervisedKLFunction.apply(logits, target, float(eps), _normalised_weight(weight), bool(return_dice))
+    loss, dice, _ = SupervisedKLFunction.apply(logits, target, float(eps), _normalised_weight(weight),
+                                               bool(return_dice), ignore_index)
     checks.finish(logits.device, loss, "prob / target is not a simplex over dim 1")
     if return_dice:
         return loss, (dice[0], dice[1])

@@ -37,8 +37,10 @@ _LIBDEF.define("flip_batch(Tensor x, Tensor flips) -> Tensor")
 _LIBDEF.define("uda_flip_forward(Tensor prob, Tensor target, Tensor flips, int kind, float eps, bool from_logits) -> Tensor")
 _LIBDEF.define("uda_flip_backward(Tensor prob, Tensor target, Tensor flips, int kind, float eps, bool from_logits, "
                "Tensor grad) -> Tensor")
-_LIBDEF.define("sup_forward(Tensor logits, Tensor labels, float eps, Tensor? weight, bool want_dice) -> (Tensor, Tensor)")
-_LIBDEF.define("sup_backward(Tensor logits, Tensor labels, float eps, Tensor? weight, Tensor grad) -> Tensor")
+_LIBDEF.define("sup_forward(Tensor logits, Tensor labels, float eps, Tensor? weight, bool want_dice, "
+               "int? ignore_index=None) -> (Tensor, Tensor, Tensor)")
+_LIBDEF.define("sup_backward(Tensor logits, Tensor labels, float eps, Tensor? weight, Tensor grad, "
+               "int? ignore_index=None, Tensor? n_valid=None) -> Tensor")
 
 
 # ---- per (device, stream) persistent state ---------------------------------------------------------
@@ -519,31 +521,50 @@ def _sup_args(logits, labels, weight):
     return logits.contiguous(), labels.contiguous(), weight
 
 
-def _sup_forward(logits, labels, eps, weight, want_dice):
+def _sup_forward(logits, labels, eps, weight, want_dice, ignore_index=None):
+    """-> (loss, dice counts or an empty tensor, n_valid): with ``ignore_index`` the one-element int64 count of pixels
+    whose label is not ``ignore_index`` (the loss's denominator, left on the device for the backward), else empty."""
     lib = _lib.load()
     logits, labels, weight = _sup_args(logits, labels, weight)
     outer, C, inner = _as_oci(logits)
     st = _state(logits.device)
     loss = torch.empty((), dtype=torch.float32, device=logits.device)
     dice = torch.empty((2, outer, C) if want_dice else (0,), dtype=torch.int64, device=logits.device)
+    n_valid = torch.empty((0,) if ignore_index is None else (1,), dtype=torch.int64, device=logits.device)
+    dice_ptr = dice.data_ptr() if want_dice else None
     with torch.cuda.device(logits.device):
-        rc = lib.iic_sup_forward(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps), _ptr(weight),
-                                 loss.data_ptr(), dice.data_ptr() if want_dice else None, st.flags.data_ptr(),
-                                 st.supervised_ws(outer, logits.device).data_ptr(), _stream(logits.device))
-    _lib.check(rc, "iic_sup_forward")
-    return loss, dice
+        if ignore_index is None:
+            rc = lib.iic_sup_forward(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps), _ptr(weight),
+                                     loss.data_ptr(), dice_ptr, st.flags.data_ptr(),
+                                     st.supervised_ws(outer, logits.device).data_ptr(), _stream(logits.device))
+        else:
+            rc = lib.iic_sup_forward_ignore(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps),
+                                            _ptr(weight), int(ignore_index), loss.data_ptr(), dice_ptr,
+                                            n_valid.data_ptr(), st.flags.data_ptr(),
+                                            st.supervised_ws(outer, logits.device).data_ptr(), _stream(logits.device))
+    _lib.check(rc, "iic_sup_forward" if ignore_index is None else "iic_sup_forward_ignore")
+    return loss, dice, n_valid
 
 
-def _sup_backward(logits, labels, eps, weight, grad):
+def _sup_backward(logits, labels, eps, weight, grad, ignore_index=None, n_valid=None):
     lib = _lib.load()
     logits, labels, weight = _sup_args(logits, labels, weight)
     outer, C, inner = _as_oci(logits)
     out = torch.empty_like(logits)
     grad = grad.to(torch.float32).reshape(())
     with torch.cuda.device(logits.device):
-        rc = lib.iic_sup_backward(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps), _ptr(weight),
-                                  grad.data_ptr(), out.data_ptr(), _stream(logits.device))
-    _lib.check(rc, "iic_sup_backward")
+        if ignore_index is None:
+            rc = lib.iic_sup_backward(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps), _ptr(weight),
+                                      grad.data_ptr(), out.data_ptr(), _stream(logits.device))
+        else:
+            if (n_valid is None or n_valid.dtype != torch.int64 or n_valid.numel() != 1
+                    or n_valid.device != logits.device):
+                raise ValueError("iic_b200.sup_backward: ignore_index needs the one-element int64 n_valid of the "
+                                 "forward on the logits' device")
+            rc = lib.iic_sup_backward_ignore(logits.data_ptr(), labels.data_ptr(), outer, C, inner, float(eps),
+                                             _ptr(weight), int(ignore_index), n_valid.data_ptr(), grad.data_ptr(),
+                                             out.data_ptr(), _stream(logits.device))
+    _lib.check(rc, "iic_sup_backward" if ignore_index is None else "iic_sup_backward_ignore")
     return out
 
 
@@ -1309,21 +1330,27 @@ class UDAFunction(torch.autograd.Function):
 
 class SupervisedKLFunction(torch.autograd.Function):
     """KL_div()(softmax(logits), one_hot(labels)) (semi_seg/epocher.py:165-166) and the Dice counts of the
-    `sup_dice` meter (epocher.py:183-184) from one pass over the logits; the gradient flows to `logits` only."""
+    `sup_dice` meter (epocher.py:183-184) from one pass over the logits; the gradient flows to `logits` only.
+    Returns (loss, dice, n_valid); with ``ignore_index`` the device-side count n_valid is the loss's denominator and
+    is saved for the backward (no host synchronisation)."""
 
     @staticmethod
-    def forward(ctx, logits, labels, eps, weight, want_dice):
-        loss, dice = ops.sup_forward(logits, labels, eps, weight, want_dice)
-        ctx.save_for_backward(logits, labels, weight)
+    def forward(ctx, logits, labels, eps, weight, want_dice, ignore_index=None):
+        loss, dice, n_valid = ops.sup_forward(logits, labels, eps, weight, want_dice, ignore_index)
+        ctx.save_for_backward(logits, labels, weight, n_valid)
         ctx.eps = eps
-        ctx.mark_non_differentiable(dice)
-        return loss, dice
+        ctx.ignore_index = ignore_index
+        ctx.mark_non_differentiable(dice, n_valid)
+        return loss, dice, n_valid
 
     @staticmethod
-    def backward(ctx, grad, _grad_dice):
-        logits, labels, weight = ctx.saved_tensors
-        g = ops.sup_backward(logits, labels, ctx.eps, weight, grad.contiguous())
-        return g, None, None, None, None
+    def backward(ctx, grad, _grad_dice, _grad_n_valid):
+        logits, labels, weight, n_valid = ctx.saved_tensors
+        if ctx.ignore_index is None:
+            g = ops.sup_backward(logits, labels, ctx.eps, weight, grad.contiguous())
+        else:
+            g = ops.sup_backward(logits, labels, ctx.eps, weight, grad.contiguous(), ctx.ignore_index, n_valid)
+        return g, None, None, None, None, None
 
 
 class FlipBatchFunction(torch.autograd.Function):
